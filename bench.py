@@ -3,6 +3,7 @@
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload rollout|reach|mug] [--envs-per-gpu E] [--dtype f32|f64]
     python bench.py --impl reference ...      # the CPU arm: oracle port of the reference step on all host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's obs / reward / terminated / truncated as DIR/*.npy
 
 One "step" = one Env.step for every environment on every rank.  Prints ONE JSON line.
 Workloads (BASELINE.json configs):
@@ -48,7 +49,16 @@ def parse():
     p.add_argument("--no-extra", action="store_true", help="skip the `workloads` block (mug / reach) of the default line")
     p.add_argument("--solver-iters", type=int, default=0, help="Newton iteration cap (0 = library default for the dtype)")
     p.add_argument("--no-l2-flush", action="store_true", help="profiling aid: skip the L2 flush between timed steps")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned (rank 0's environments) as DIR/<name>.npy, "
+                                                         "in the run's float dtype; inputs are seeded, so two builds can be compared output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.warmup < 0:
+        p.error("--warmup must not be negative")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs writes the GPU path's outputs; it does not apply to --impl reference")
+    return a
 
 
 WORKLOADS = {
@@ -84,15 +94,14 @@ class ClockSampler(threading.Thread):
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons, "samples": len(self.rows)}
 
 
-def cpu_leg(workload, steps_per_proc, procs=None):
-    """Oracle port of the reference step on the host cores (bounded sample)."""
+def cpu_leg(workload, steps_per_proc, procs=None, warmup=20):
+    """Oracle port of the reference step on the host cores: `warmup` untimed, then `steps_per_proc` timed env-steps per core."""
     from oracle import cpu_bench
     xml = os.path.join(ROOT, "ur3e_b200", "assets", "main.xml")
     # all three workloads' CPU legs run the v2 env step on main.xml, the reference's training env (train_rl.py:38-44), from reset
     # through truncation / auto-reset like the GPU arm's steady state; the reach workload (no mug) is cheaper per step, so this
     # is a conservative (slower) CPU number only for `reach`.
-    rate, procs, total, wall = cpu_bench.run(xml, "v2", steps_per_proc, procs)
-    return rate, procs, total, wall
+    return cpu_bench.run(xml, "v2", steps_per_proc, procs, warmup)
 
 
 def flops_per_env_step(model_name, frame_skip, nefc, ncon, it):
@@ -106,25 +115,21 @@ def flops_per_env_step(model_name, frame_skip, nefc, ncon, it):
 
 
 def run_reference(args):
-    """--impl reference: the reference's CPU implementation of the path.  mujoco/gymnasium are not installable here and the
-    reference's meshes are absent (SURVEY F3/F4; probe log profiles/r2_mujoco_probe.log), so this is the oracle port (kind
-    'port'), all host cores."""
+    """--impl reference: the reference's CPU implementation of the path.  The reference runs on the mujoco wheel and meshes that
+    this project does not ship (SURVEY F3/F4; probe log profiles/r2_mujoco_probe.log), so this is the oracle port (kind 'port'),
+    one environment per host core.  Every core takes --warmup untimed env-steps, then --steps timed ones; one step = one env-step
+    of every core's environment, timed by the slowest core."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     cores = os.cpu_count() or 1
-    per = args.cpu_steps or 8000
-    t_all = []
-    total_steps = 0
-    for _ in range(max(1, min(args.steps, 3))):    # bounded: a few samples, each ~ per x cores env-steps
-        rate, procs, total, wall = cpu_leg(args.workload, per, cores)
-        t_all.append(rate); total_steps += total
-    value = sorted(t_all)[len(t_all) // 2]
+    value, procs, total, slowest, wall = cpu_leg(args.workload, args.steps, cores, warmup=args.warmup)
     line = {"metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
-            "ms_per_step": 1e3 / value, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
-            "impl": "reference", "config": {"workload": WORKLOADS[args.workload]["desc"], "note": "one step here = one env-step of one CPU env; value aggregates all %d host cores" % cores},
-            "cpu_baseline": {"value": value, "unit": UNIT, "cores": cores, "kind": "port",
-                             "sample": "%d processes x %d ur3e-v2 env-steps (oracle float64 restatement; MuJoCo itself is not installable here), median of %d runs" % (cores, per, len(t_all))},
+            "ms_per_step": slowest * 1e3 / args.steps, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f64", "data": "synthetic",
+            "impl": "reference", "config": {"workload": WORKLOADS[args.workload]["desc"], "timed_env_steps": total,
+                                            "note": "one step here = one env-step of each of the %d CPU envs (one per host core); value aggregates them" % procs},
+            "cpu_baseline": {"value": value, "unit": UNIT, "cores": procs, "kind": "port",
+                             "sample": "%d processes x %d timed ur3e-v2 env-steps after %d untimed (float64 oracle restatement of the reference step)" % (procs, args.steps, args.warmup)},
             "e2e": {"value": value, "unit": UNIT, "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}, "gpu_launches": 0}
     print(json.dumps(line))
 
@@ -314,6 +319,25 @@ def rooflines(w, res, peaks):
     return r32, rh, ki
 
 
+DUMP_LIMIT = 64 * 10 ** 6       # bytes of all --dump-outputs files together, .npy headers included
+NPY_HEADER = 256                # upper bound of np.save's header for these shapes
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT):
+    """Write every [n, ...] array of `arrays` as out_dir/<name>.npy.  If they would exceed `limit` bytes together, the same fixed,
+    seeded sample of rows (environments) is written from each, in ascending order, and env_index.npy holds the row numbers."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    row = sum(a.nbytes for a in arrays.values()) // n
+    if n * row + NPY_HEADER * len(arrays) > limit:
+        k = (limit - NPY_HEADER * (len(arrays) + 1)) // (row + 8)
+        idx = np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+        arrays = dict({name: a[idx] for name, a in arrays.items()}, env_index=idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     args = parse()
     if args.impl == "reference":
@@ -340,6 +364,10 @@ def main():
     sampler = ClockSampler(local)
     res = measure(w, args.steps, n_warm, settle, flush, world, dist, sampler)
     value, total_ms = res["value"], res["total_ms"]
+    if args.dump_outputs and rank == 0:
+        # the batch-owned tensors SimBatch.step returns, as the last timed step left them; copied before the e2e leg steps the batch again
+        last = (batch.obs, batch.reward, batch.terminated, batch.truncated)
+        dump_outputs(args.dump_outputs, {name: t.to(dtype).cpu().numpy() for name, t in zip(("obs", "reward", "terminated", "truncated"), last)})
 
     # ---- e2e: the host-buffer C-ABI call, pinned host buffers, H2D + D2H inside the timed region
     e2e = None
@@ -417,7 +445,7 @@ def main():
     if not args.no_cpu_baseline:
         cores = os.cpu_count() or 1
         per = args.cpu_steps or 80000
-        rate, procs, total, wall = cpu_leg(args.workload, per, cores)
+        rate, procs, total, _, wall = cpu_leg(args.workload, per, cores)
         cpu = {"value": rate, "unit": UNIT, "cores": procs, "kind": "port",
                "sample": "%d processes (one per host core) x %d ur3e-v2 env-steps of the float64 oracle restatement, resets included (%.1f s wall); MuJoCo 3.3.3 is not installable here" % (procs, per, wall)}
 

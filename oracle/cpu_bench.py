@@ -10,13 +10,13 @@ import numpy as np
 
 
 def _worker(args):
-    xml, kind, steps, seed = args
+    xml, kind, steps, warmup, seed = args
     from oracle.envs import OracleEnv
     env = OracleEnv(xml, kind)
     rng = np.random.default_rng(seed)
     lo = np.array([0.29799994 - 0.25, 0.13349916 - 0.25, 0.0, 0.0]); hi = np.array([0.29799994 + 0.25, 0.13349916 + 0.25, 0.5, 1.0])
     env.reset((rng.uniform(0, 0.02), rng.uniform(-0.25, 0.2)))
-    for _ in range(20):
+    for _ in range(warmup):
         env.step(lo + (hi - lo) * rng.random(4))
     t0 = time.perf_counter(); n = 0
     for _ in range(steps):
@@ -26,17 +26,18 @@ def _worker(args):
     return n, time.perf_counter() - t0
 
 
-def run(xml, kind="v2", steps_per_proc=3000, procs=None):
-    """Returns (env_steps_per_second aggregated over processes, procs, total steps, wall seconds)."""
+def run(xml, kind="v2", steps_per_proc=3000, procs=None, warmup=20):
+    """Every process steps one environment `warmup` untimed env-steps, then `steps_per_proc` timed ones.  Returns
+    (timed env-steps per second aggregated over processes, procs, total timed env-steps, slowest timed window in s, wall seconds)."""
     procs = procs or (os.cpu_count() or 1)
     ctx = mp.get_context("spawn")
     t0 = time.perf_counter()
     with ctx.Pool(procs) as pool:
-        res = pool.map(_worker, [(xml, kind, steps_per_proc, 1000 + i) for i in range(procs)])
+        res = pool.map(_worker, [(xml, kind, steps_per_proc, warmup, 1000 + i) for i in range(procs)])
     wall = time.perf_counter() - t0
     total = sum(r[0] for r in res)
     slowest = max(r[1] for r in res)
-    return total / slowest, procs, total, wall
+    return total / slowest, procs, total, slowest, wall
 
 
 if __name__ == "__main__":

@@ -43,16 +43,13 @@ def test_model_arrays_match_oracle_loader():
         m.keyframe("missing")
 
 
-def test_loader_errors_are_reported():
+def test_loader_errors_are_reported(tmp_path):
     with pytest.raises(ValueError, match="cannot open"):
         Model("/nonexistent/model.xml")
-    bad = os.path.join(ROOT, "tests", "golden", "_bad.xml")
+    bad = str(tmp_path / "_bad.xml")
     open(bad, "w").write("<mujoco><compiler angle='radian'/><worldbody><body><joint type='ball'/></body></worldbody></mujoco>")
-    try:
-        with pytest.raises(ValueError, match="not supported"):
-            Model(bad)
-    finally:
-        os.remove(bad)
+    with pytest.raises(ValueError, match="not supported"):
+        Model(bad)
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
