@@ -23,7 +23,7 @@ typedef struct ur3e_batch ur3e_batch;
 
 enum { UR3E_F32 = 0, UR3E_F64 = 1 };
 /* object kinds for name lookups: numeric values of mujoco.mjtObj used by utils/utils.py:29-66 */
-enum { UR3E_OBJ_BODY = 1, UR3E_OBJ_JOINT = 3, UR3E_OBJ_GEOM = 5, UR3E_OBJ_SITE = 6, UR3E_OBJ_TENDON = 18, UR3E_OBJ_ACTUATOR = 19, UR3E_OBJ_KEY = 23 };
+enum { UR3E_OBJ_BODY = 1, UR3E_OBJ_XBODY = 2 /* body frame (mjOBJ_XBODY); kinematics queries only */, UR3E_OBJ_JOINT = 3, UR3E_OBJ_GEOM = 5, UR3E_OBJ_SITE = 6, UR3E_OBJ_TENDON = 18, UR3E_OBJ_ACTUATOR = 19, UR3E_OBJ_KEY = 23 };
 /* controller evaluated inside the step kernel */
 enum { UR3E_CTRL_RAW = 0,          /* action = actuator ctrl (imitation_env_direct.py:90) */
        UR3E_CTRL_PD_JOINT = 1,     /* controller_func.py:128-167 pd_joint_ctrl + move_j.py:14-38 */
@@ -122,6 +122,19 @@ int ur3e_batch_kernel_timing(ur3e_batch* b, int enable);
 int ur3e_batch_kernel_times(ur3e_batch* b, double* out6);
 /* bytes of the persistent per-environment record in HBM (read + written once per step) */
 int ur3e_batch_state_bytes(const ur3e_batch* b);
+/* Kinematics queries: d.xpos/xmat, d.xipos/ximat, d.geom_xpos/xmat, d.site_xpos/xmat and mj_objectVelocity (utils/utils.py:129-189,
+ * utils/gym_utils.py:20-39,207-219) for k objects of every environment.
+ * ur3e_batch_query_create compiles k (objtype, id) pairs of the loaded model, 1 <= k <= 256, objtype one of UR3E_OBJ_BODY (inertial
+ * frame: xipos / ximat), UR3E_OBJ_XBODY (body frame: xpos / xmat, what d.body(name).xpos returns), UR3E_OBJ_GEOM, UR3E_OBJ_SITE
+ * (ids as ur3e_model_name2id returns them); it returns the query's id (>= 0).  The batch owns its queries until ur3e_batch_destroy.
+ * ur3e_batch_query writes, for every environment, pos_dev [n, k, 3], mat_dev [n, k, 9] (row-major) and vel_dev [n, k, 6]
+ * ([rot(3), lin(3)] as mj_objectVelocity; flg_local = 1: in the object's frame) in the batch's dtype; any of them may be NULL, not
+ * all.  Asynchronous on `stream`, one kernel launch; the stored state is not modified.
+ * Semantics: the values are evaluated at the STORED state, i.e. what MuJoCo's arrays hold after set_state / reset + mj_forward.
+ * After a step, MuJoCo's arrays still hold the last substep's pre-integration kinematics (SURVEY F9); the query is one substep
+ * newer than those (the tcp pose of that stale kind is in the sensor record). */
+int ur3e_batch_query_create(ur3e_batch* b, const int32_t* objtype, const int32_t* objid, int32_t k);
+int ur3e_batch_query(ur3e_batch* b, int query_id, void* pos_dev, void* mat_dev, void* vel_dev, int flg_local, void* stream);
 
 #ifdef __cplusplus
 }

@@ -8,6 +8,7 @@ LIB_PATH = os.environ.get("UR3E_B200_LIB") or os.path.join(_HERE, "libur3e_b200.
 
 F32, F64 = 0, 1
 OBJ_BODY, OBJ_JOINT, OBJ_GEOM, OBJ_SITE, OBJ_TENDON, OBJ_ACTUATOR, OBJ_KEY = 1, 3, 5, 6, 18, 19, 23
+OBJ_XBODY = 2   # body frame (mjOBJ_XBODY), kinematics queries only
 CTRL_RAW, CTRL_PD_JOINT, CTRL_PID_TASK, CTRL_PID_TASK_ENV, CTRL_PINV = 0, 1, 2, 3, 4
 OBS_STATE, OBS_V2, OBS_V0, OBS_DIRECT = 0, 1, 2, 3
 REW_NONE, REW_V2, REW_V0, REW_MINUS1 = 0, 1, 2, 3
@@ -34,7 +35,8 @@ class EnvConfig(C.Structure):
 EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_model_info", "ur3e_model_name2id", "ur3e_model_id2name",
            "ur3e_model_array", "ur3e_model_num_warnings", "ur3e_model_warning", "ur3e_batch_create", "ur3e_batch_destroy", "ur3e_batch_reset",
            "ur3e_batch_step", "ur3e_batch_step_host", "ur3e_batch_get_state", "ur3e_batch_set_state", "ur3e_batch_stats", "ur3e_batch_set_sensor_buffer",
-           "ur3e_batch_debug_forward", "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info"]
+           "ur3e_batch_debug_forward", "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
+           "ur3e_batch_query_create", "ur3e_batch_query"]
 
 _lib = None
 
@@ -74,6 +76,8 @@ def load():
     L.ur3e_batch_mid_tier_info.argtypes = [vp] + [C.POINTER(C.c_int32)] * 3
     L.ur3e_batch_kernel_timing.argtypes = [vp, C.c_int]
     L.ur3e_batch_kernel_times.argtypes = [vp, dp]
+    L.ur3e_batch_query_create.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int32]
+    L.ur3e_batch_query.argtypes = [vp, C.c_int, vp, vp, vp, C.c_int, vp]
     _lib = L
     return L
 

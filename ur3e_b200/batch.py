@@ -125,6 +125,11 @@ class SimBatch:
         return dict(M=M, qfrc_bias=bias, qacc=qacc, qfrc_constraint=fc, ncon=int(info[0]), nefc=int(info[1]), solver_iter=int(info[2]),
                     overflow=int(info[3]), contacts=con[:int(info[0])], tcp_pos=cache[:3], tcp_mat=cache[3:12].reshape(3, 3), J_arm=cache[12:48].reshape(6, 6), bias_arm=cache[48:54])
 
+    def query(self, objects):
+        """A kinematics query over a fixed list of objects: [(kind, name_or_id), ...] with kind "body" (inertial frame, d.xipos /
+        d.ximat), "xbody" (body frame, d.xpos / d.xmat, what d.body(name).xpos returns), "geom" or "site".  See Query."""
+        return Query(self, objects)
+
     @property
     def launch_count(self):
         return int(self._L.ur3e_batch_launch_count(self.ptr))
@@ -165,3 +170,57 @@ class SimBatch:
             self.close()
         except Exception:
             pass
+
+
+class Query:
+    """Poses and velocities of k objects in every environment of a batch (ur3e_batch_query_create / ur3e_batch_query).
+
+    Calling it launches one kernel on the current torch stream and returns (pos [n, k, 3], mat [n, k, 3, 3], vel [n, k, 6]), None
+    for an output not asked for.  vel is mj_objectVelocity's [rot(3), lin(3)], in the object's frame when local=True.  Each output
+    argument is False, True (a tensor owned by the query, overwritten by its next call, like step's outputs) or a tensor of that
+    shape and the batch's dtype on its device to write into.
+
+    The values are evaluated at the stored state: what MuJoCo's d.xpos / d.site_xpos / ... hold after reset or set_state +
+    mj_forward.  After a step MuJoCo's arrays still hold the last substep's pre-integration kinematics (SURVEY F9); the query's
+    values are one substep newer than those.
+    """
+    KINDS = {"body": _lib.OBJ_BODY, "xbody": _lib.OBJ_XBODY, "geom": _lib.OBJ_GEOM, "site": _lib.OBJ_SITE}
+
+    def __init__(self, batch, objects):
+        self.batch = batch
+        types, ids = [], []
+        for kind, obj in objects:
+            if kind not in self.KINDS:
+                raise ValueError("object kind %r is not one of %s" % (kind, sorted(self.KINDS)))
+            if isinstance(obj, str):
+                i = batch.model.name2id(_lib.OBJ_BODY if kind == "xbody" else self.KINDS[kind], obj)
+                if i < 0:
+                    raise KeyError("%s %r is not in the model" % (kind, obj))
+                obj = i
+            types.append(self.KINDS[kind]); ids.append(int(obj))
+        self.k = len(types)
+        t = (C.c_int32 * max(self.k, 1))(*types); i = (C.c_int32 * max(self.k, 1))(*ids)
+        qid = batch._L.ur3e_batch_query_create(batch.ptr, t, i, self.k)
+        if qid < 0:
+            raise ValueError("ur3e_batch_query_create: " + _lib.last_error())
+        self.id = qid
+        self._own = {}
+
+    def _out(self, name, arg, shape):
+        if arg is False or arg is None:
+            return None
+        if arg is True:
+            if name not in self._own:
+                self._own[name] = torch.empty(shape, dtype=self.batch.dtype, device=self.batch.device)
+            return self._own[name]
+        self.batch._chk(arg, shape)
+        return arg
+
+    def __call__(self, pos=True, mat=False, vel=False, local=False):
+        n, k = self.batch.n, self.k
+        outs = (self._out("pos", pos, (n, k, 3)), self._out("mat", mat, (n, k, 3, 3)), self._out("vel", vel, (n, k, 6)))
+        if all(o is None for o in outs):
+            raise ValueError("a query needs at least one of pos, mat, vel")
+        p = [C.c_void_p(o.data_ptr()) if o is not None else None for o in outs]
+        _lib.check(self.batch._L.ur3e_batch_query(self.batch.ptr, self.id, p[0], p[1], p[2], int(bool(local)), self.batch._stream()), "ur3e_batch_query")
+        return outs

@@ -31,6 +31,9 @@ struct BatchBase {
   // optional CUDA-event timing of every step-kernel launch (bench.py's roofline: the duration of the dominant kernel alone)
   virtual int kernel_timing(int enable) = 0;
   virtual int kernel_times(double* out6) = 0;   // {ms, launches} x {lite tier, grasp / generic tier on the caller's stream, generic tier on the side stream}; synchronises
+  // kinematics queries (query.cuh): the batch owns the compiled object tables; query_create returns the query's id
+  virtual int query_create(const int32_t* objtype, const int32_t* objid, int k) = 0;
+  virtual int query(int id, void* pos, void* mat, void* vel, int local, cudaStream_t s) = 0;
   int64_t launches = 0;
   virtual void tier_steps(int64_t* lite, int64_t* full) const { *lite = 0; *full = 0; }
   virtual int64_t last_overflow() const { return 0; }

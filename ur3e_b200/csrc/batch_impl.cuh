@@ -11,6 +11,7 @@
 #include "compile_model.h"
 #include "merge_bodies.h"
 #include "env.cuh"
+#include "query.cuh"
 
 #ifndef UR3E_BLOCKS_PER_SM
 #define UR3E_BLOCKS_PER_SM 2
@@ -217,6 +218,35 @@ __global__ void stats_kernel(EnvState<Real, D>* st, long long n, double* out, in
   }
 }
 
+template <typename Real, typename D>
+struct QArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;
+  const QueryEntry<Real>* q; int k;
+  long long n;
+  Real *pos, *mat, *vel; int local;
+};
+
+// Kinematics queries (query.cuh): one warp per environment on the contact-free arena QueryDims<D>; reads qpos (and qvel when
+// velocities are wanted) of the record, writes [n, k, 3 | 9 | 6] outputs, never the record.
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) query_kernel(const QArgs<Real, D> a) {
+  using DK = QueryDims<D>;
+  constexpr int WPB = warps_per_block<Real, DK>();
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long e = (long long)blockIdx.x * WPB + warp;
+  if (e >= a.n) return;
+  Arena<Real, DK>& s = *reinterpret_cast<Arena<Real, DK>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, DK>());
+  const DevModel<Real>& m = *a.m;
+  const EnvState<Real, D>& rec = a.st[e];
+  WARP_FOR(i, m.nq) s.st.qpos[i] = rec.qpos[i];
+  if (a.vel) { WARP_FOR(i, m.nv) s.st.qvel[i] = rec.qvel[i]; }
+  WARP_SYNC();
+  const long long k = a.k;
+  query_env(m, s, a.q, a.k, a.pos ? a.pos + e * k * 3 : nullptr, a.mat ? a.mat + e * k * 9 : nullptr, a.vel ? a.vel + e * k * 6 : nullptr, a.local);
+}
+
 // D: generic size class of the model family; DL: lite twin (small caps, exact-fit) or D; DM: grasp-tier twin (caps between DL's and D's,
 // exact-fit) or D.  Tiers hand environments up through device-side lists: DL -> DM -> D.
 template <typename Real, typename D, typename DL = D, typename DM = D>
@@ -253,6 +283,7 @@ struct Batch : BatchBase {
     cudaFree(d_model); cudaFree(d_consts); cudaFree(d_state); cudaFree(d_act); cudaFree(d_obs); cudaFree(d_rew); cudaFree(d_term); cudaFree(d_trunc); cudaFree(d_dbg);
     for (auto& t : timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
     for (auto e : ev_pool) cudaEventDestroy(e);
+    for (auto& q : queries) cudaFree(q.table);
     if (own_stream) cudaStreamDestroy(own_stream);
     if (own_stream2) cudaStreamDestroy(own_stream2);
   }
@@ -535,6 +566,37 @@ struct Batch : BatchBase {
     }
     CUDA_OK(cudaStreamSynchronize(own_stream));
     CUDA_OK(cudaStreamSynchronize(own_stream2));
+    return 0;
+  }
+  // ---- kinematics queries (query.cuh); the tables live until the batch is destroyed
+  struct Query { QueryEntry<Real>* table; int k; };
+  std::vector<Query> queries;
+  int query_create(const int32_t* objtype, const int32_t* objid, int k) override {
+    CUDA_OK(cudaSetDevice(device));
+    std::vector<QueryEntry<Real>> tab;
+    const std::string err = compile_query<Real>(hm, objtype, objid, k, tab);
+    if (!err.empty()) return set_err("query_create: " + err);
+    if (queries.empty()) {
+      using DK = QueryDims<D>;
+      CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(arena_stride<Real, DK>() * warps_per_block<Real, DK>())));
+    }
+    Query q{nullptr, k};
+    CUDA_OK(cudaMalloc(&q.table, sizeof(QueryEntry<Real>) * k));
+    queries.push_back(q);
+    CUDA_OK(cudaMemcpy(q.table, tab.data(), sizeof(QueryEntry<Real>) * k, cudaMemcpyHostToDevice));
+    return (int)queries.size() - 1;
+  }
+  int query(int id, void* pos, void* mat, void* vel, int local, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    if (id < 0 || id >= (int)queries.size()) return set_err("query: unknown query id " + std::to_string(id));
+    if (!pos && !mat && !vel) return set_err("query: all outputs are null");
+    // a read-only call: last_stream (what step_host orders itself after) stays that of the latest state-changing call
+    using DK = QueryDims<D>;
+    constexpr int W = warps_per_block<Real, DK>();
+    QArgs<Real, D> a{d_model, d_state, queries[id].table, queries[id].k, n, (Real*)pos, (Real*)mat, (Real*)vel, local != 0};
+    query_kernel<Real, D><<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DK>() * W, s>>>(a);
+    ++launches;
+    CUDA_OK(cudaGetLastError());
     return 0;
   }
   int set_sensor_buffer(void* buf) override { sens_dev = buf; return 0; }

@@ -108,5 +108,12 @@ int ur3e_batch_mid_tier_info(const ur3e_batch* b, int32_t* arena_bytes, int32_t*
 int ur3e_batch_kernel_timing(ur3e_batch* b, int enable) { GUARD(b); return b->impl->kernel_timing(enable); }
 int ur3e_batch_kernel_times(ur3e_batch* b, double* out6) { GUARD(b); if (!out6) return set_err("null argument"); return b->impl->kernel_times(out6); }
 int ur3e_batch_state_bytes(const ur3e_batch* b) { return (b && b->impl) ? b->impl->state_bytes : -1; }
+int ur3e_batch_query_create(ur3e_batch* b, const int32_t* objtype, const int32_t* objid, int32_t k) {
+  GUARD(b);
+  try { return b->impl->query_create(objtype, objid, k); } catch (const std::exception& e) { return set_err(e.what()); }
+}
+int ur3e_batch_query(ur3e_batch* b, int query_id, void* pos, void* mat, void* vel, int flg_local, void* stream) {
+  GUARD(b); return b->impl->query(query_id, pos, mat, vel, flg_local, (cudaStream_t)stream);
+}
 
 }  // extern "C"

@@ -13,6 +13,23 @@
 The sensors are the ones of the step's last mj_step (MuJoCo fills d.sensordata in the forward pass, before integrating),
 so a call after `step` returns what the reference's loops log after `mj_step`.  Environments that were auto-reset in that
 step report the sensors of their terminal step.
+
+Poses and velocities of named objects (utils/utils.py:129-189, utils/gym_utils.py:20-39,207-219) take the reference's (m, d, name)
+signature; `m` is accepted for drop-in use and may be None.  They run a kinematics query (SimBatch.query) at the stored state:
+
+    get_site_xpos(m, d, "tcp")        # [N, 3]     d.site("tcp").xpos
+    get_site_xmat / get_site_R        # [N, 9] / [N, 3, 3]
+    get_site_xrotvec                  # [N, 3]     scipy Rotation.from_matrix(site_xmat).as_rotvec()
+    get_site_vel(m, d, "tcp")         # [N, 6]     mj_objectVelocity(mjOBJ_SITE, flg_local=0): [rot(3), lin(3)]
+    get_body_xpos / get_body_xmat     # [N, 3] / [N, 9]  d.body(name).xpos / .xmat (body frame)
+    get_geom_xpos / get_geom_xmat     # [N, 3] / [N, 9]
+    get_ghost_xpos(m, d)              # [N, 3]     body "ghost" (the v2 observation's target)
+    get_finger_jnt_disp / _vel(m, d)  # [N]        qpos[6] / qvel[6]
+
+These are MuJoCo's values after reset / set_state + mj_forward.  After a step MuJoCo's d.xpos etc. still hold the last substep's
+pre-integration kinematics (SURVEY F9) while these are one substep newer; the stale tcp pose is get_task_space_state's.  Every
+accessor reuses one cached query per (batch, kind, name): one kernel launch per call, and the returned tensor is overwritten by
+the next call of the same accessor.
 """
 import math
 
@@ -103,3 +120,69 @@ def get_joint_space_state(d):
     b = _batch(d)
     qpos, _, _ = b.get_state()
     return torch.cat([qpos[:, :6], get_boolean_grasp_contact(d).to(qpos.dtype)[:, None]], 1)
+
+
+def _query(d, kind, name):
+    b = _batch(d)
+    cache = b.__dict__.setdefault("_accessor_queries", {})
+    q = cache.get((kind, name))
+    if q is None:
+        q = cache[(kind, name)] = b.query([(kind, name)])
+    return q
+
+
+def _pos(d, kind, name):
+    return _query(d, kind, name)(pos=True)[0][:, 0]
+
+
+def _mat(d, kind, name):
+    return _query(d, kind, name)(pos=False, mat=True)[1][:, 0]
+
+
+def get_site_xpos(m, d, name):
+    return _pos(d, "site", name)
+
+
+def get_site_R(m, d, name):
+    return _mat(d, "site", name)
+
+
+def get_site_xmat(m, d, name):
+    return get_site_R(m, d, name).reshape(-1, 9)
+
+
+def get_site_xrotvec(m, d, name):
+    return _rotvec(get_site_R(m, d, name))
+
+
+def get_site_vel(m, d, name):
+    """mj_objectVelocity(mjOBJ_SITE, flg_local=0): [angular (3), linear (3)] in world axes."""
+    return _query(d, "site", name)(pos=False, vel=True)[2][:, 0]
+
+
+def get_body_xpos(m, d, name):
+    return _pos(d, "xbody", name)
+
+
+def get_body_xmat(m, d, name):
+    return _mat(d, "xbody", name).reshape(-1, 9)
+
+
+def get_geom_xpos(m, d, name):
+    return _pos(d, "geom", name)
+
+
+def get_geom_xmat(m, d, name):
+    return _mat(d, "geom", name).reshape(-1, 9)
+
+
+def get_ghost_xpos(m, d):
+    return get_body_xpos(m, d, "ghost")
+
+
+def get_finger_jnt_disp(m, d):
+    return _batch(d).get_state()[0][:, 6]
+
+
+def get_finger_jnt_vel(m, d):
+    return _batch(d).get_state()[1][:, 6]
