@@ -135,6 +135,17 @@ int ur3e_batch_state_bytes(const ur3e_batch* b);
  * newer than those (the tcp pose of that stale kind is in the sensor record). */
 int ur3e_batch_query_create(ur3e_batch* b, const int32_t* objtype, const int32_t* objid, int32_t k);
 int ur3e_batch_query(ur3e_batch* b, int query_id, void* pos_dev, void* mat_dev, void* vel_dev, int flg_local, void* stream);
+/* mj_jacSite / mj_jacBody / mj_jacBodyCom / mj_jacGeom for the k objects of a kinematics query, plus mj_fullM and d.qfrc_bias,
+ * for every environment, at the stored state.  jacp_dev, jacr_dev [n, k, 3, nv]; M_dev [n, nv, nv]; qfrc_bias_dev [n, nv]; batch dtype.
+ * query_id = -1: no objects (jacp_dev and jacr_dev must be NULL).  Any output may be NULL, not all.  One launch, asynchronous.
+ * The Jacobian of an object is taken at its world point: the site (UR3E_OBJ_SITE, mj_jacSite), the body frame's origin
+ * (UR3E_OBJ_XBODY, mj_jacBody), the body's centre of mass (UR3E_OBJ_BODY, mj_jacBodyCom) or the geom (UR3E_OBJ_GEOM, mj_jacGeom);
+ * jacp and jacr are MuJoCo's row-major (3, nv) per object.  M is dense and symmetric, armature included.  The stored state is not
+ * modified.
+ * Semantics: the values are evaluated at the STORED state, i.e. what MuJoCo's arrays hold after set_state / reset + mj_forward.
+ * After a step, MuJoCo's d.qfrc_bias and the Jacobian it would compute are the last substep's pre-integration values (SURVEY F9),
+ * and so is the cache the fused task-space controllers read; this call is one substep newer than those. */
+int ur3e_batch_query_jac(ur3e_batch* b, int query_id, void* jacp_dev, void* jacr_dev, void* M_dev, void* qfrc_bias_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -130,6 +130,22 @@ class SimBatch:
         d.ximat), "xbody" (body frame, d.xpos / d.xmat, what d.body(name).xpos returns), "geom" or "site".  See Query."""
         return Query(self, objects)
 
+    def mass_matrix(self, M=True, qfrc_bias=False):
+        """mj_fullM and d.qfrc_bias of every environment at the stored state: (M [n, nv, nv], qfrc_bias [n, nv]), None for an
+        output not asked for.  One launch on the current torch stream; the output convention and the semantics are Query.jac's
+        (this is Query.jac without objects)."""
+        nv = self.model.nv
+        own = self.__dict__.setdefault("_mass_own", {})
+        outs = (_out(self, own, "M", M, (self.n, nv, nv)), _out(self, own, "qfrc_bias", qfrc_bias, (self.n, nv)))
+        if all(o is None for o in outs):
+            raise ValueError("mass_matrix needs at least one of M, qfrc_bias")
+        self._query_jac(-1, (None, None) + outs)
+        return outs
+
+    def _query_jac(self, query_id, outs):
+        p = [C.c_void_p(o.data_ptr()) if o is not None else None for o in outs]
+        _lib.check(self._L.ur3e_batch_query_jac(self.ptr, query_id, p[0], p[1], p[2], p[3], self._stream()), "ur3e_batch_query_jac")
+
     @property
     def launch_count(self):
         return int(self._L.ur3e_batch_launch_count(self.ptr))
@@ -207,14 +223,7 @@ class Query:
         self._own = {}
 
     def _out(self, name, arg, shape):
-        if arg is False or arg is None:
-            return None
-        if arg is True:
-            if name not in self._own:
-                self._own[name] = torch.empty(shape, dtype=self.batch.dtype, device=self.batch.device)
-            return self._own[name]
-        self.batch._chk(arg, shape)
-        return arg
+        return _out(self.batch, self._own, name, arg, shape)
 
     def __call__(self, pos=True, mat=False, vel=False, local=False):
         n, k = self.batch.n, self.k
@@ -224,3 +233,37 @@ class Query:
         p = [C.c_void_p(o.data_ptr()) if o is not None else None for o in outs]
         _lib.check(self.batch._L.ur3e_batch_query(self.batch.ptr, self.id, p[0], p[1], p[2], int(bool(local)), self.batch._stream()), "ur3e_batch_query")
         return outs
+
+    def jac(self, jacp=True, jacr=False, M=False, qfrc_bias=False):
+        """Jacobians of the k objects, with the mass matrix and the bias forces (ur3e_batch_query_jac): one launch on the current
+        torch stream, returning (jacp [n, k, 3, nv], jacr [n, k, 3, nv], M [n, nv, nv], qfrc_bias [n, nv]), None for an output not
+        asked for.  Outputs follow __call__'s convention (False, True or a caller tensor).
+
+        jacp / jacr are MuJoCo's (3, nv) translational / rotational Jacobians per object, at the object's world point: mj_jacSite
+        for a "site", mj_jacBody for an "xbody" (the body frame's origin), mj_jacBodyCom for a "body" (its centre of mass),
+        mj_jacGeom for a "geom".  M is mj_fullM (dense, symmetric, armature included); qfrc_bias is d.qfrc_bias (Coriolis,
+        centrifugal and gravity forces).
+
+        The values are evaluated at the stored state: what MuJoCo holds after reset or set_state + mj_forward.  After a step
+        MuJoCo's d.qfrc_bias and the Jacobian it would compute are the last substep's pre-integration values (SURVEY F9), as is the
+        cache the fused task-space controllers read; these are one substep newer, the same state __call__ sees.
+        """
+        n, k, nv = self.batch.n, self.k, self.batch.model.nv
+        outs = (self._out("jacp", jacp, (n, k, 3, nv)), self._out("jacr", jacr, (n, k, 3, nv)), self._out("M", M, (n, nv, nv)),
+                self._out("qfrc_bias", qfrc_bias, (n, nv)))
+        if all(o is None for o in outs):
+            raise ValueError("Query.jac needs at least one of jacp, jacr, M, qfrc_bias")
+        self.batch._query_jac(self.id, outs)
+        return outs
+
+
+def _out(batch, own, name, arg, shape):
+    """An output argument: False / None (not wanted), True (a tensor kept in `own`, overwritten by the next call) or a caller tensor."""
+    if arg is False or arg is None:
+        return None
+    if arg is True:
+        if name not in own:
+            own[name] = torch.empty(shape, dtype=batch.dtype, device=batch.device)
+        return own[name]
+    batch._chk(arg, shape)
+    return arg

@@ -34,6 +34,8 @@ struct BatchBase {
   // kinematics queries (query.cuh): the batch owns the compiled object tables; query_create returns the query's id
   virtual int query_create(const int32_t* objtype, const int32_t* objid, int k) = 0;
   virtual int query(int id, void* pos, void* mat, void* vel, int local, cudaStream_t s) = 0;
+  // Jacobians of a query's objects, mass matrix and bias forces (query.cuh query_jac_env); id = -1: no objects
+  virtual int query_jac(int id, void* jacp, void* jacr, void* M, void* bias, cudaStream_t s) = 0;
   int64_t launches = 0;
   virtual void tier_steps(int64_t* lite, int64_t* full) const { *lite = 0; *full = 0; }
   virtual int64_t last_overflow() const { return 0; }

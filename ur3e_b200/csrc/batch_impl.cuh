@@ -247,6 +247,36 @@ __global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) qu
   query_env(m, s, a.q, a.k, a.pos ? a.pos + e * k * 3 : nullptr, a.mat ? a.mat + e * k * 9 : nullptr, a.vel ? a.vel + e * k * 6 : nullptr, a.local);
 }
 
+template <typename Real, typename D>
+struct QJArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;
+  const QueryEntry<Real>* q; int k;   // k = 0 (q null): no objects, M / qfrc_bias only
+  long long n;
+  Real *jacp, *jacr, *M, *bias;
+};
+
+// Jacobians, mass matrix and bias forces (query.cuh query_jac_env): one warp per environment on the same arena as query_kernel;
+// reads qpos (and qvel when M or qfrc_bias is wanted) of the record, writes [n, k, 3, nv] / [n, nv, nv] / [n, nv], never the record.
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) query_jac_kernel(const QJArgs<Real, D> a) {
+  using DK = QueryDims<D>;
+  constexpr int WPB = warps_per_block<Real, DK>();
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long e = (long long)blockIdx.x * WPB + warp;
+  if (e >= a.n) return;
+  Arena<Real, DK>& s = *reinterpret_cast<Arena<Real, DK>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, DK>());
+  const DevModel<Real>& m = *a.m;
+  const EnvState<Real, D>& rec = a.st[e];
+  WARP_FOR(i, m.nq) s.st.qpos[i] = rec.qpos[i];
+  if (a.M || a.bias) { WARP_FOR(i, m.nv) s.st.qvel[i] = rec.qvel[i]; }
+  WARP_SYNC();
+  const long long nv = m.nv, kj = (long long)a.k * 3 * nv;
+  query_jac_env(m, s, a.q, a.k, a.jacp ? a.jacp + e * kj : nullptr, a.jacr ? a.jacr + e * kj : nullptr, a.M ? a.M + e * nv * nv : nullptr,
+                a.bias ? a.bias + e * nv : nullptr);
+}
+
 // D: generic size class of the model family; DL: lite twin (small caps, exact-fit) or D; DM: grasp-tier twin (caps between DL's and D's,
 // exact-fit) or D.  Tiers hand environments up through device-side lists: DL -> DM -> D.
 template <typename Real, typename D, typename DL = D, typename DM = D>
@@ -595,6 +625,24 @@ struct Batch : BatchBase {
     constexpr int W = warps_per_block<Real, DK>();
     QArgs<Real, D> a{d_model, d_state, queries[id].table, queries[id].k, n, (Real*)pos, (Real*)mat, (Real*)vel, local != 0};
     query_kernel<Real, D><<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DK>() * W, s>>>(a);
+    ++launches;
+    CUDA_OK(cudaGetLastError());
+    return 0;
+  }
+  bool jac_ready = false;   // query_jac_kernel's shared-memory attribute is set
+  int query_jac(int id, void* jacp, void* jacr, void* M, void* bias, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const std::string err = query_jac_check(id, (int)queries.size(), jacp || jacr, jacp || jacr || M || bias);
+    if (!err.empty()) return set_err("query_jac: " + err);
+    using DK = QueryDims<D>;
+    constexpr int W = warps_per_block<Real, DK>();
+    if (!jac_ready) {
+      CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(arena_stride<Real, DK>() * W)));
+      jac_ready = true;
+    }
+    // read-only, like query(): last_stream stays that of the latest state-changing call
+    QJArgs<Real, D> a{d_model, d_state, id >= 0 ? queries[id].table : nullptr, id >= 0 ? queries[id].k : 0, n, (Real*)jacp, (Real*)jacr, (Real*)M, (Real*)bias};
+    query_jac_kernel<Real, D><<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DK>() * W, s>>>(a);
     ++launches;
     CUDA_OK(cudaGetLastError());
     return 0;

@@ -115,5 +115,8 @@ int ur3e_batch_query_create(ur3e_batch* b, const int32_t* objtype, const int32_t
 int ur3e_batch_query(ur3e_batch* b, int query_id, void* pos, void* mat, void* vel, int flg_local, void* stream) {
   GUARD(b); return b->impl->query(query_id, pos, mat, vel, flg_local, (cudaStream_t)stream);
 }
+int ur3e_batch_query_jac(ur3e_batch* b, int query_id, void* jacp, void* jacr, void* M, void* qfrc_bias, void* stream) {
+  GUARD(b); return b->impl->query_jac(query_id, jacp, jacr, M, qfrc_bias, (cudaStream_t)stream);
+}
 
 }  // extern "C"

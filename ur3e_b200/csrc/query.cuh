@@ -1,10 +1,11 @@
 // Kinematics queries: poses and velocities of a fixed list of objects (query_model.h) for one environment, evaluated at its
-// stored state.  Read-only: the caller loads qpos (and qvel when velocities are wanted) into the arena's record copy; nothing is
-// written back.  Like engine.cuh this file uses only warp_model.cuh constructs, so tests/hostcheck compiles it for the CPU.
+// stored state, and their Jacobians with the mass matrix and the bias forces.  Read-only: the caller loads qpos (and qvel when
+// velocities or dynamics are wanted) into the arena's record copy; nothing is written back.  Like engine.cuh this file uses only
+// warp_model.cuh constructs, so tests/hostcheck compiles it for the CPU.
 //
-// Semantics: MuJoCo's d.xpos / d.xipos / d.geom_xpos / d.site_xpos (and xmat) and mj_objectVelocity after mj_forward at
-// (qpos, qvel), i.e. after reset / set_state.  After mj_step MuJoCo's arrays still hold the last substep's pre-integration
-// kinematics (SURVEY F9); a query after a step is one substep newer than those.
+// Semantics: MuJoCo's d.xpos / d.xipos / d.geom_xpos / d.site_xpos (and xmat), mj_objectVelocity, mj_jac*, mj_fullM and
+// d.qfrc_bias after mj_forward at (qpos, qvel), i.e. after reset / set_state.  After mj_step MuJoCo's arrays still hold the last
+// substep's pre-integration values (SURVEY F9); a query after a step is one substep newer than those.
 #pragma once
 #include "engine.cuh"
 #include "query_model.h"
@@ -75,6 +76,54 @@ UR3E_HD void query_env(const DevModel<Real>& m, Arena<Real, D>& s, const QueryEn
       }
     }
   }
+}
+
+// Arguments of a Jacobian / mass-matrix call (ur3e_batch_query_jac): query `id` of `nquery` compiled ones, or -1 for none, with
+// `jac` = jacp or jacr requested and `any` = some output requested.  Returns "" when valid, else the reason the call is rejected.
+inline std::string query_jac_check(int id, int nquery, bool jac, bool any) {
+  if (id < -1 || id >= nquery) return "unknown query id " + std::to_string(id);
+  if (!any) return "all outputs are null";
+  if (id == -1 && jac) return "jacp / jacr need a query's objects (query_id = -1 has none)";
+  return "";
+}
+
+// mj_jacSite / mj_jacBody / mj_jacBodyCom / mj_jacGeom of the k objects, at each object's world point xpos[a] + R_a lpos (the
+// site, body frame, inertial frame or geom of query_model.h's entry): jacp, jacr [k][3][nv] (MuJoCo's row-major (3, nv) per
+// object); mj_fullM: M [nv][nv], dense and symmetric; d.qfrc_bias [nv].  Any output may be null; q may be null when k = 0.  The
+// caller loads qpos, and qvel when M or qfrc_bias is wanted.  M and qfrc_bias are the step's own dynamics() (CRBA with armature,
+// RNE); that pass also forms the actuator forces, so ctrl is zeroed first rather than left as uninitialised shared memory.
+template <typename Real, typename D>
+UR3E_HD void query_jac_env(const DevModel<Real>& m, Arena<Real, D>& s, const QueryEntry<Real>* q, int k, Real* jacp, Real* jacr, Real* M, Real* bias) {
+  kinematics(m, s);
+  if (M || bias) {
+    WARP_FOR(a, nu_<D>(m)) s.ctrl[a] = 0;
+    WARP_SYNC();
+    dynamics(m, s);
+  }
+  const int nv = nv_<D>(m);
+  if (jacp || jacr) {
+    const auto& xmat = s.fr.k.xmat;
+    const int per = 3 * nv;
+    WARP_FOR(i, k * per) {
+      const int j = i / per, e = i - per * j, r = e / nv, d = e - nv * r;
+      const QueryEntry<Real>& o = q[j];
+      if (jacp) {
+        Real v[3], p[3], col[3];
+        mat_vec3(v, xmat[o.body], o.lpos);
+        for (int c = 0; c < 3; ++c) p[c] = s.xpos[o.body][c] + v[c];
+        jac_col(m, s, d, p, o.body, col);
+        jacp[i] = r == 0 ? col[0] : (r == 1 ? col[1] : col[2]);   // selects, not a dynamically indexed (local-memory) array
+      }
+      if (jacr) jacr[i] = ((m.body_dofmask[o.body] >> d) & 1u) ? s.cdof[d][r] : Real(0);
+    }
+  }
+  if (M) {
+    WARP_FOR(i, nv * nv) {
+      const int r = i / nv, c = i - nv * r, hi = r > c ? r : c, lo = r > c ? c : r;
+      M[i] = s.M[hi * (hi + 1) / 2 + lo];
+    }
+  }
+  if (bias) { WARP_FOR(i, nv) bias[i] = s.qfrc_bias[i]; }
 }
 
 }  // namespace ur3e

@@ -30,6 +30,17 @@ These are MuJoCo's values after reset / set_state + mj_forward.  After a step Mu
 pre-integration kinematics (SURVEY F9) while these are one substep newer; the stale tcp pose is get_task_space_state's.  Every
 accessor reuses one cached query per (batch, kind, name): one kernel launch per call, and the returned tensor is overwritten by
 the next call of the same accessor.
+
+Jacobians, the mass matrix and the bias forces (controller_func.py:87-104, move_l.py:46-47,69-70) run Query.jac /
+SimBatch.mass_matrix at the same stored state, one launch per call:
+
+    mj_jacSite(m, d, jacp, jacr, site)    # writes jacp, jacr: caller tensors [N, 3, nv] or None; site an id or a name
+    mj_jacBody / mj_jacBodyCom / mj_jacGeom(m, d, jacp, jacr, obj)   # body frame / centre of mass / geom
+    get_full_M(m, d)                      # [N, nv, nv]  mj_fullM(m, M, d.qM)
+    get_qfrc_bias(m, d)                   # [N, nv]      d.qfrc_bias
+
+After a step MuJoCo's d.qfrc_bias and the Jacobian it would compute belong to the last substep's pre-integration state (SURVEY F9);
+these are one substep newer, the same state as the pose accessors above.
 """
 import math
 
@@ -186,3 +197,45 @@ def get_finger_jnt_disp(m, d):
 
 def get_finger_jnt_vel(m, d):
     return _batch(d).get_state()[1][:, 6]
+
+
+def _jac(d, kind, obj, jacp, jacr):
+    """MuJoCo's mj_jac* calling convention: writes into jacp / jacr ([N, 3, nv] tensors, either may be None), returns nothing."""
+    if jacp is None and jacr is None:
+        return
+    b = _batch(d)
+    nv = b.model.nv
+    outs = []
+    for t in (jacp, jacr):
+        if t is None:
+            outs.append(False)
+        else:
+            b._chk(t, (b.n, 3, nv))
+            outs.append(t.view(b.n, 1, 3, nv))   # the query's [N, k = 1, 3, nv] layout, same memory
+    _query(d, kind, obj).jac(jacp=outs[0], jacr=outs[1])
+
+
+def mj_jacSite(m, d, jacp, jacr, site):
+    _jac(d, "site", site, jacp, jacr)
+
+
+def mj_jacBody(m, d, jacp, jacr, body):
+    """Jacobian of the body frame's origin (d.xpos[body])."""
+    _jac(d, "xbody", body, jacp, jacr)
+
+
+def mj_jacBodyCom(m, d, jacp, jacr, body):
+    """Jacobian of the body's centre of mass (d.xipos[body])."""
+    _jac(d, "body", body, jacp, jacr)
+
+
+def mj_jacGeom(m, d, jacp, jacr, geom):
+    _jac(d, "geom", geom, jacp, jacr)
+
+
+def get_full_M(m, d):
+    return _batch(d).mass_matrix(M=True)[0]
+
+
+def get_qfrc_bias(m, d):
+    return _batch(d).mass_matrix(M=False, qfrc_bias=True)[1]
