@@ -146,6 +146,37 @@ int ur3e_batch_query(ur3e_batch* b, int query_id, void* pos_dev, void* mat_dev, 
  * After a step, MuJoCo's d.qfrc_bias and the Jacobian it would compute are the last substep's pre-integration values (SURVEY F9),
  * and so is the cache the fused task-space controllers read; this call is one substep newer than those. */
 int ur3e_batch_query_jac(ur3e_batch* b, int query_id, void* jacp_dev, void* jacr_dev, void* M_dev, void* qfrc_bias_dev, void* stream);
+/* Forward-dynamics queries: d.ncon, d.contact[k].geom1/geom2/dist/pos/frame, mj_contactForce, d.qacc, d.qfrc_constraint and
+ * d.sensordata for every environment (the contact reads of utils/gym_utils.py:98-201 get_robust_block_grasp_state,
+ * get_block_grasp_state, get_self_collision, get_table_collision; the sensor reads of utils/utils.py:201-245).
+ * C = ur3e_batch_max_contacts(b): contacts stored per environment, the step's largest cap (24 for main.xml, 12 for ur3e_2f85.xml, 0
+ * for a model without contact pairs).  Device outputs, any may be NULL, not all; float ones in the batch's dtype:
+ *   qacc, qfrc_constraint [n, nv]
+ *   info [n, 4] int32: ncon, nefc, solver iterations, overflow bits (1: more contacts / narrow-phase candidates than the caps,
+ *        2: more constraint rows than the cap; the bits the step sets)
+ *   contact_geom [n, C, 2] int32: geom1, geom2 (ids of the loaded model); contact_dist [n, C]; contact_pos [n, C, 3];
+ *   contact_frame [n, C, 9]: MuJoCo's mjContact fields; row 0 of the frame is the normal, from geom1 to geom2
+ *   contact_force [n, C, 6]: mj_contactForce in the contact frame, [fn, ft1, ft2, 0, 0, 0] (elliptic cones, condim 3); a contact
+ *        without constraint rows (row overflow) reports 0
+ *   flags [n] int32: 1 mug - left pad, 2 mug - right pad, 4 gripper - table, 8 self-collision (gym_utils.py:108-201), over all
+ *        ncon contacts (the list MuJoCo's d.contact holds); on a row overflow the step's own bits see only the contacts with rows
+ *   sensordata [n, 46]: the layout of the step's sensor record (ur3e_batch_set_sensor_buffer)
+ * Entries past ncon are written as geom -1 and zeros.  Contacts are in pair-list order (the candidate pairs of the model that survive
+ * the static pruning), then in the narrow phase's point order within a pair.
+ * ctrl_dev: contiguous [n, nu] (batch dtype; environment e at ctrl_dev + e * nu) or NULL (zero ctrl), the actuation the dynamics see.  When no output needs dynamics (qacc,
+ * qfrc_constraint, contact_force, sensordata) only kinematics and collision run: info then reports nefc = 0 and 0 iterations.
+ * Rejected: out NULL, every output NULL, a contact_* output when C = 0.  Asynchronous on `stream`, one kernel launch; the stored
+ * state is not modified.
+ * Semantics: the values are mj_forward's at the STORED state (qpos, qvel and the solver's warm start) with this ctrl, i.e. MuJoCo's
+ * d.contact / d.efc_force / d.qacc / d.sensordata after set_state / reset + mj_forward.  After a step, MuJoCo's d.contact still holds
+ * the contacts of the last substep before integration (SURVEY F9); this call is one substep newer, the state ur3e_batch_query sees. */
+typedef struct ur3e_forward_out {
+  void* qacc; void* qfrc_constraint; int32_t* info;
+  int32_t* contact_geom; void* contact_dist; void* contact_pos; void* contact_frame; void* contact_force;
+  int32_t* flags; void* sensordata;
+} ur3e_forward_out;
+int ur3e_batch_max_contacts(const ur3e_batch* b);
+int ur3e_batch_forward(ur3e_batch* b, const void* ctrl_dev, const ur3e_forward_out* out, void* stream);
 
 #ifdef __cplusplus
 }

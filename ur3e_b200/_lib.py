@@ -19,6 +19,7 @@ STAT_NAMES = ["episodes", "return_sum", "length_sum", "successes", "term_reach",
 MAXCON = 32
 CACHE_SIZE = 54
 NSENSOR = 46
+SENSOR_NCTRL = 7   # d.ctrl columns of the sensor record, [21, 28), zero past nu (utils.get_ctrl)
 
 
 class ModelDims(C.Structure):
@@ -32,11 +33,19 @@ class EnvConfig(C.Structure):
         ("single_tier", C.c_int32), ("lite_max_contacts", C.c_int32), ("lite_max_rows", C.c_int32), ("reserved_", C.c_int32)]
 
 
+# ur3e_forward_out: the ten device pointers of ur3e_batch_forward, in this order (FORWARD_OUTPUTS)
+FORWARD_OUTPUTS = ("qacc", "qfrc_constraint", "info", "contact_geom", "contact_dist", "contact_pos", "contact_frame", "contact_force", "flags", "sensordata")
+
+
+class ForwardOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in FORWARD_OUTPUTS]
+
+
 EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_model_info", "ur3e_model_name2id", "ur3e_model_id2name",
            "ur3e_model_array", "ur3e_model_num_warnings", "ur3e_model_warning", "ur3e_batch_create", "ur3e_batch_destroy", "ur3e_batch_reset",
            "ur3e_batch_step", "ur3e_batch_step_host", "ur3e_batch_get_state", "ur3e_batch_set_state", "ur3e_batch_stats", "ur3e_batch_set_sensor_buffer",
            "ur3e_batch_debug_forward", "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
-           "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac"]
+           "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward"]
 
 _lib = None
 
@@ -79,6 +88,8 @@ def load():
     L.ur3e_batch_query_create.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int32]
     L.ur3e_batch_query.argtypes = [vp, C.c_int, vp, vp, vp, C.c_int, vp]
     L.ur3e_batch_query_jac.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp]
+    L.ur3e_batch_max_contacts.argtypes = [vp]
+    L.ur3e_batch_forward.argtypes = [vp, vp, C.POINTER(ForwardOut), vp]
     _lib = L
     return L
 

@@ -4,6 +4,7 @@ Thin torch front-end over the C ABI (include/ur3e_b200.h): tensors are passed by
 torch supplies device memory and streams only.  dtype float32 = production, float64 = validation build.
 """
 import ctypes as C
+from collections import namedtuple
 
 import numpy as np
 import torch
@@ -30,6 +31,9 @@ def env_config(**kw):
     for i in range(3):
         c.tool_rotvec[i] = rotvec[i]
     return c
+
+
+ForwardResult = namedtuple("ForwardResult", _lib.FORWARD_OUTPUTS)
 
 
 class SimBatch:
@@ -147,6 +151,66 @@ class SimBatch:
         _lib.check(self._L.ur3e_batch_query_jac(self.ptr, query_id, p[0], p[1], p[2], p[3], self._stream()), "ur3e_batch_query_jac")
 
     @property
+    def max_contacts(self):
+        """C: contacts stored per environment by the step's largest size class and by forward() (24 for main.xml, 12 for
+        ur3e_2f85.xml, 0 for a model without contact pairs)."""
+        return int(self._L.ur3e_batch_max_contacts(self.ptr))
+
+    def forward(self, ctrl=None, qacc=True, qfrc_constraint=False, info=False, contact_geom=False, contact_dist=False, contact_pos=False,
+                contact_frame=False, contact_force=False, flags=False, sensordata=False):
+        """One mj_forward per environment at the stored state (ur3e_batch_forward): one launch on the current torch stream,
+        returning a ForwardResult named tuple with None for every output not asked for.  Each output argument is False, True (a
+        tensor owned by the batch, overwritten by the next call) or a tensor of its shape to write into; the integer outputs are
+        int32, the others in the batch's dtype.  C = max_contacts.
+
+            qacc, qfrc_constraint [n, nv]      d.qacc, d.qfrc_constraint
+            info [n, 4] int32                  ncon, nefc, solver iterations, overflow bits (1 contacts, 2 constraint rows)
+            contact_geom [n, C, 2] int32       d.contact[k].geom1 / geom2 (ids of the loaded model), -1 past ncon
+            contact_dist [n, C], contact_pos [n, C, 3], contact_frame [n, C, 3, 3]   d.contact[k].dist / pos / frame (row 0: the
+                                               normal, from geom1 to geom2)
+            contact_force [n, C, 6]            mj_contactForce: [fn, ft1, ft2, 0, 0, 0] in the contact frame
+            flags [n] int32                    1 mug - left pad, 2 mug - right pad, 4 gripper - table, 8 self-collision, over
+                                               all ncon contacts (on a row overflow the step's bits see only those with rows)
+            sensordata [n, 46]                 the layout of the step's sensor record (enable_sensors)
+
+        Entries past ncon are geom -1 and zeros.  Contacts are in pair-list order, then in the narrow phase's point order within a pair.
+        ctrl [n, nu] (batch dtype, any strides: a strided tensor is copied) is the actuation the dynamics see; None means zero.  The
+        [n, 7] d.ctrl block of the sensor record is accepted as it is (its columns past nu are zero), so passing
+        ur3e_b200.utils.get_ctrl(self) (with sensors enabled) applies the actuation of the last step.  When only contact geometry, info or flags are asked for, the
+        kernel runs kinematics and collision alone: info then reports nefc = 0 and 0 iterations.
+
+        The values are mj_forward's at the stored state (qpos, qvel and the solver's warm start), i.e. MuJoCo's d.contact,
+        d.efc_force, d.qacc and d.sensordata after reset or set_state.  After a step MuJoCo's d.contact still holds the contacts of
+        the last substep before integration (SURVEY F9); these are one substep newer, the state query() sees.
+        """
+        n, nv, Cn = self.n, self.model.nv, self.max_contacts
+        own = self.__dict__.setdefault("_forward_own", {})
+        i32 = torch.int32
+        spec = dict(qacc=((n, nv), None), qfrc_constraint=((n, nv), None), info=((n, 4), i32), contact_geom=((n, Cn, 2), i32),
+                    contact_dist=((n, Cn), None), contact_pos=((n, Cn, 3), None), contact_frame=((n, Cn, 3, 3), None),
+                    contact_force=((n, Cn, 6), None), flags=((n,), i32), sensordata=((n, _lib.NSENSOR), None))
+        args = dict(qacc=qacc, qfrc_constraint=qfrc_constraint, info=info, contact_geom=contact_geom, contact_dist=contact_dist,
+                    contact_pos=contact_pos, contact_frame=contact_frame, contact_force=contact_force, flags=flags, sensordata=sensordata)
+        if Cn == 0:
+            asked = [k for k in args if k.startswith("contact_") and args[k] is not False and args[k] is not None]
+            if asked:
+                raise ValueError("%s: the model has no contact pairs (max_contacts = 0)" % ", ".join(asked))
+        outs = ForwardResult(*[_out(self, own, k, args[k], *spec[k]) for k in _lib.FORWARD_OUTPUTS])
+        if all(o is None for o in outs):
+            raise ValueError("forward needs at least one output")
+        u = None
+        if ctrl is not None:
+            nu = self.model.nu
+            if tuple(ctrl.shape) == (n, _lib.SENSOR_NCTRL) and nu < _lib.SENSOR_NCTRL:
+                ctrl = ctrl[:, :nu]   # utils.get_ctrl's width: the record pads d.ctrl with zeros past nu
+            # the kernel reads ctrl + e * nu: a strided view (get_ctrl's rows are NSENSOR apart) is copied, on the current stream
+            ctrl = ctrl.contiguous()
+            u = self._chk(ctrl, (n, nu))
+        st = _lib.ForwardOut(*[o.data_ptr() if o is not None else None for o in outs])
+        _lib.check(self._L.ur3e_batch_forward(self.ptr, u, C.byref(st), self._stream()), "ur3e_batch_forward")
+        return outs
+
+    @property
     def launch_count(self):
         return int(self._L.ur3e_batch_launch_count(self.ptr))
 
@@ -257,13 +321,14 @@ class Query:
         return outs
 
 
-def _out(batch, own, name, arg, shape):
-    """An output argument: False / None (not wanted), True (a tensor kept in `own`, overwritten by the next call) or a caller tensor."""
+def _out(batch, own, name, arg, shape, dtype=None):
+    """An output argument: False / None (not wanted), True (a tensor kept in `own`, overwritten by the next call) or a caller tensor.
+    dtype: the output's element type (default: the batch's)."""
     if arg is False or arg is None:
         return None
     if arg is True:
         if name not in own:
-            own[name] = torch.empty(shape, dtype=batch.dtype, device=batch.device)
+            own[name] = torch.empty(shape, dtype=dtype or batch.dtype, device=batch.device)
         return own[name]
-    batch._chk(arg, shape)
+    batch._chk(arg, shape, dtype)
     return arg

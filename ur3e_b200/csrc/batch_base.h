@@ -36,6 +36,9 @@ struct BatchBase {
   virtual int query(int id, void* pos, void* mat, void* vel, int local, cudaStream_t s) = 0;
   // Jacobians of a query's objects, mass matrix and bias forces (query.cuh query_jac_env); id = -1: no objects
   virtual int query_jac(int id, void* jacp, void* jacr, void* M, void* bias, cudaStream_t s) = 0;
+  // one mj_forward per environment at the stored state: contacts, contact forces, qacc, sensordata (query_fwd.cuh forward_query_env)
+  virtual int max_contacts() const = 0;
+  virtual int forward(const void* ctrl, const ur3e_forward_out* out, cudaStream_t s) = 0;
   int64_t launches = 0;
   virtual void tier_steps(int64_t* lite, int64_t* full) const { *lite = 0; *full = 0; }
   virtual int64_t last_overflow() const { return 0; }

@@ -12,6 +12,7 @@
 #include "merge_bodies.h"
 #include "env.cuh"
 #include "query.cuh"
+#include "query_fwd.cuh"
 
 #ifndef UR3E_BLOCKS_PER_SM
 #define UR3E_BLOCKS_PER_SM 2
@@ -277,6 +278,47 @@ __global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) qu
                 a.bias ? a.bias + e * nv : nullptr);
 }
 
+template <typename Real, typename D>
+struct QFArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;
+  SolverOpts<Real> opt;   // the step's own solver options
+  long long n;
+  const Real* ctrl;       // [n, nu] or null (zero)
+  FwdOut<Real> o;         // batch-wide outputs: environment e's start at e times each output's per-environment size
+};
+
+// Forward-dynamics queries (query_fwd.cuh forward_query_env): one warp per environment on the generic size class's own arena, so the
+// contact and row caps are the step's largest; reads the whole record (the solver warm-starts from qacc_ws), never writes it.
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, D>() * 32, 1) query_fwd_kernel(const QFArgs<Real, D> a) {
+  constexpr int WPB = warps_per_block<Real, D>();
+  constexpr long long C = D::HAS_CONTACT ? D::MAXCON : 0;
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long e = (long long)blockIdx.x * WPB + warp;
+  if (e >= a.n) return;
+  Arena<Real, D>& s = *reinterpret_cast<Arena<Real, D>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, D>());
+  const DevModel<Real>& m = *a.m;
+  constexpr int NW = sizeof(EnvState<Real, D>) / 16;
+  const int4* gst = reinterpret_cast<const int4*>(a.st + e);
+  int4* sst = reinterpret_cast<int4*>(&s.st);
+  WARP_FOR(i, NW) sst[i] = gst[i];
+  const long long nv = m.nv;
+  FwdOut<Real> o;
+  o.qacc = a.o.qacc ? a.o.qacc + e * nv : nullptr;
+  o.qfrc_constraint = a.o.qfrc_constraint ? a.o.qfrc_constraint + e * nv : nullptr;
+  o.info = a.o.info ? a.o.info + e * 4 : nullptr;
+  o.contact_geom = a.o.contact_geom ? a.o.contact_geom + e * C * 2 : nullptr;
+  o.contact_dist = a.o.contact_dist ? a.o.contact_dist + e * C : nullptr;
+  o.contact_pos = a.o.contact_pos ? a.o.contact_pos + e * C * 3 : nullptr;
+  o.contact_frame = a.o.contact_frame ? a.o.contact_frame + e * C * 9 : nullptr;
+  o.contact_force = a.o.contact_force ? a.o.contact_force + e * C * 6 : nullptr;
+  o.flags = a.o.flags ? a.o.flags + e : nullptr;
+  o.sensordata = a.o.sensordata ? a.o.sensordata + e * NSENSOR : nullptr;
+  forward_query_env(m, s, a.opt, a.ctrl ? a.ctrl + e * m.nu : nullptr, o);
+}
+
 // D: generic size class of the model family; DL: lite twin (small caps, exact-fit) or D; DM: grasp-tier twin (caps between DL's and D's,
 // exact-fit) or D.  Tiers hand environments up through device-side lists: DL -> DM -> D.
 template <typename Real, typename D, typename DL = D, typename DM = D>
@@ -336,23 +378,7 @@ struct Batch : BatchBase {
     if (m.ngeom > D::NG || m.npair > D::NPAIR || m.nv > D::NV || m.nq > D::NQ || m.nu > D::NU) return set_err("model exceeds the kernel size class (geoms / pairs / dofs)");
     if (m.ndeq > 3 * D::MAXCONNECT) return set_err("model has more connect equalities than the kernel size class stores rows for");
     auto body = [&](const char* nm) { int b = h.name2id(OBJ_BODY, nm); return b >= 0 ? bmap[b] : -1; };
-    {  // the contact predicates of utils/gym_utils.py name bodies of the loaded model: classify every collidable geom by them
-      const auto& par = h.I("body_parentid"); const auto& gbid = h.I("geom_bodyid");
-      auto under = [&](int b, int root) { if (root < 0) return false; for (int a = b; a > 0; a = par[a]) if (a == root) return true; return false; };
-      const int arm = h.name2id(OBJ_BODY, "robot_base"), grip = h.name2id(OBJ_BODY, "robotiq_base_mount"), table = h.name2id(OBJ_BODY, "table"),
-                mug = h.name2id(OBJ_BODY, "fish"), lpad = h.name2id(OBJ_BODY, "left_pad"), rpad = h.name2id(OBJ_BODY, "right_pad");
-      for (int i = 0; i < m.ngeom; ++i) {
-        const int b = gbid[m.geom_src[i]];
-        int f = 0;
-        if (under(b, arm)) f |= GF_ARM;
-        if (under(b, grip)) f |= GF_GRIPPER;
-        if (b == table && table >= 0) f |= GF_TABLE;
-        if (b == mug && mug >= 0) f |= GF_MUG;
-        if (b == lpad && lpad >= 0) f |= GF_LPAD;
-        if (b == rpad && rpad >= 0) f |= GF_RPAD;
-        m.geom_flags[i] = f;
-      }
-    }
+    set_geom_flags(h, m);
     CUDA_OK(cudaMalloc(&d_model, sizeof m)); CUDA_OK(cudaMemcpy(d_model, &m, sizeof m, cudaMemcpyHostToDevice));
     CUDA_OK(cudaMalloc(&d_state, sizeof(EnvState<Real, D>) * n_envs)); CUDA_OK(cudaMemset(d_state, 0, sizeof(EnvState<Real, D>) * n_envs));
     std::memset(&base, 0, sizeof base);
@@ -643,6 +669,29 @@ struct Batch : BatchBase {
     // read-only, like query(): last_stream stays that of the latest state-changing call
     QJArgs<Real, D> a{d_model, d_state, id >= 0 ? queries[id].table : nullptr, id >= 0 ? queries[id].k : 0, n, (Real*)jacp, (Real*)jacr, (Real*)M, (Real*)bias};
     query_jac_kernel<Real, D><<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DK>() * W, s>>>(a);
+    ++launches;
+    CUDA_OK(cudaGetLastError());
+    return 0;
+  }
+  static constexpr int NCMAX = D::HAS_CONTACT ? D::MAXCON : 0;
+  int max_contacts() const override { return NCMAX; }
+  bool fwd_ready = false;   // query_fwd_kernel's shared-memory attribute is set
+  int forward(const void* ctrl, const ur3e_forward_out* out, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const bool con = out && (out->contact_geom || out->contact_dist || out->contact_pos || out->contact_frame || out->contact_force);
+    const bool any = out && (con || out->qacc || out->qfrc_constraint || out->info || out->flags || out->sensordata);
+    const std::string err = forward_query_check(out != nullptr, con, any, NCMAX);
+    if (!err.empty()) return set_err("forward: " + err);
+    const size_t smem = arena_stride<Real, D>() * WPB;
+    if (!fwd_ready) {
+      CUDA_OK(cudaFuncSetAttribute(query_fwd_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+      fwd_ready = true;
+    }
+    // read-only, like query(): last_stream stays that of the latest state-changing call
+    QFArgs<Real, D> a{d_model, d_state, base.opt, n, (const Real*)ctrl,
+                      FwdOut<Real>{(Real*)out->qacc, (Real*)out->qfrc_constraint, out->info, out->contact_geom, (Real*)out->contact_dist,
+                                   (Real*)out->contact_pos, (Real*)out->contact_frame, (Real*)out->contact_force, out->flags, (Real*)out->sensordata}};
+    query_fwd_kernel<Real, D><<<(unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, s>>>(a);
     ++launches;
     CUDA_OK(cudaGetLastError());
     return 0;

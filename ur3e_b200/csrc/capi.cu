@@ -118,5 +118,9 @@ int ur3e_batch_query(ur3e_batch* b, int query_id, void* pos, void* mat, void* ve
 int ur3e_batch_query_jac(ur3e_batch* b, int query_id, void* jacp, void* jacr, void* M, void* qfrc_bias, void* stream) {
   GUARD(b); return b->impl->query_jac(query_id, jacp, jacr, M, qfrc_bias, (cudaStream_t)stream);
 }
+int ur3e_batch_max_contacts(const ur3e_batch* b) { GUARD(b); return b->impl->max_contacts(); }
+int ur3e_batch_forward(ur3e_batch* b, const void* ctrl, const ur3e_forward_out* out, void* stream) {
+  GUARD(b); return b->impl->forward(ctrl, out, (cudaStream_t)stream);
+}
 
 }  // extern "C"

@@ -226,4 +226,25 @@ DevModel<Real> compile_model(const HostModel& h) {
   return m;
 }
 
+// The contact predicates of utils/gym_utils.py name bodies of the loaded model `h`: classify every collidable geom of `m` (compiled
+// from h, or from h with its fixed bodies merged: geom ids are the same) by them (GeomFlag)
+template <typename Real>
+void set_geom_flags(const HostModel& h, DevModel<Real>& m) {
+  const auto& par = h.I("body_parentid"); const auto& gbid = h.I("geom_bodyid");
+  auto under = [&](int b, int root) { if (root < 0) return false; for (int a = b; a > 0; a = par[a]) if (a == root) return true; return false; };
+  const int arm = h.name2id(OBJ_BODY, "robot_base"), grip = h.name2id(OBJ_BODY, "robotiq_base_mount"), table = h.name2id(OBJ_BODY, "table"),
+            mug = h.name2id(OBJ_BODY, "fish"), lpad = h.name2id(OBJ_BODY, "left_pad"), rpad = h.name2id(OBJ_BODY, "right_pad");
+  for (int i = 0; i < m.ngeom; ++i) {
+    const int b = gbid[m.geom_src[i]];
+    int f = 0;
+    if (under(b, arm)) f |= GF_ARM;
+    if (under(b, grip)) f |= GF_GRIPPER;
+    if (b == table && table >= 0) f |= GF_TABLE;
+    if (b == mug && mug >= 0) f |= GF_MUG;
+    if (b == lpad && lpad >= 0) f |= GF_LPAD;
+    if (b == rpad && rpad >= 0) f |= GF_RPAD;
+    m.geom_flags[i] = f;
+  }
+}
+
 }  // namespace ur3e

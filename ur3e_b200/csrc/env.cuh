@@ -136,11 +136,12 @@ UR3E_HD void controller(const DevModel<Real>& m, const EnvCfg<Real>& c, Arena<Re
 // ---------------------------------------------------------------- observation / reward / termination
 struct ContactFlags { int grasp_count; int table_hit; int self_hit; };
 
+// The contact predicates of the first s.ncon contacts as bits, the same in every lane: 1 mug - left pad, 2 mug - right pad,
+// 4 gripper - table, 8 self-collision.  gym_utils.py:108-128 (distinct pad bodies touching the mug), :174-201 (gripper subtree vs
+// table) and :146-172 (two bodies of the robot_base subtree that are not both in the gripper subtree); bodies as in the loaded
+// model (GeomFlag)
 template <typename Real, typename D>
-UR3E_HD ContactFlags contact_flags(const DevModel<Real>& m, const EnvCfg<Real>& c, const Arena<Real, D>& s) {
-  // gym_utils.py:108-128 (distinct pad bodies touching the mug), :174-201 (gripper subtree vs table) and :146-172 (two bodies of
-  // the robot_base subtree that are not both in the gripper subtree); bodies as in the loaded model (GeomFlag)
-  (void)c;
+UR3E_HD int contact_bits(const DevModel<Real>& m, const Arena<Real, D>& s) {
   int f = 0;
   if constexpr (D::HAS_CONTACT) {
     WARP_FOR(k, s.ncon) {
@@ -151,7 +152,13 @@ UR3E_HD ContactFlags contact_flags(const DevModel<Real>& m, const EnvCfg<Real>& 
       if ((f1 & GF_ARM) && (f2 & GF_ARM) && !((f1 & GF_GRIPPER) && (f2 & GF_GRIPPER))) f |= 8;
     }
   }
-  f = warp_or(f);
+  return warp_or(f);
+}
+
+template <typename Real, typename D>
+UR3E_HD ContactFlags contact_flags(const DevModel<Real>& m, const EnvCfg<Real>& c, const Arena<Real, D>& s) {
+  (void)c;
+  const int f = contact_bits(m, s);
   ContactFlags r; r.grasp_count = (f & 1) + ((f >> 1) & 1); r.table_hit = (f >> 2) & 1; r.self_hit = (f >> 3) & 1;
   return r;
 }

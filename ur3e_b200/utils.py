@@ -41,6 +41,18 @@ SimBatch.mass_matrix at the same stored state, one launch per call:
 
 After a step MuJoCo's d.qfrc_bias and the Jacobian it would compute belong to the last substep's pre-integration state (SURVEY F9);
 these are one substep newer, the same state as the pose accessors above.
+
+The contact predicates (utils/gym_utils.py:98-201) read the contact list of SimBatch.forward at the same stored state; they need no
+ctrl, so they run its contacts-only pass (kinematics and collision), one launch per call:
+
+    get_ncon(m, d)                                   # [N] int32    d.ncon
+    get_self_collision(m, d, collision_cache=None)   # [N] bool     two robot_base bodies not both in the gripper subtree touch
+    get_table_collision(m, d, collision_cache=None)  # [N] bool     the gripper subtree touches the table
+    get_block_grasp_state(m, d)                      # [N] int32    distinct pads touching the mug (the v0 observation's o[9])
+    get_robust_block_grasp_state(m, d)               # [N] bool     both pads, and the tcp within the mug-handle thresholds
+
+After a step MuJoCo's d.contact still holds the contacts of the last substep before integration (SURVEY F9); these are one substep
+newer, the same state as the pose accessors above.
 """
 import math
 
@@ -239,3 +251,52 @@ def get_full_M(m, d):
 
 def get_qfrc_bias(m, d):
     return _batch(d).mass_matrix(M=False, qfrc_bias=True)[1]
+
+
+def _contact_flags(d):
+    """contact_bits of every environment (1 mug - left pad, 2 mug - right pad, 4 gripper - table, 8 self-collision), one launch."""
+    return _batch(d).forward(qacc=False, flags=True).flags
+
+
+def init_collision_cache(m):
+    """Accepted for drop-in use: the batch classifies the collidable geoms once, when it is created.  Returns an opaque value that
+    the collision accessors ignore."""
+    return None
+
+
+def get_ncon(m, d):
+    return _batch(d).forward(qacc=False, info=True).info[:, 0]
+
+
+def get_self_collision(m, d, collision_cache=None):
+    return (_contact_flags(d) & 8) != 0
+
+
+def get_table_collision(m, d, collision_cache=None):
+    return (_contact_flags(d) & 4) != 0
+
+
+def get_block_grasp_state(m, d):
+    """Number of distinct gripper pads (left_pad, right_pad bodies) in contact with the mug: 0, 1 or 2 (gym_utils.py:108-128, the v0
+    observation's o[9]).  The reference's exact signature is not recorded in this repository; (m, d) follows its other accessors."""
+    f = _contact_flags(d)
+    return (f & 1) + ((f >> 1) & 1)
+
+
+def get_robust_block_grasp_state(m, d):
+    """Both pads touch the mug and the tcp is within (0.01, 0.005, 0.05) of the handle_site per axis (gym_utils.py:98-106, the v2
+    observation's o[23]).  Two launches: the contact flags and one kinematics query of the two sites.  The reference's exact
+    signature is not recorded in this repository; (m, d) follows its other accessors."""
+    both = (_contact_flags(d) & 3) == 3
+    p = _query_pair(d, (("site", "tcp"), ("site", "handle_site")))(pos=True)[0]
+    e = (p[:, 0] - p[:, 1]).abs()
+    return both & (e[:, 0] < 0.01) & (e[:, 1] < 0.005) & (e[:, 2] < 0.05)
+
+
+def _query_pair(d, objects):
+    b = _batch(d)
+    cache = b.__dict__.setdefault("_accessor_queries", {})
+    q = cache.get(objects)
+    if q is None:
+        q = cache[objects] = b.query(list(objects))
+    return q
