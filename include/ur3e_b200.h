@@ -99,10 +99,6 @@ int ur3e_batch_stats(ur3e_batch* b, double* stats16_dev, int reset_counters, voi
 enum { UR3E_STAT_EPISODES = 0, UR3E_STAT_RETURN, UR3E_STAT_LENGTH, UR3E_STAT_SUCCESS, UR3E_STAT_TERM_REACH, UR3E_STAT_TERM_TOPPLE,
        UR3E_STAT_TERM_COLLISION, UR3E_STAT_TRUNC, UR3E_STAT_UNSTABLE, UR3E_STAT_NEFC, UR3E_STAT_NCON, UR3E_STAT_ITER, UR3E_STAT_SUBSTEPS, UR3E_STAT_OVERFLOW,
        UR3E_STAT_PAD_CONTACT_STEPS /* env-steps that ended with >= 1 gripper-pad / mug contact */, UR3E_STAT_STEPS /* env-steps */ };
-/* d.* reads of one environment after a forward pass at its current state (mj_forward, mj_fullM, d.qfrc_bias, d.qacc,
- * d.ncon, d.contact[].dist/pos, mj_jacSite for the tcp): writes float64 host arrays; any pointer may be NULL */
-int ur3e_batch_debug_forward(ur3e_batch* b, int64_t env, double* M_nvnv, double* qfrc_bias, double* qacc, double* qfrc_constraint,
-                             int32_t* info8 /* ncon nefc iters overflow ... */, double* contact_dist_pos4 /* [MAXCON][4] */, double* cache54);
 /* kernels launched by this batch so far; bytes of shared memory per environment; environments resident per SM */
 int64_t ur3e_batch_launch_count(const ur3e_batch* b);
 int ur3e_batch_kernel_info(const ur3e_batch* b, int32_t* arena_bytes, int32_t* warps_per_block, int32_t* blocks_per_sm, int32_t* regs_per_thread);

@@ -1,24 +1,38 @@
-"""TEST-ONLY helper: compile ur3e_b200/csrc/engine.cuh as plain C++ (see host_engine.cpp) and bind it."""
+"""TEST-ONLY helper: compile the kernel source (engine.cuh) and the query sources (query.cuh, query_fwd.cuh) as plain C++ (see
+host_check.cpp) and bind them."""
 import ctypes as C
+import atexit
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
-SO = os.path.join(HERE, "libhostcheck.so")
+SRCS = [os.path.join(HERE, "host_check.cpp"), os.path.join(ROOT, "ur3e_b200", "csrc", "mjcf.cpp")]
+NSENSOR = 46
+FLOAT_OUTS = ("qacc", "qfrc_constraint", "contact_dist", "contact_pos", "contact_frame", "contact_force", "sensordata")
+INT_OUTS = ("info", "contact_geom", "flags")
 _L = None
 
 
 def lib():
+    """Compiled once per process into a temporary directory (the tree may be read-only)."""
     global _L
     if _L is None:
-        srcs = [os.path.join(HERE, "host_engine.cpp"), os.path.join(ROOT, "ur3e_b200", "csrc", "mjcf.cpp")]
-        deps = srcs + [os.path.join(ROOT, "ur3e_b200", "csrc", f) for f in ("engine.cuh", "warp_model.cuh", "dev_model.h", "compile_model.h", "host_model.h", "xml_mini.h", "merge_bodies.h")]
-        if not os.path.exists(SO) or any(os.path.getmtime(d) > os.path.getmtime(SO) for d in deps):
-            subprocess.check_call(["g++", "-O1", "-std=c++17", "-fPIC", "-shared", "-Wno-unused", "-ffp-contract=off", "-o", SO] + srcs)
-        _L = C.CDLL(SO)
+        tmp = tempfile.mkdtemp(prefix="ur3e_hostcheck_")
+        atexit.register(shutil.rmtree, tmp, True)
+        so = os.path.join(tmp, "libhostcheck.so")
+        subprocess.check_call(["g++", "-O1", "-std=c++17", "-fPIC", "-shared", "-Wno-unused", "-ffp-contract=off", "-o", so] + SRCS)
+        _L = C.CDLL(so)
+        dp, ip = C.POINTER(C.c_double), C.POINTER(C.c_int32)
+        _L.hc_query.argtypes = [C.c_char_p, dp, dp, ip, ip, C.c_int, C.c_int, dp, dp, dp]
+        _L.hc_query_jac.argtypes = [C.c_char_p, dp, dp, ip, ip, C.c_int, C.c_int, dp, dp, dp, dp]
+        _L.hc_forward.argtypes = [C.c_char_p, dp, dp, dp, dp, C.POINTER(dp), C.POINTER(ip)]
+        _L.hc_max_contacts.argtypes = [C.c_char_p]
+        _L.hc_forward_check.argtypes = [C.c_int] * 4
     return _L
 
 
@@ -41,7 +55,7 @@ def run(xml, qpos, qvel, ctrl, ws, nsteps, use_float=0, max_iter=50, tol=1e-15):
 
 def sensors(xml, qpos, qvel, ctrl):
     """The step kernel's logging record (include/ur3e_b200.h UR3E_NSENSOR) after a forward pass at the given state."""
-    out = np.zeros(46)
+    out = np.zeros(NSENSOR)
     a = [np.ascontiguousarray(x, dtype=np.float64) for x in (qpos, qvel, ctrl)]
     assert lib().hc_sensors(xml.encode(), _p(a[0]), _p(a[1]), _p(a[2]), _p(out)) == 0
     return out
@@ -52,3 +66,72 @@ def model_array(xml, name, cap=8192):
     k = lib().hc_model_array(xml.encode(), name.encode(), _p(out), cap)
     assert k >= 0, name
     return out[:k]
+
+
+def query(xml, qpos, qvel, objtype, objid, local=0):
+    """(pos [k, 3], mat [k, 3, 3], vel [k, 6]) of the objects at (qpos, qvel), float64."""
+    k = len(objtype)
+    pos = np.zeros((k, 3)); mat = np.zeros((k, 9)); vel = np.zeros((k, 6))
+    qp, qv = (np.ascontiguousarray(x, dtype=np.float64) for x in (qpos, qvel))
+    t, i = (np.ascontiguousarray(x, dtype=np.int32) for x in (objtype, objid))
+    ip = lambda a: a.ctypes.data_as(C.POINTER(C.c_int32))
+    rc = lib().hc_query(xml.encode(), _p(qp), _p(qv), ip(t), ip(i), k, int(local), _p(pos), _p(mat), _p(vel))
+    if rc != 0:
+        raise ValueError("hc_query rejected the query (%d)" % rc)
+    return pos, mat.reshape(k, 3, 3), vel
+
+
+def query_jac(xml, qpos, qvel, objtype=(), objid=(), jacp=True, jacr=True, M=True, qfrc_bias=True, query_id=None):
+    """(jacp [k, 3, nv], jacr [k, 3, nv], M [nv, nv], qfrc_bias [nv]) at (qpos, qvel), float64, None for an output not asked for.
+    The objects are compiled as the batch's query 0 (none when empty); query_id defaults to 0 with objects, -1 without."""
+    k, nv = len(objtype), len(qvel)
+    if query_id is None:
+        query_id = 0 if k else -1
+    outs = [np.zeros(s) if want else None for want, s in ((jacp, (k, 3, nv)), (jacr, (k, 3, nv)), (M, (nv, nv)), (qfrc_bias, (nv,)))]
+    qp, qv = (np.ascontiguousarray(x, dtype=np.float64) for x in (qpos, qvel))
+    t, i = (np.ascontiguousarray(x, dtype=np.int32).reshape(-1) for x in (objtype, objid))
+    dp = lambda a: _p(a) if a is not None else None
+    ip = lambda a: a.ctypes.data_as(C.POINTER(C.c_int32))
+    rc = lib().hc_query_jac(xml.encode(), _p(qp), _p(qv), ip(t), ip(i), k, int(query_id), *[dp(o) for o in outs])
+    if rc != 0:
+        raise ValueError("hc_query_jac rejected the call (%d)" % rc)
+    return tuple(outs)
+
+
+def forward_check(out, con, any_, ncmax):
+    """forward_query_check: True when ur3e_batch_forward accepts the combination."""
+    return lib().hc_forward_check(int(out), int(con), int(any_), int(ncmax)) == 0
+
+
+def max_contacts(xml):
+    return lib().hc_max_contacts(xml.encode())
+
+
+def forward(xml, qpos, qvel, ws=None, ctrl=None, qacc=True, qfrc_constraint=False, info=False, contact_geom=False, contact_dist=False,
+            contact_pos=False, contact_frame=False, contact_force=False, flags=False, sensordata=False):
+    """dict of the requested outputs of one mj_forward at (qpos, qvel, warm start ws = 0 by default) with ctrl (None = zero), float64;
+    shapes as SimBatch.forward's without the environment axis (contact_frame [C, 3, 3]).  Outputs are pre-filled with NaN / a sentinel,
+    so that an entry the query leaves unwritten shows.  Raises ValueError when the call is rejected."""
+    nv, Cn = len(qvel), max_contacts(xml)
+    want = dict(qacc=qacc, qfrc_constraint=qfrc_constraint, info=info, contact_geom=contact_geom, contact_dist=contact_dist,
+                contact_pos=contact_pos, contact_frame=contact_frame, contact_force=contact_force, flags=flags, sensordata=sensordata)
+    shape = dict(qacc=(nv,), qfrc_constraint=(nv,), info=(4,), contact_geom=(Cn, 2), contact_dist=(Cn,), contact_pos=(Cn, 3),
+                 contact_frame=(Cn, 3, 3), contact_force=(Cn, 6), flags=(1,), sensordata=(NSENSOR,))
+    out = {}
+    for k, w in want.items():
+        if w:
+            out[k] = np.full(shape[k], -7, dtype=np.int32) if k in INT_OUTS else np.full(shape[k], np.nan)
+            if out[k].size == 0:   # a zero-length output still counts as asked for (the call then rejects it)
+                out[k] = np.full(1, np.nan)
+    dp = C.POINTER(C.c_double); ip = C.POINTER(C.c_int32)
+    fo = (dp * len(FLOAT_OUTS))(*[out[k].ctypes.data_as(dp) if k in out else dp() for k in FLOAT_OUTS])
+    io = (ip * len(INT_OUTS))(*[out[k].ctypes.data_as(ip) if k in out else ip() for k in INT_OUTS])
+    qp, qv = (np.ascontiguousarray(x, dtype=np.float64) for x in (qpos, qvel))
+    w = np.zeros(nv) if ws is None else np.ascontiguousarray(ws, dtype=np.float64)
+    u = None if ctrl is None else np.ascontiguousarray(ctrl, dtype=np.float64)
+    rc = lib().hc_forward(xml.encode(), _p(qp), _p(qv), _p(w), _p(u) if u is not None else None, fo, io)
+    if rc != 0:
+        raise ValueError("hc_forward rejected the call (%d)" % rc)
+    if "flags" in out:
+        out["flags"] = int(out["flags"][0])
+    return out

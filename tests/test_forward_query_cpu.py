@@ -1,4 +1,4 @@
-"""CPU suite: the forward-dynamics query (query_fwd.cuh forward_query_env), compiled as plain C++ by tests/hostcheck/forward.py, in
+"""CPU suite: the forward-dynamics query (query_fwd.cuh forward_query_env), compiled as plain C++ by tests/hostcheck, in
 float64, against the oracle's forward() at the same (qpos, qvel, warm start, ctrl): the contact list, the contact forces, qacc,
 qfrc_constraint and the sensor record; the box-at-rest pin on the query's own contact forces; the contacts-only pass against the full
 one; the argument check."""
@@ -9,7 +9,6 @@ import pytest
 
 from oracle import oracle as O
 from tests.hostcheck import build as HC
-from tests.hostcheck import forward as HF
 from tests.test_analytic_pins import G, M_BOX, model_path
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -60,7 +59,7 @@ def _check(path, m, states, need_contacts):
     seen = 0
     for qp, qv, ws, u in states:
         d = _oracle(m, qp, qv, ws, u)
-        r = HF.forward(path, qp, qv, ws, u, **ALL)
+        r = HC.forward(path, qp, qv, ws, u, **ALL)
         ncon, nefc, _, ovf = r["info"]
         assert (ncon, nefc, ovf) == (d.ncon, d.nefc, 0)
         seen += ncon > 0
@@ -86,7 +85,7 @@ def _check(path, m, states, need_contacts):
         assert (r["contact_geom"][ncon:] == -1).all()
         for k in ("contact_dist", "contact_pos", "contact_frame", "contact_force"):
             assert not r[k][ncon:].any(), k
-        # the solver-tolerance bound of test_gpu_parity.py::test_main_forward_internals_f64
+        # the solver-tolerance bound of test_gpu_parity.py::test_main_forward_internals_via_queries_f64
         assert rel(r["qacc"], d.qacc, 1e-1) < 1e-6
         assert rel(r["qfrc_constraint"], d.qfrc_constraint, 1e-1) < 1e-6
         s = r["sensordata"]
@@ -117,7 +116,7 @@ def test_forward_matches_oracle_closing_on_mug(assets):
     m = O.Model(path)
     states = _closing(m, 255.0, 450, 90)
     _check(path, m, states, 5)
-    r = HF.forward(path, *states[-1], flags=True)
+    r = HC.forward(path, *states[-1], flags=True)
     assert r["flags"] & 3 == 3      # both pads on the mug
 
 
@@ -139,12 +138,12 @@ def test_forward_raw_arm(assets):
     """ur3e_raw.xml: no contact pairs (C = 0); qacc, the sensor record and info against the oracle."""
     path = assets + "/ur3e_raw.xml"
     m = O.Model(path)
-    assert HF.max_contacts(path) == 0
+    assert HC.max_contacts(path) == 0
     rng = np.random.default_rng(33)
     for _ in range(3):
         qp = rng.uniform(-1, 1, m.nq); qv = rng.uniform(-1, 1, m.nv); u = rng.uniform(-5, 5, m.nu)
         d = _oracle(m, qp, qv, np.zeros(m.nv), u)
-        r = HF.forward(path, qp, qv, ctrl=u, qfrc_constraint=True, info=True, flags=True, sensordata=True)
+        r = HC.forward(path, qp, qv, ctrl=u, qfrc_constraint=True, info=True, flags=True, sensordata=True)
         assert list(r["info"]) == [0, d.nefc, r["info"][2], 0] and r["flags"] == 0
         assert rel(r["qacc"], d.qacc, 1e-1) < 1e-6 and rel(r["qfrc_constraint"], d.qfrc_constraint, 1e-1) < 1e-6
         assert rel(r["sensordata"][:7], d.sensors()[:7], 1e-1) < 1e-9
@@ -156,7 +155,7 @@ def test_folded_arm_flags_match_reference_fixture(assets):
     g = np.load(os.path.join(HERE, "golden", "collision.npz"))
     for kind in ("v2", "v0"):
         for e, q in enumerate(g[kind + "_qpos"]):
-            r = HF.forward(path, q, g["qvel"], qacc=False, info=True, flags=True)
+            r = HC.forward(path, q, g["qvel"], qacc=False, info=True, flags=True)
             assert r["info"][0] == g[kind + "_ncon"][e]
             assert bool(r["flags"] & 8) == bool(g[kind + "_self_collision"][e]) and bool(r["flags"] & 4) == bool(g[kind + "_table_collision"][e])
 
@@ -172,7 +171,7 @@ def test_box_at_rest_contact_forces_from_query():
         m = O.Model(p)
         r = HC.run(p, np.array(m.arr("qpos0")).copy(), np.zeros(m.nv), np.zeros(m.nu), np.zeros(m.nv), 3000)
         assert r["warn"] == 0 and r["overflow"] == 0
-        q = HF.forward(p, r["qpos"], r["qvel"], r["qacc"], info=True, contact_force=True)
+        q = HC.forward(p, r["qpos"], r["qvel"], r["qacc"], info=True, contact_force=True)
     n = q["info"][0]
     assert n == 4
     f = q["contact_force"][:n]
@@ -188,8 +187,8 @@ def test_contacts_only_pass_equals_full_pass(assets, states):
     m = O.Model(path)
     S = _pressed(m, np.random.default_rng(35)) if states == "pressed" else _closing(m, 255.0, 450, 90)
     for qp, qv, ws, u in S:
-        full = HF.forward(path, qp, qv, ws, u, **ALL)
-        geo = HF.forward(path, qp, qv, ws, u, qacc=False, info=True, flags=True, **{k: True for k in GEOMETRY})
+        full = HC.forward(path, qp, qv, ws, u, **ALL)
+        geo = HC.forward(path, qp, qv, ws, u, qacc=False, info=True, flags=True, **{k: True for k in GEOMETRY})
         for k in GEOMETRY:
             assert np.array_equal(geo[k], full[k]), k
         assert geo["flags"] == full["flags"]
@@ -203,9 +202,9 @@ def test_forward_outputs_are_independent(assets):
     path = assets + "/main.xml"
     m = O.Model(path)
     qp, qv, ws, u = _closing(m, 255.0, 360, 360)[0]
-    full = HF.forward(path, qp, qv, ws, u, **ALL)
+    full = HC.forward(path, qp, qv, ws, u, **ALL)
     for k in ALL:
-        one = HF.forward(path, qp, qv, ws, u, **{j: j == k for j in ALL})
+        one = HC.forward(path, qp, qv, ws, u, **{j: j == k for j in ALL})
         if k == "info":
             assert one[k][0] == full[k][0] and one[k][1] == one[k][2] == 0
         else:
@@ -216,8 +215,8 @@ def test_forward_zero_ctrl_is_default(assets):
     path = assets + "/main.xml"
     m = O.Model(path)
     qp, qv, ws, _ = _pressed(m, np.random.default_rng(36), 1)[0]
-    a = HF.forward(path, qp, qv, ws, None, qacc=True, sensordata=True)
-    b = HF.forward(path, qp, qv, ws, np.zeros(m.nu), qacc=True, sensordata=True)
+    a = HC.forward(path, qp, qv, ws, None, qacc=True, sensordata=True)
+    b = HC.forward(path, qp, qv, ws, np.zeros(m.nu), qacc=True, sensordata=True)
     assert np.array_equal(a["qacc"], b["qacc"]) and np.array_equal(a["sensordata"], b["sensordata"])
 
 
@@ -227,15 +226,15 @@ def test_forward_rejections(assets):
         for con in (0, 1):
             for any_ in (0, 1):
                 for C in (0, 12, 24):
-                    ok = HF.check(out, con, any_, C)
+                    ok = HC.forward_check(out, con, any_, C)
                     assert ok == (bool(out) and bool(any_) and not (con and C == 0)), (out, con, any_, C)
     # through the host-compiled entry point
     main, raw = assets + "/main.xml", assets + "/ur3e_raw.xml"
     qp, qv = O.Model(main).key("down")
     with pytest.raises(ValueError):
-        HF.forward(main, qp, qv, qacc=False)
+        HC.forward(main, qp, qv, qacc=False)
     mr = O.Model(raw)
     for k in GEOMETRY + ("contact_force",):
         with pytest.raises(ValueError):
-            HF.forward(raw, np.zeros(mr.nq), np.zeros(mr.nv), **{k: True})
-    HF.forward(raw, np.zeros(mr.nq), np.zeros(mr.nv), qacc=False, flags=True)   # flags need no contact storage
+            HC.forward(raw, np.zeros(mr.nq), np.zeros(mr.nv), **{k: True})
+    HC.forward(raw, np.zeros(mr.nq), np.zeros(mr.nv), qacc=False, flags=True)   # flags need no contact storage

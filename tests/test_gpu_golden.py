@@ -138,18 +138,27 @@ def test_folded_arm_self_collision_vs_oracle(kind):
     assert st["term_collision"] == 2 and st["episodes"] == 2
 
 
-@pytest.mark.parametrize("kind", ["v2", "v0", "indirect", "direct"])
+@pytest.mark.parametrize("kind", ["v2", "v0", "indirect"])
 def test_truncation_step_vs_reference_fixture(kind):
     """SURVEY 8a row a15: ur3e-v2 increments t before the truncation test (first truncated step 2500), the other three test first
     (501 / 2501 / 1201).  tests/golden/truncation.npz holds what the reference's own classes reported under a hold-still action;
     the production float32 kernel, with the shipped max_steps, must truncate on exactly that step (and auto-reset right there)."""
+    _check_truncation_vs_fixture(kind)
+
+
+def test_direct_truncation_step_vs_reference_fixture():
+    """The same for imitation_direct-v0, whose hold-still action is the gravity compensation at the keyframe (from mass_matrix)."""
+    _check_truncation_vs_fixture("direct")
+
+
+def _check_truncation_vs_fixture(kind):
     first_ref, term_ref = np.load(GOLD + "/truncation.npz")[kind]
     assert term_ref == 0
     env = UR3eVecEnv(IDS[kind], 3, dtype=torch.float32, auto_reset=True, reset_noise=lib.NOISE_NONE)
     obs, _ = env.reset()
     if kind == "direct":
         hold = torch.zeros(3, 7, device="cuda")
-        hold[:, :6] = torch.tensor(env.batch.debug_forward(0)["bias_arm"], device="cuda", dtype=torch.float32)    # gravity compensation at the keyframe
+        hold[:, :6] = env.batch.mass_matrix(M=False, qfrc_bias=True)[1][0, :6]    # gravity compensation at the keyframe
     else:
         hold = torch.cat([obs[:, :3], torch.zeros(3, 1, device="cuda")], 1).contiguous()
     first = -1
@@ -212,8 +221,9 @@ def test_vec_env_api_and_sb3_adapter():
     assert o.shape == (4, 13) and (r == -1).all() and not te.any()
 
 
-def test_controller_entry_points_track_targets():
-    """move_j on ur3e_raw.xml and move_l (pid_task_ctrl) on ur3e_2f85.xml converge to their targets."""
+def test_controller_entry_points_track_targets_via_query():
+    """move_j on ur3e_raw.xml and move_l (pid_task_ctrl) on ur3e_2f85.xml converge to their targets (move_l's tcp read through a
+    kinematics query)."""
     tgt = np.tile(np.array([0.3, -0.4, 0.5, -0.2, 0.1, 0.2, 0.0]), (3000, 1))
     q, v, _ = controller.move_j.run(tgt, n_envs=4, xml="ur3e_raw.xml", dtype=torch.float64, record_every=3000)
     err = (q[-1, 0] - torch.tensor(tgt[0, :6], device="cuda")).abs()            # 0.3 s of PD without gravity compensation
@@ -221,12 +231,12 @@ def test_controller_entry_points_track_targets():
     tcp = np.array([0.29799994, 0.13349916, 0.1682003])
     tl = np.tile(np.hstack([tcp + [0.03, 0.02, 0.03], presets.TOOL_ROTVEC, 0.0]), (1500, 1))
     q, v, b = controller.move_l.run(tl, n_envs=4, record_every=1500)
-    dbg = b.debug_forward(0)
-    assert np.abs(dbg["tcp_pos"] - tl[0, :3]).max() < 0.02
+    tcp_pos = b.query([("site", "tcp")])()[0][0, 0].cpu().numpy()
+    assert np.abs(tcp_pos - tl[0, :3]).max() < 0.02
     assert controller.task_space.pid_task_ctrl is controller.move_l.run
 
 
-def test_device_built_per_env_trajectories_drive_move_l():
+def test_device_built_per_env_trajectories_drive_move_l_via_query():
     """build_traj on the device -> [T, N, 7] per-environment waypoint streams -> the batched move_l loop, no host round trip."""
     tcp = torch.tensor([0.29799994, 0.13349916, 0.1682003], device="cuda", dtype=torch.float64)
     rot = torch.tensor(presets.TOOL_ROTVEC, device="cuda", dtype=torch.float64)
@@ -237,8 +247,9 @@ def test_device_built_per_env_trajectories_drive_move_l():
     assert traj.is_cuda and traj.shape == (1500, 4, 7)
     traj = torch.cat([traj, traj[-1:].expand(1000, 4, 7)])                                              # settle on the last waypoint
     q, v, b = controller.move_l.run(traj, n_envs=4, record_every=2500)
+    tcp_pos = b.query([("site", "tcp")])()[0][:, 0].cpu().numpy()
     for e in range(4):
-        assert np.abs(b.debug_forward(e)["tcp_pos"] - stop[e, :3].cpu().numpy()).max() < 0.02
+        assert np.abs(tcp_pos[e] - stop[e, :3].cpu().numpy()).max() < 0.02
 
 
 def test_two_tier_stepping_f32():

@@ -104,8 +104,9 @@ def _random_states(m, rng, n, lift=False):
     return qp, qv
 
 
-def test_main_forward_internals_f64(assets):
-    """mj_forward quantities (M, qfrc_bias, qacc, ncon, nefc) on random main.xml states with mug-table contacts."""
+def test_main_forward_internals_via_queries_f64(assets):
+    """mj_forward quantities (M, qfrc_bias, qacc, ncon, nefc, the tcp Jacobian) on random main.xml states with mug-table contacts,
+    read for every environment through forward(), mass_matrix() and Query.jac."""
     m = O.Model(assets + "/main.xml"); d = O.Data(m)
     rng = np.random.default_rng(3)
     n = 8
@@ -113,15 +114,18 @@ def test_main_forward_internals_f64(assets):
     b = make(assets, "main.xml", n, torch.float64, ctrl_mode=lib.CTRL_PID_TASK_ENV, obs_kind=lib.OBS_V2, obs_dim=24, act_dim=4, gains=OE.GAINS_MUG, frame_skip=2, reset_key=1, term_kind=lib.TERM_V2, reward_kind=lib.REW_V2, max_steps=2500)
     b.reset()
     b.set_state(torch.tensor(qp, device="cuda"), torch.tensor(qv, device="cuda"))
+    fwd = b.forward(qacc=True, info=True)
+    qacc, info = fwd.qacc.cpu().numpy(), fwd.info.cpu().numpy()
+    M, bias = (x.cpu().numpy() for x in b.mass_matrix(M=True, qfrc_bias=True))
+    jacp, jacr = (x.cpu().numpy() for x in b.query([("site", "tcp")]).jac(jacp=True, jacr=True)[:2])
     for e in range(n):
         d.reset(); d.set_state(qp[e], qv[e]); d.forward()
-        g = b.debug_forward(e)
-        assert g["ncon"] == d.ncon and g["nefc"] == d.nefc
-        assert rel(g["M"], d.fullM(), 1e-6) < 1e-9
-        assert rel(g["qfrc_bias"], d.qfrc_bias) < 1e-9
-        assert rel(g["qacc"], d.qacc, 1e-1) < 1e-6
+        assert info[e, 0] == d.ncon and info[e, 1] == d.nefc
+        assert rel(M[e], d.fullM(), 1e-6) < 1e-9
+        assert rel(bias[e], d.qfrc_bias) < 1e-9
+        assert rel(qacc[e], d.qacc, 1e-1) < 1e-6
         jp, jr = d.jac_site(m.id("site", "tcp"))
-        assert rel(g["J_arm"], np.vstack([jp[:, :6], jr[:, :6]]), 1e-3) < 1e-9
+        assert rel(np.vstack([jacp[e, 0, :, :6], jacr[e, 0, :, :6]]), np.vstack([jp[:, :6], jr[:, :6]]), 1e-3) < 1e-9
 
 
 @pytest.mark.parametrize("kind", ["v2", "v0", "indirect"])

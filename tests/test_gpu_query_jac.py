@@ -1,6 +1,6 @@
 """GPU suite for the Jacobian / mass-matrix queries (ur3e_batch_query_jac, Query.jac, SimBatch.mass_matrix, the mj_jac* accessors of
-ur3e_b200/utils.py): the compiled sm_100a kernel against the float64 oracle and the debug forward pass at the batch's stored
-state, float32 against float64, a user-side pid_task_ctrl against the fused controller, and non-interference with the step path."""
+ur3e_b200/utils.py): the compiled sm_100a kernel against the float64 oracle and the step's own forward pass (compiled for the
+CPU) at the batch's stored state, float32 against float64, a user-side pid_task_ctrl against the fused controller, and non-interference with the step path."""
 import ctypes as C
 
 import numpy as np
@@ -15,6 +15,7 @@ import ur3e_b200._lib as lib
 from ur3e_b200 import utils as U
 from ur3e_b200.batch import SimBatch, env_config
 from ur3e_b200.model import Model
+from tests.hostcheck import build as HC
 from tests.test_gpu_query import _move_j, _run, _v2, _whole_model_query
 from tests.test_query_jac_cpu import _owner
 from tests.test_query_cpu import _reference
@@ -46,10 +47,10 @@ def _check_jac_against_oracle(b, om, types, ids, q, envs, tol):
 
 
 @pytest.mark.parametrize("scene", ["main.xml", "ur3e_2f85.xml", "ur3e_raw.xml"])
-def test_query_jac_matches_oracle_f64(assets, scene):
+def test_query_jac_matches_oracle_and_step_forward_f64(assets, scene):
     """After 300 seeded random steps (the recipe of test_gpu_query.py::test_whole_model_query_matches_oracle_f64), 16 sampled envs:
-    jacp / jacr of every object, M and qfrc_bias within 1e-10 of the oracle at get_state(); M and qfrc_bias within 1e-12 of
-    debug_forward, which runs the step's own forward pass."""
+    jacp / jacr of every object, M and qfrc_bias within 1e-10 of the oracle at get_state(); M and qfrc_bias within 1e-12 of the
+    step's own forward pass (engine.cuh forward(), compiled for the CPU by tests/hostcheck) at the same stored state."""
     b, lo, hi = _batch_for(assets, scene, 256, torch.float64)
     _run(b, lo, hi, 300, seed=3)
     if scene == "main.xml":
@@ -59,9 +60,10 @@ def test_query_jac_matches_oracle_f64(assets, scene):
     envs = np.random.default_rng(0).choice(b.n, 16, replace=False)
     _check_jac_against_oracle(b, om, types, ids, q, envs, 1e-10)
     M, bias = (x.cpu().numpy() for x in b.mass_matrix(M=True, qfrc_bias=True))
+    qp, qv, ws = (x.cpu().numpy() for x in b.get_state())
     for e in envs[:4]:
-        dbg = b.debug_forward(int(e))
-        assert np.abs(M[e] - dbg["M"]).max() <= 1e-12 and np.abs(bias[e] - dbg["qfrc_bias"]).max() <= 1e-12, e
+        ref = HC.run(b.model.path, qp[e], qv[e], np.zeros(b.model.nu), ws[e], 0)
+        assert np.abs(M[e] - ref["M"]).max() <= 1e-12 and np.abs(bias[e] - ref["bias"]).max() <= 1e-12, e
 
 
 def test_query_jac_f32_against_f64(assets):

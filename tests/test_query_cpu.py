@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.hostcheck import query as HQ
+from tests.hostcheck import build as HC
 
 XMLS = ["ur3e_raw.xml", "ur3e_2f85.xml", "main.xml"]
 BODY, XBODY, GEOM, SITE = 1, 2, 5, 6
@@ -69,8 +69,8 @@ def test_query_matches_oracle_f64(assets, xml):
         qp, qv = _state(m, rng, xml)
         d.reset(); d.set_state(qp, qv); d.forward()
         rp, rm, rvw, rvl = _reference(m, d, types, ids)
-        pos, mat, vw = HQ.query(path, qp, qv, types, ids, local=0)
-        _, _, vl = HQ.query(path, qp, qv, types, ids, local=1)
+        pos, mat, vw = HC.query(path, qp, qv, types, ids, local=0)
+        _, _, vl = HC.query(path, qp, qv, types, ids, local=1)
         assert np.abs(pos - rp).max() <= 1e-12
         assert np.abs(mat - rm).max() <= 1e-12
         assert np.abs(vw - rvw).max() <= 1e-12
@@ -90,9 +90,9 @@ def test_query_velocity_is_derivative_of_pose(assets, xml):
     eps = 1e-5
     for _ in range(4):
         qp, qv = _state(m, rng, xml)
-        _, R, v = HQ.query(path, qp, qv, types, ids)
-        pp, Rp, _ = HQ.query(path, _integrate(m, qp, qv, eps, xml), qv, types, ids)
-        pm, Rm, _ = HQ.query(path, _integrate(m, qp, qv, -eps, xml), qv, types, ids)
+        _, R, v = HC.query(path, qp, qv, types, ids)
+        pp, Rp, _ = HC.query(path, _integrate(m, qp, qv, eps, xml), qv, types, ids)
+        pm, Rm, _ = HC.query(path, _integrate(m, qp, qv, -eps, xml), qv, types, ids)
         assert np.abs((pp - pm) / (2 * eps) - v[:, 3:]).max() < 1e-6
         w = v[:, :3]
         W = np.zeros((len(w), 3, 3))
@@ -106,7 +106,7 @@ def test_tcp_at_keyframe_down_matches_reference_record(assets):
     path = assets + "/main.xml"
     m = O.Model(path)
     qp, qv = m.key("down")
-    pos, _, _ = HQ.query(path, qp, qv, [SITE], [m.id("site", "tcp")])
+    pos, _, _ = HC.query(path, qp, qv, [SITE], [m.id("site", "tcp")])
     assert np.abs(pos[0] - [0.29799994, 0.13349916, 0.1682003]).max() <= 5e-8
 
 
@@ -116,8 +116,8 @@ def test_query_rejects_bad_objects(assets):
     qp, qv = m.key("down")
     for t, i in (([3], [0]), ([BODY], [m.nbody]), ([GEOM], [-1]), ([SITE], [m.nsite])):
         with pytest.raises(ValueError):
-            HQ.query(path, qp, qv, t, i)
+            HC.query(path, qp, qv, t, i)
     for k in (0, 257):
         with pytest.raises(ValueError):
-            HQ.query(path, qp, qv, [SITE] * k, [0] * k)
-    HQ.query(path, qp, qv, [SITE] * 256, [0] * 256)
+            HC.query(path, qp, qv, [SITE] * k, [0] * k)
+    HC.query(path, qp, qv, [SITE] * 256, [0] * 256)

@@ -1,4 +1,4 @@
-"""CPU suite: the Jacobian / mass-matrix query (query.cuh query_jac_env), compiled as plain C++ by tests/hostcheck/query_jac.py, in
+"""CPU suite: the Jacobian / mass-matrix query (query.cuh query_jac_env), compiled as plain C++ by tests/hostcheck, in
 float64.
 
 Every body (inertial and body frame), geom and site of each scene is queried at random states and its jacp / jacr compared with
@@ -10,8 +10,7 @@ import numpy as np
 import pytest
 
 from oracle import oracle as O
-from tests.hostcheck import query as HQ
-from tests.hostcheck import query_jac as HQJ
+from tests.hostcheck import build as HC
 from tests.test_query_cpu import BODY, GEOM, SITE, XBODY, XMLS, _all_objects, _integrate, _reference, _state
 
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -33,7 +32,7 @@ def test_query_jac_matches_oracle_f64(assets, xml):
         qp, qv = _state(m, rng, xml)
         d.reset(); d.set_state(qp, qv); d.forward()
         points = _reference(m, d, types, ids)[0]
-        jacp, jacr, M, bias = HQJ.query_jac(path, qp, qv, types, ids)
+        jacp, jacr, M, bias = HC.query_jac(path, qp, qv, types, ids)
         for j in range(len(types)):
             rp, rr = d.jac(points[j], int(owner[j]))
             assert np.abs(jacp[j] - rp).max() <= 1e-12, (types[j], ids[j])
@@ -52,8 +51,8 @@ def test_query_jac_times_qvel_is_object_velocity(assets, xml):
     types, ids = _all_objects(m)
     for _ in range(4):
         qp, qv = _state(m, rng, xml)
-        jacp, jacr, _, _ = HQJ.query_jac(path, qp, qv, types, ids, M=False, qfrc_bias=False)
-        _, _, vel = HQ.query(path, qp, qv, types, ids, local=0)
+        jacp, jacr, _, _ = HC.query_jac(path, qp, qv, types, ids, M=False, qfrc_bias=False)
+        _, _, vel = HC.query(path, qp, qv, types, ids, local=0)
         assert np.abs(jacr @ qv - vel[:, :3]).max() <= 1e-12
         assert np.abs(jacp @ qv - vel[:, 3:]).max() <= 1e-12
 
@@ -68,10 +67,10 @@ def test_query_jac_is_derivative_of_pose(assets, xml):
     eps = 1e-5
     for _ in range(4):
         qp, v = _state(m, rng, xml)
-        jacp, jacr, _, _ = HQJ.query_jac(path, qp, v, types, ids, M=False, qfrc_bias=False)
-        _, R, _ = HQ.query(path, qp, v, types, ids)
-        pp, Rp, _ = HQ.query(path, _integrate(m, qp, v, eps, xml), v, types, ids)
-        pm, Rm, _ = HQ.query(path, _integrate(m, qp, v, -eps, xml), v, types, ids)
+        jacp, jacr, _, _ = HC.query_jac(path, qp, v, types, ids, M=False, qfrc_bias=False)
+        _, R, _ = HC.query(path, qp, v, types, ids)
+        pp, Rp, _ = HC.query(path, _integrate(m, qp, v, eps, xml), v, types, ids)
+        pm, Rm, _ = HC.query(path, _integrate(m, qp, v, -eps, xml), v, types, ids)
         assert np.abs((pp - pm) / (2 * eps) - jacp @ v).max() < 1e-6
         w = jacr @ v
         W = np.zeros((len(w), 3, 3))
@@ -95,12 +94,12 @@ def test_query_mass_matrix_and_bias_double_pendulum_textbook():
         h = -m2 * l1 * lc2 * s2
         grav = np.array([m1 * G * lc1 * np.sin(q[0]) + m2 * G * (l1 * np.sin(q[0]) + lc2 * np.sin(q[0] + q[1])), m2 * G * lc2 * np.sin(q[0] + q[1])])
         bias = np.array([h * (2 * v[0] * v[1] + v[1] ** 2), -h * v[0] ** 2]) + grav
-        jp, jr, gotM, gotb = HQJ.query_jac(path, q, v, jacp=False, jacr=False)
+        jp, jr, gotM, gotb = HC.query_jac(path, q, v, jacp=False, jacr=False)
         assert jp is None and jr is None
         assert np.abs(gotM - M).max() < 1e-12 and np.abs(gotb - bias).max() < 1e-11, (gotM, M, gotb, bias)
         # each output alone is the same value
-        assert np.array_equal(HQJ.query_jac(path, q, v, jacp=False, jacr=False, qfrc_bias=False)[2], gotM)
-        assert np.array_equal(HQJ.query_jac(path, q, v, jacp=False, jacr=False, M=False)[3], gotb)
+        assert np.array_equal(HC.query_jac(path, q, v, jacp=False, jacr=False, qfrc_bias=False)[2], gotM)
+        assert np.array_equal(HC.query_jac(path, q, v, jacp=False, jacr=False, M=False)[3], gotb)
 
 
 def test_query_jac_outputs_are_independent(assets):
@@ -109,10 +108,10 @@ def test_query_jac_outputs_are_independent(assets):
     m = O.Model(path)
     qp, qv = _state(m, np.random.default_rng(25), "main.xml")
     types, ids = _all_objects(m)
-    full = HQJ.query_jac(path, qp, qv, types, ids)
-    assert np.array_equal(HQJ.query_jac(path, qp, qv, types, ids, jacr=False, M=False, qfrc_bias=False)[0], full[0])
-    assert np.array_equal(HQJ.query_jac(path, qp, qv, types, ids, jacp=False, M=False, qfrc_bias=False)[1], full[1])
-    assert np.array_equal(HQJ.query_jac(path, qp, qv, types, ids, jacp=False, jacr=False)[2], full[2])
+    full = HC.query_jac(path, qp, qv, types, ids)
+    assert np.array_equal(HC.query_jac(path, qp, qv, types, ids, jacr=False, M=False, qfrc_bias=False)[0], full[0])
+    assert np.array_equal(HC.query_jac(path, qp, qv, types, ids, jacp=False, M=False, qfrc_bias=False)[1], full[1])
+    assert np.array_equal(HC.query_jac(path, qp, qv, types, ids, jacp=False, jacr=False)[2], full[2])
 
 
 def test_query_jac_rejections(assets):
@@ -121,17 +120,17 @@ def test_query_jac_rejections(assets):
     qp, qv = m.key("down")
     tcp = m.id("site", "tcp")
     with pytest.raises(ValueError):    # unknown query id
-        HQJ.query_jac(path, qp, qv, [SITE], [tcp], query_id=1)
+        HC.query_jac(path, qp, qv, [SITE], [tcp], query_id=1)
     with pytest.raises(ValueError):
-        HQJ.query_jac(path, qp, qv, [SITE], [tcp], query_id=-2)
+        HC.query_jac(path, qp, qv, [SITE], [tcp], query_id=-2)
     with pytest.raises(ValueError):    # no query compiled: id 0 is unknown too
-        HQJ.query_jac(path, qp, qv, query_id=0, jacp=False, jacr=False)
+        HC.query_jac(path, qp, qv, query_id=0, jacp=False, jacr=False)
     for jp, jr in ((True, False), (False, True)):   # jacp / jacr without objects
         with pytest.raises(ValueError):
-            HQJ.query_jac(path, qp, qv, [SITE], [tcp], query_id=-1, jacp=jp, jacr=jr, M=True)
+            HC.query_jac(path, qp, qv, [SITE], [tcp], query_id=-1, jacp=jp, jacr=jr, M=True)
     with pytest.raises(ValueError):    # all outputs null
-        HQJ.query_jac(path, qp, qv, [SITE], [tcp], jacp=False, jacr=False, M=False, qfrc_bias=False)
+        HC.query_jac(path, qp, qv, [SITE], [tcp], jacp=False, jacr=False, M=False, qfrc_bias=False)
     with pytest.raises(ValueError):
-        HQJ.query_jac(path, qp, qv, jacp=False, jacr=False, M=False, qfrc_bias=False)
+        HC.query_jac(path, qp, qv, jacp=False, jacr=False, M=False, qfrc_bias=False)
     # the same objects with query_id = -1 are fine for M / qfrc_bias alone
-    HQJ.query_jac(path, qp, qv, [SITE], [tcp], query_id=-1, jacp=False, jacr=False)
+    HC.query_jac(path, qp, qv, [SITE], [tcp], query_id=-1, jacp=False, jacr=False)

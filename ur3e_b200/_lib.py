@@ -16,8 +16,6 @@ TERM_NONE, TERM_V2, TERM_V0 = 0, 1, 2
 NOISE_NONE, NOISE_LOW, NOISE_MED, NOISE_HIGH = 0, 1, 2, 3
 STAT_NAMES = ["episodes", "return_sum", "length_sum", "successes", "term_reach", "term_toppled", "term_collision", "truncations",
               "unstable_resets", "nefc_sum", "ncon_sum", "solver_iter_sum", "substeps", "overflow_steps", "pad_contact_steps", "steps"]
-MAXCON = 32
-CACHE_SIZE = 54
 NSENSOR = 46
 SENSOR_NCTRL = 7   # d.ctrl columns of the sensor record, [21, 28), zero past nu (utils.get_ctrl)
 
@@ -44,7 +42,7 @@ class ForwardOut(C.Structure):
 EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_model_info", "ur3e_model_name2id", "ur3e_model_id2name",
            "ur3e_model_array", "ur3e_model_num_warnings", "ur3e_model_warning", "ur3e_batch_create", "ur3e_batch_destroy", "ur3e_batch_reset",
            "ur3e_batch_step", "ur3e_batch_step_host", "ur3e_batch_get_state", "ur3e_batch_set_state", "ur3e_batch_stats", "ur3e_batch_set_sensor_buffer",
-           "ur3e_batch_debug_forward", "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
+           "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
            "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward"]
 
 _lib = None
@@ -77,7 +75,6 @@ def load():
     L.ur3e_batch_set_state.argtypes = [vp, vp, vp, vp, vp]
     L.ur3e_batch_stats.argtypes = [vp, vp, C.c_int, vp]
     L.ur3e_batch_set_sensor_buffer.argtypes = [vp, vp]
-    L.ur3e_batch_debug_forward.argtypes = [vp, i64, dp, dp, dp, dp, C.POINTER(C.c_int32), dp, dp]
     L.ur3e_batch_launch_count.restype = i64; L.ur3e_batch_launch_count.argtypes = [vp]
     L.ur3e_batch_kernel_info.argtypes = [vp] + [C.POINTER(C.c_int32)] * 4
     L.ur3e_batch_state_bytes.argtypes = [vp]

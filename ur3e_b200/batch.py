@@ -118,17 +118,6 @@ class SimBatch:
         v = self.stats(reset).cpu().numpy()
         return {k: float(v[i]) for i, k in enumerate(_lib.STAT_NAMES)}
 
-    def debug_forward(self, env=0):
-        """Forward pass (with constraint solve, zero ctrl) of one environment at its current state; float64 host copies."""
-        nv = self.model.nv
-        M = np.zeros((nv, nv)); bias = np.zeros(nv); qacc = np.zeros(nv); fc = np.zeros(nv)
-        info = np.zeros(8, dtype=np.int32); con = np.zeros((_lib.MAXCON, 4)); cache = np.zeros(_lib.CACHE_SIZE)
-        dp = lambda a: a.ctypes.data_as(C.POINTER(C.c_double))
-        torch.cuda.synchronize(self.device)
-        _lib.check(self._L.ur3e_batch_debug_forward(self.ptr, env, dp(M), dp(bias), dp(qacc), dp(fc), info.ctypes.data_as(C.POINTER(C.c_int32)), dp(con), dp(cache)), "ur3e_batch_debug_forward")
-        return dict(M=M, qfrc_bias=bias, qacc=qacc, qfrc_constraint=fc, ncon=int(info[0]), nefc=int(info[1]), solver_iter=int(info[2]),
-                    overflow=int(info[3]), contacts=con[:int(info[0])], tcp_pos=cache[:3], tcp_mat=cache[3:12].reshape(3, 3), J_arm=cache[12:48].reshape(6, 6), bias_arm=cache[48:54])
-
     def query(self, objects):
         """A kinematics query over a fixed list of objects: [(kind, name_or_id), ...] with kind "body" (inertial frame, d.xipos /
         d.ximat), "xbody" (body frame, d.xpos / d.xmat, what d.body(name).xpos returns), "geom" or "site".  See Query."""
@@ -139,16 +128,10 @@ class SimBatch:
         output not asked for.  One launch on the current torch stream; the output convention and the semantics are Query.jac's
         (this is Query.jac without objects)."""
         nv = self.model.nv
-        own = self.__dict__.setdefault("_mass_own", {})
-        outs = (_out(self, own, "M", M, (self.n, nv, nv)), _out(self, own, "qfrc_bias", qfrc_bias, (self.n, nv)))
-        if all(o is None for o in outs):
-            raise ValueError("mass_matrix needs at least one of M, qfrc_bias")
-        self._query_jac(-1, (None, None) + outs)
-        return outs
-
-    def _query_jac(self, query_id, outs):
-        p = [C.c_void_p(o.data_ptr()) if o is not None else None for o in outs]
-        _lib.check(self._L.ur3e_batch_query_jac(self.ptr, query_id, p[0], p[1], p[2], p[3], self._stream()), "ur3e_batch_query_jac")
+        outs = _outs(self, self.__dict__.setdefault("_mass_own", {}), "mass_matrix",
+                     dict(M=(M, (self.n, nv, nv), None), qfrc_bias=(qfrc_bias, (self.n, nv), None)))
+        _lib.check(self._L.ur3e_batch_query_jac(self.ptr, -1, None, None, *map(_ptr, outs.values()), self._stream()), "ur3e_batch_query_jac")
+        return tuple(outs.values())
 
     @property
     def max_contacts(self):
@@ -184,20 +167,16 @@ class SimBatch:
         the last substep before integration (SURVEY F9); these are one substep newer, the state query() sees.
         """
         n, nv, Cn = self.n, self.model.nv, self.max_contacts
-        own = self.__dict__.setdefault("_forward_own", {})
         i32 = torch.int32
-        spec = dict(qacc=((n, nv), None), qfrc_constraint=((n, nv), None), info=((n, 4), i32), contact_geom=((n, Cn, 2), i32),
-                    contact_dist=((n, Cn), None), contact_pos=((n, Cn, 3), None), contact_frame=((n, Cn, 3, 3), None),
-                    contact_force=((n, Cn, 6), None), flags=((n,), i32), sensordata=((n, _lib.NSENSOR), None))
-        args = dict(qacc=qacc, qfrc_constraint=qfrc_constraint, info=info, contact_geom=contact_geom, contact_dist=contact_dist,
-                    contact_pos=contact_pos, contact_frame=contact_frame, contact_force=contact_force, flags=flags, sensordata=sensordata)
+        table = dict(qacc=(qacc, (n, nv), None), qfrc_constraint=(qfrc_constraint, (n, nv), None), info=(info, (n, 4), i32),
+                     contact_geom=(contact_geom, (n, Cn, 2), i32), contact_dist=(contact_dist, (n, Cn), None),
+                     contact_pos=(contact_pos, (n, Cn, 3), None), contact_frame=(contact_frame, (n, Cn, 3, 3), None),
+                     contact_force=(contact_force, (n, Cn, 6), None), flags=(flags, (n,), i32), sensordata=(sensordata, (n, _lib.NSENSOR), None))
         if Cn == 0:
-            asked = [k for k in args if k.startswith("contact_") and args[k] is not False and args[k] is not None]
+            asked = [k for k, (a, _, _) in table.items() if k.startswith("contact_") and a is not False and a is not None]
             if asked:
                 raise ValueError("%s: the model has no contact pairs (max_contacts = 0)" % ", ".join(asked))
-        outs = ForwardResult(*[_out(self, own, k, args[k], *spec[k]) for k in _lib.FORWARD_OUTPUTS])
-        if all(o is None for o in outs):
-            raise ValueError("forward needs at least one output")
+        outs = ForwardResult(**_outs(self, self.__dict__.setdefault("_forward_own", {}), "forward", table))
         u = None
         if ctrl is not None:
             nu = self.model.nu
@@ -286,17 +265,11 @@ class Query:
         self.id = qid
         self._own = {}
 
-    def _out(self, name, arg, shape):
-        return _out(self.batch, self._own, name, arg, shape)
-
     def __call__(self, pos=True, mat=False, vel=False, local=False):
         n, k = self.batch.n, self.k
-        outs = (self._out("pos", pos, (n, k, 3)), self._out("mat", mat, (n, k, 3, 3)), self._out("vel", vel, (n, k, 6)))
-        if all(o is None for o in outs):
-            raise ValueError("a query needs at least one of pos, mat, vel")
-        p = [C.c_void_p(o.data_ptr()) if o is not None else None for o in outs]
-        _lib.check(self.batch._L.ur3e_batch_query(self.batch.ptr, self.id, p[0], p[1], p[2], int(bool(local)), self.batch._stream()), "ur3e_batch_query")
-        return outs
+        outs = _outs(self.batch, self._own, "a query", dict(pos=(pos, (n, k, 3), None), mat=(mat, (n, k, 3, 3), None), vel=(vel, (n, k, 6), None)))
+        _lib.check(self.batch._L.ur3e_batch_query(self.batch.ptr, self.id, *map(_ptr, outs.values()), int(bool(local)), self.batch._stream()), "ur3e_batch_query")
+        return tuple(outs.values())
 
     def jac(self, jacp=True, jacr=False, M=False, qfrc_bias=False):
         """Jacobians of the k objects, with the mass matrix and the bias forces (ur3e_batch_query_jac): one launch on the current
@@ -313,22 +286,31 @@ class Query:
         cache the fused task-space controllers read; these are one substep newer, the same state __call__ sees.
         """
         n, k, nv = self.batch.n, self.k, self.batch.model.nv
-        outs = (self._out("jacp", jacp, (n, k, 3, nv)), self._out("jacr", jacr, (n, k, 3, nv)), self._out("M", M, (n, nv, nv)),
-                self._out("qfrc_bias", qfrc_bias, (n, nv)))
-        if all(o is None for o in outs):
-            raise ValueError("Query.jac needs at least one of jacp, jacr, M, qfrc_bias")
-        self.batch._query_jac(self.id, outs)
-        return outs
+        outs = _outs(self.batch, self._own, "Query.jac", dict(jacp=(jacp, (n, k, 3, nv), None), jacr=(jacr, (n, k, 3, nv), None),
+                                                              M=(M, (n, nv, nv), None), qfrc_bias=(qfrc_bias, (n, nv), None)))
+        _lib.check(self.batch._L.ur3e_batch_query_jac(self.batch.ptr, self.id, *map(_ptr, outs.values()), self.batch._stream()), "ur3e_batch_query_jac")
+        return tuple(outs.values())
 
 
-def _out(batch, own, name, arg, shape, dtype=None):
-    """An output argument: False / None (not wanted), True (a tensor kept in `own`, overwritten by the next call) or a caller tensor.
-    dtype: the output's element type (default: the batch's)."""
-    if arg is False or arg is None:
-        return None
-    if arg is True:
-        if name not in own:
-            own[name] = torch.empty(shape, dtype=dtype or batch.dtype, device=batch.device)
-        return own[name]
-    batch._chk(arg, shape, dtype)
-    return arg
+def _outs(batch, own, what, table):
+    """Output arguments {name: (arg, shape, dtype)}: each is False / None (not wanted), True (a tensor kept in `own` under its
+    name, overwritten by the next call) or a caller tensor, checked; dtype None is the batch's.  Returns {name: tensor or None} in
+    the table's order; raises ValueError when no output is wanted."""
+    outs = {}
+    for name, (arg, shape, dtype) in table.items():
+        if arg is False or arg is None:
+            outs[name] = None
+        elif arg is True:
+            if name not in own:
+                own[name] = torch.empty(shape, dtype=dtype or batch.dtype, device=batch.device)
+            outs[name] = own[name]
+        else:
+            batch._chk(arg, shape, dtype)
+            outs[name] = arg
+    if all(o is None for o in outs.values()):
+        raise ValueError("%s needs at least one of %s" % (what, ", ".join(table)))
+    return outs
+
+
+def _ptr(t):
+    return C.c_void_p(t.data_ptr()) if t is not None else None

@@ -27,7 +27,6 @@ struct BatchBase {
   virtual int set_state(const void* qpos, const void* qvel, const void* ws, cudaStream_t s) = 0;
   virtual int stats(double* out, int reset, cudaStream_t s) = 0;
   virtual int set_sensor_buffer(void* buf) = 0;
-  virtual int debug(long long env, double* M, double* bias, double* qacc, double* fc, int32_t* info, double* con, double* cache) = 0;
   // optional CUDA-event timing of every step-kernel launch (bench.py's roofline: the duration of the dominant kernel alone)
   virtual int kernel_timing(int enable) = 0;
   virtual int kernel_times(double* out6) = 0;   // {ms, launches} x {lite tier, grasp / generic tier on the caller's stream, generic tier on the side stream}; synchronises

@@ -25,7 +25,7 @@
 #endif
 
 namespace ur3e {
-enum Op { OP_STEP = 0, OP_RESET = 1, OP_SET_STATE = 2, OP_DEBUG = 3 };
+enum Op { OP_STEP = 0, OP_RESET = 1, OP_SET_STATE = 2 };
 
 template <typename Real>
 struct KArgs {
@@ -51,7 +51,6 @@ struct KArgs {
   const uint8_t* mask;
   unsigned long long seed, env_base;
   const Real* qpos_in; const Real* qvel_in; const Real* ws_in;
-  long long dbg_env; double* dbg;
 };
 
 template <typename Real, typename D> __host__ __device__ constexpr size_t arena_stride() { return (sizeof(Arena<Real, D>) + 15) / 16 * 16; }
@@ -69,15 +68,13 @@ template <typename Real, typename D> __host__ __device__ constexpr int warps_per
 #endif
   return w > UR3E_MAX_WPB ? UR3E_MAX_WPB : (w < 1 ? 1 : w);
 }
-constexpr int DBG_DOUBLES = MAXV * MAXV + 3 * MAXV + 8 + 4 * MAXCON + CACHE_SIZE;
 
 template <typename Real, typename D>
 __global__ void __launch_bounds__(warps_per_block<Real, D>() * 32) env_kernel(const KArgs<Real> a) {
   constexpr int WPB = warps_per_block<Real, D>();
   extern __shared__ int4 smem_raw[];
   const int warp = threadIdx.x >> 5;
-  long long e = (long long)blockIdx.x * WPB + warp;
-  if (a.op == OP_DEBUG) { if (blockIdx.x != 0 || warp != 0) return; e = a.dbg_env; }
+  const long long e = (long long)blockIdx.x * WPB + warp;
   if (e >= a.n) return;
   Arena<Real, D>& s = *reinterpret_cast<Arena<Real, D>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, D>());
   const DevModel<Real>& m = *a.m;
@@ -90,7 +87,7 @@ __global__ void __launch_bounds__(warps_per_block<Real, D>() * 32) env_kernel(co
   IF_LANE0 { s.overflow = 0; s.ncon = 0; s.nefc = 0; s.solver_iter = 0; s.cap_con = D::MAXCON; s.cap_efc = D::MAXEFC; }
   WARP_SYNC();
   const int od = c.obs_dim;
-  if (a.op != OP_DEBUG) { IF_LANE0 s.st.tier = 0; }   // a reset / injected state starts on the lite tier again
+  IF_LANE0 s.st.tier = 0;   // a reset / injected state starts on the lite tier again
   if (a.op == OP_RESET) {
     env_reset(m, c, s, a.opt, a.seed, a.env_base + (unsigned long long)e);
     ContactFlags cf = contact_flags(m, c, s);
@@ -102,23 +99,6 @@ __global__ void __launch_bounds__(warps_per_block<Real, D>() * 32) env_kernel(co
     WARP_SYNC();
     forward_cold(m, s, a.opt, false);
     update_cache(m, c, s);
-  } else {  // OP_DEBUG: full forward at the current state, dump internals of one environment
-    WARP_FOR(i, m.nu) s.ctrl[i] = 0;
-    WARP_SYNC();
-    forward_cold(m, s, a.opt, true);
-    update_cache(m, c, s);
-    double* o = a.dbg;
-    const int nv = m.nv;
-    WARP_FOR(i, nv * nv) { int r = i / nv, c2 = i % nv, hi = r > c2 ? r : c2, lo = r > c2 ? c2 : r; o[i] = (double)s.M[hi * (hi + 1) / 2 + lo]; }
-    o += MAXV * MAXV;
-    WARP_FOR(i, nv) { o[i] = (double)s.qfrc_bias[i]; o[MAXV + i] = (double)s.qacc[i]; o[2 * MAXV + i] = (double)s.qfrc_constraint[i]; }
-    o += 3 * MAXV;
-    IF_LANE0 { o[0] = s.ncon; o[1] = s.nefc; o[2] = s.solver_iter; o[3] = s.overflow; o[4] = s.ne; o[5] = s.nf; o[6] = s.nl; o[7] = 0; }
-    o += 8;
-    if constexpr (D::HAS_CONTACT) { WARP_FOR(i, s.ncon) { o[4 * i] = (double)s.con_dist[i]; for (int k = 0; k < 3; ++k) o[4 * i + 1 + k] = (double)s.con_pos[i][k]; } }
-    o += 4 * MAXCON;
-    WARP_FOR(i, CACHE_SIZE) o[i] = (double)s.st.cache[i];
-    return;  // debug does not modify the stored state
   }
   WARP_SYNC();
   WARP_FOR(i, NW) gst[i] = sst[i];
@@ -343,7 +323,7 @@ struct Batch : BatchBase {
   HostModel hm;
   int act_dim = 0, obs_dim = 0;
   // staging for the host-buffer entry point
-  Real *d_act = nullptr, *d_obs = nullptr, *d_rew = nullptr; uint8_t *d_term = nullptr, *d_trunc = nullptr; double* d_dbg = nullptr;
+  Real *d_act = nullptr, *d_obs = nullptr, *d_rew = nullptr; uint8_t *d_term = nullptr, *d_trunc = nullptr;
   cudaStream_t own_stream = nullptr, own_stream2 = nullptr;
   uint64_t seed = 0;
   int sm_count = 148;
@@ -352,7 +332,7 @@ struct Batch : BatchBase {
     cudaSetDevice(device);
     cudaFree(d_ovf_count); cudaFree(d_ovf_list); cudaFree(d_ovf_list2); cudaFree(d_ovf_list3);
     for (int k = 0; k < 4; ++k) { if (aux_stream[k]) cudaStreamDestroy(aux_stream[k]); if (fork_ev[k]) cudaEventDestroy(fork_ev[k]); if (join_ev[k]) cudaEventDestroy(join_ev[k]); } if (h_ovf) cudaFreeHost(h_ovf); if (ovf_ev) cudaEventDestroy(ovf_ev); if (order_ev) cudaEventDestroy(order_ev);
-    cudaFree(d_model); cudaFree(d_consts); cudaFree(d_state); cudaFree(d_act); cudaFree(d_obs); cudaFree(d_rew); cudaFree(d_term); cudaFree(d_trunc); cudaFree(d_dbg);
+    cudaFree(d_model); cudaFree(d_consts); cudaFree(d_state); cudaFree(d_act); cudaFree(d_obs); cudaFree(d_rew); cudaFree(d_term); cudaFree(d_trunc);
     for (auto& t : timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
     for (auto e : ev_pool) cudaEventDestroy(e);
     for (auto& q : queries) cudaFree(q.table);
@@ -360,10 +340,10 @@ struct Batch : BatchBase {
     if (own_stream2) cudaStreamDestroy(own_stream2);
   }
   static constexpr int WPB = warps_per_block<Real, D>();
-  int launch(KArgs<Real>& a, cudaStream_t s, long long envs) {
-    size_t smem = arena_stride<Real, D>() * WPB;
-    unsigned blocks = (unsigned)((envs + WPB - 1) / WPB);
-    env_kernel<Real, D><<<blocks, WPB * 32, smem, s>>>(a);
+  // env_kernel and the queries: one warp per environment of the batch, one arena of class DA per warp
+  template <typename DA, typename A> int launch_warps(void (*kernel)(A), const A& a, cudaStream_t s) {
+    constexpr int W = warps_per_block<Real, DA>();
+    kernel<<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DA>() * W, s>>>(a);
     ++launches;
     CUDA_OK(cudaGetLastError());
     return 0;
@@ -448,6 +428,11 @@ struct Batch : BatchBase {
     CUDA_OK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, env_kernel<Real, D>, WPB * 32, smem));
     CUDA_OK(cudaFuncSetAttribute(step_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_OK(cudaFuncSetAttribute(step_kernel<Real, D, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_OK(cudaFuncSetAttribute(query_fwd_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    { using DK = QueryDims<D>;
+      const int qsmem = (int)(arena_stride<Real, DK>() * warps_per_block<Real, DK>());
+      CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
+      CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
     cudaDeviceProp prop; CUDA_OK(cudaGetDeviceProperties(&prop, dev)); sm_count = prop.multiProcessorCount;
     if constexpr (HAS_LITE) {
       constexpr int WL = warps_per_block<Real, DL>();
@@ -469,7 +454,7 @@ struct Batch : BatchBase {
     CUDA_OK(cudaSetDevice(device));
     seed = sd; last_stream = s;
     KArgs<Real> a = base; a.op = OP_RESET; a.mask = mask; a.seed = sd; a.obs = (Real*)obs;
-    return launch(a, s, n);
+    return launch_warps<D>(env_kernel<Real, D>, a, s);
   }
   // ---- optional per-launch timing (cudaEvent pairs on the launching stream)
   struct Timed { cudaEvent_t a, b; int tier; };
@@ -632,10 +617,6 @@ struct Batch : BatchBase {
     std::vector<QueryEntry<Real>> tab;
     const std::string err = compile_query<Real>(hm, objtype, objid, k, tab);
     if (!err.empty()) return set_err("query_create: " + err);
-    if (queries.empty()) {
-      using DK = QueryDims<D>;
-      CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(arena_stride<Real, DK>() * warps_per_block<Real, DK>())));
-    }
     Query q{nullptr, k};
     CUDA_OK(cudaMalloc(&q.table, sizeof(QueryEntry<Real>) * k));
     queries.push_back(q);
@@ -647,54 +628,30 @@ struct Batch : BatchBase {
     if (id < 0 || id >= (int)queries.size()) return set_err("query: unknown query id " + std::to_string(id));
     if (!pos && !mat && !vel) return set_err("query: all outputs are null");
     // a read-only call: last_stream (what step_host orders itself after) stays that of the latest state-changing call
-    using DK = QueryDims<D>;
-    constexpr int W = warps_per_block<Real, DK>();
     QArgs<Real, D> a{d_model, d_state, queries[id].table, queries[id].k, n, (Real*)pos, (Real*)mat, (Real*)vel, local != 0};
-    query_kernel<Real, D><<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DK>() * W, s>>>(a);
-    ++launches;
-    CUDA_OK(cudaGetLastError());
-    return 0;
+    return launch_warps<QueryDims<D>>(query_kernel<Real, D>, a, s);
   }
-  bool jac_ready = false;   // query_jac_kernel's shared-memory attribute is set
   int query_jac(int id, void* jacp, void* jacr, void* M, void* bias, cudaStream_t s) override {
     CUDA_OK(cudaSetDevice(device));
     const std::string err = query_jac_check(id, (int)queries.size(), jacp || jacr, jacp || jacr || M || bias);
     if (!err.empty()) return set_err("query_jac: " + err);
-    using DK = QueryDims<D>;
-    constexpr int W = warps_per_block<Real, DK>();
-    if (!jac_ready) {
-      CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(arena_stride<Real, DK>() * W)));
-      jac_ready = true;
-    }
     // read-only, like query(): last_stream stays that of the latest state-changing call
     QJArgs<Real, D> a{d_model, d_state, id >= 0 ? queries[id].table : nullptr, id >= 0 ? queries[id].k : 0, n, (Real*)jacp, (Real*)jacr, (Real*)M, (Real*)bias};
-    query_jac_kernel<Real, D><<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DK>() * W, s>>>(a);
-    ++launches;
-    CUDA_OK(cudaGetLastError());
-    return 0;
+    return launch_warps<QueryDims<D>>(query_jac_kernel<Real, D>, a, s);
   }
   static constexpr int NCMAX = D::HAS_CONTACT ? D::MAXCON : 0;
   int max_contacts() const override { return NCMAX; }
-  bool fwd_ready = false;   // query_fwd_kernel's shared-memory attribute is set
   int forward(const void* ctrl, const ur3e_forward_out* out, cudaStream_t s) override {
     CUDA_OK(cudaSetDevice(device));
     const bool con = out && (out->contact_geom || out->contact_dist || out->contact_pos || out->contact_frame || out->contact_force);
     const bool any = out && (con || out->qacc || out->qfrc_constraint || out->info || out->flags || out->sensordata);
     const std::string err = forward_query_check(out != nullptr, con, any, NCMAX);
     if (!err.empty()) return set_err("forward: " + err);
-    const size_t smem = arena_stride<Real, D>() * WPB;
-    if (!fwd_ready) {
-      CUDA_OK(cudaFuncSetAttribute(query_fwd_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-      fwd_ready = true;
-    }
     // read-only, like query(): last_stream stays that of the latest state-changing call
     QFArgs<Real, D> a{d_model, d_state, base.opt, n, (const Real*)ctrl,
                       FwdOut<Real>{(Real*)out->qacc, (Real*)out->qfrc_constraint, out->info, out->contact_geom, (Real*)out->contact_dist,
                                    (Real*)out->contact_pos, (Real*)out->contact_frame, (Real*)out->contact_force, out->flags, (Real*)out->sensordata}};
-    query_fwd_kernel<Real, D><<<(unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, s>>>(a);
-    ++launches;
-    CUDA_OK(cudaGetLastError());
-    return 0;
+    return launch_warps<D>(query_fwd_kernel<Real, D>, a, s);
   }
   int set_sensor_buffer(void* buf) override { sens_dev = buf; return 0; }
   int get_state(void* qpos, void* qvel, void* ws, cudaStream_t s) override {
@@ -711,7 +668,7 @@ struct Batch : BatchBase {
     if (!qpos || !qvel) return set_err("set_state: null buffer");
     last_stream = s;
     KArgs<Real> a = base; a.op = OP_SET_STATE; a.qpos_in = (const Real*)qpos; a.qvel_in = (const Real*)qvel; a.ws_in = (const Real*)ws;
-    return launch(a, s, n);
+    return launch_warps<D>(env_kernel<Real, D>, a, s);
   }
   int stats(double* out, int rst, cudaStream_t s) override {
     CUDA_OK(cudaSetDevice(device));
@@ -720,29 +677,6 @@ struct Batch : BatchBase {
     stats_kernel<Real, D><<<(unsigned)((n + 255) / 256), 256, 0, s>>>(d_state, n, out, rst);
     ++launches;
     CUDA_OK(cudaGetLastError());
-    return 0;
-  }
-  int debug(long long env, double* M, double* bias, double* qacc, double* fc, int32_t* info, double* con, double* cache) override {
-    CUDA_OK(cudaSetDevice(device));
-    if (env < 0 || env >= n) return set_err("debug: env out of range");
-    if (!d_dbg) CUDA_OK(cudaMalloc(&d_dbg, sizeof(double) * DBG_DOUBLES));
-    CUDA_OK(cudaMemset(d_dbg, 0, sizeof(double) * DBG_DOUBLES));
-    KArgs<Real> a = base; a.op = OP_DEBUG; a.dbg_env = env; a.dbg = d_dbg;
-    if (int rc = launch(a, 0, 1)) return rc;
-    std::vector<double> hbuf(DBG_DOUBLES);
-    CUDA_OK(cudaMemcpy(hbuf.data(), d_dbg, sizeof(double) * DBG_DOUBLES, cudaMemcpyDeviceToHost));
-    const int nv = hm.nv; const double* o = hbuf.data();
-    if (M) std::memcpy(M, o, sizeof(double) * nv * nv);
-    o += MAXV * MAXV;
-    if (bias) std::memcpy(bias, o, sizeof(double) * nv);
-    if (qacc) std::memcpy(qacc, o + MAXV, sizeof(double) * nv);
-    if (fc) std::memcpy(fc, o + 2 * MAXV, sizeof(double) * nv);
-    o += 3 * MAXV;
-    if (info) for (int k = 0; k < 8; ++k) info[k] = (int32_t)o[k];
-    o += 8;
-    if (con) std::memcpy(con, o, sizeof(double) * 4 * MAXCON);
-    o += 4 * MAXCON;
-    if (cache) std::memcpy(cache, o, sizeof(double) * CACHE_SIZE);
     return 0;
   }
 };

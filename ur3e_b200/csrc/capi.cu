@@ -85,9 +85,6 @@ int ur3e_batch_get_state(ur3e_batch* b, void* qp, void* qv, void* ws, void* stre
 int ur3e_batch_set_state(ur3e_batch* b, const void* qp, const void* qv, const void* ws, void* stream) { GUARD(b); return b->impl->set_state(qp, qv, ws, (cudaStream_t)stream); }
 int ur3e_batch_set_sensor_buffer(ur3e_batch* b, void* buf) { GUARD(b); return b->impl->set_sensor_buffer(buf); }
 int ur3e_batch_stats(ur3e_batch* b, double* out, int reset, void* stream) { GUARD(b); if (!out) return set_err("null stats buffer"); return b->impl->stats(out, reset, (cudaStream_t)stream); }
-int ur3e_batch_debug_forward(ur3e_batch* b, int64_t env, double* M, double* bias, double* qacc, double* fc, int32_t* info8, double* con, double* cache) {
-  GUARD(b); return b->impl->debug(env, M, bias, qacc, fc, info8, con, cache);
-}
 int64_t ur3e_batch_launch_count(const ur3e_batch* b) { return (b && b->impl) ? b->impl->launches : -1; }
 int ur3e_batch_kernel_info(const ur3e_batch* b, int32_t* arena_bytes, int32_t* wpb, int32_t* blocks_per_sm, int32_t* regs) {
   GUARD(b);
