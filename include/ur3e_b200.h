@@ -173,6 +173,34 @@ typedef struct ur3e_forward_out {
 } ur3e_forward_out;
 int ur3e_batch_max_contacts(const ur3e_batch* b);
 int ur3e_batch_forward(ur3e_batch* b, const void* ctrl_dev, const ur3e_forward_out* out, void* stream);
+/* Offscreen rendering: rgb_array / depth_array images (gymnasium MujocoEnv.render, ur3e_env2.py:25-28) and geom segmentation for
+ * selected environments, from a camera anchored to the world or to one object of the loaded model.
+ * ur3e_batch_render_create compiles a renderer and returns its id (>= 0); the batch owns it until ur3e_batch_destroy.
+ *   cam: anchor objtype -1 = world, UR3E_OBJ_XBODY (body frame) or UR3E_OBJ_SITE with a loaded-model id; pos and xyaxes (MJCF
+ *        <camera xyaxes>: x right, y up, the view along -z) in the anchor frame; fovy the vertical field of view in degrees
+ *        (0, 180); 0 < znear < zfar in metres.  The aspect ratio is width / height.
+ *   geom_ids [k], 1 <= k <= 256: the geoms drawn (box or plane, ids of the loaded model); rgba [k, 4] or NULL = the model's geom_rgba.
+ *   width, height in [1, 2048].
+ * Scene: all geoms opaque, no shadows, textures, reflections or anti-aliasing.  A plane with size (sx, sy) is |x| <= sx, |y| <= sy
+ * of its frame (0 = unbounded) and is seen only from its front (+z) side; boxes are solid, seen from outside.  Shading is a
+ * headlight, c = rgb * (0.3 + 0.7 * max(0, -n . d)) with d the unit ray, stored as the nearest uint8 of 255 * clamp(c, 0, 1);
+ * the background is black.  One ray per pixel centre, row 0 at the top.
+ * ur3e_batch_render renders m environments: env_ids_dev int32 [m] (device) or NULL = all (then m = n).  Outputs, any may be NULL,
+ * not all: rgb_dev uint8 [m, H, W, 3]; depth_dev [m, H, W] in the batch's dtype, z-depth in metres along the camera's view axis
+ * (what gymnasium's linearised depth_array returns, not the ray length), zfar for a miss or a hit beyond zfar, hits nearer than znear
+ * ignored; seg_dev int32 [m, H, W], the hit geom's id, -1 for background.  Equal hit distances go to the lower geom id.  An id
+ * outside [0, n) renders as background.  Asynchronous on `stream`, two kernel launches; the stored state is not modified.  The
+ * pose scratch is shared by a batch's renderers: calls on different streams must be ordered by the caller.
+ * Semantics: the images are of the STORED state, i.e. what MuJoCo's d.geom_xpos / d.geom_xmat hold after set_state / reset +
+ * mj_forward.  After a step, MuJoCo's arrays still hold the last substep's pre-integration kinematics (SURVEY F9); the image is one
+ * substep newer than those, the state ur3e_batch_query sees. */
+typedef struct ur3e_camera {
+  int32_t objtype, objid;   /* anchor: objtype -1 = world, else UR3E_OBJ_XBODY or UR3E_OBJ_SITE with a loaded-model id */
+  double pos[3], xyaxes[6]; /* in the anchor frame; view along -z */
+  double fovy, znear, zfar; /* degrees, metres */
+} ur3e_camera;
+int ur3e_batch_render_create(ur3e_batch* b, const ur3e_camera* cam, const int32_t* geom_ids, int32_t k, const float* rgba, int32_t width, int32_t height);
+int ur3e_batch_render(ur3e_batch* b, int render_id, const int32_t* env_ids_dev, int64_t m, uint8_t* rgb_dev, void* depth_dev, int32_t* seg_dev, void* stream);
 
 #ifdef __cplusplus
 }

@@ -39,11 +39,18 @@ class ForwardOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in FORWARD_OUTPUTS]
 
 
+class Camera(C.Structure):
+    """ur3e_camera: anchor (objtype -1 = world, OBJ_XBODY or OBJ_SITE; objid), pos / xyaxes in the anchor frame, fovy (degrees), znear, zfar."""
+    _fields_ = [("objtype", C.c_int32), ("objid", C.c_int32), ("pos", C.c_double * 3), ("xyaxes", C.c_double * 6), ("fovy", C.c_double),
+                ("znear", C.c_double), ("zfar", C.c_double)]
+
+
 EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_model_info", "ur3e_model_name2id", "ur3e_model_id2name",
            "ur3e_model_array", "ur3e_model_num_warnings", "ur3e_model_warning", "ur3e_batch_create", "ur3e_batch_destroy", "ur3e_batch_reset",
            "ur3e_batch_step", "ur3e_batch_step_host", "ur3e_batch_get_state", "ur3e_batch_set_state", "ur3e_batch_stats", "ur3e_batch_set_sensor_buffer",
            "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
-           "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward"]
+           "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward",
+           "ur3e_batch_render_create", "ur3e_batch_render"]
 
 _lib = None
 
@@ -87,6 +94,8 @@ def load():
     L.ur3e_batch_query_jac.argtypes = [vp, C.c_int, vp, vp, vp, vp, vp]
     L.ur3e_batch_max_contacts.argtypes = [vp]
     L.ur3e_batch_forward.argtypes = [vp, vp, C.POINTER(ForwardOut), vp]
+    L.ur3e_batch_render_create.argtypes = [vp, C.POINTER(Camera), C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_float), C.c_int32, C.c_int32]
+    L.ur3e_batch_render.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp]
     _lib = L
     return L
 

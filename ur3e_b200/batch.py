@@ -189,6 +189,12 @@ class SimBatch:
         _lib.check(self._L.ur3e_batch_forward(self.ptr, u, C.byref(st), self._stream()), "ur3e_batch_forward")
         return outs
 
+    def renderer(self, width, height, camera, geoms=None, rgba=None):
+        """An offscreen renderer of this batch (ur3e_batch_render_create): width x height images of `geoms` (names or ids of box /
+        plane geoms; None = every geom whose geom_rgba alpha is > 0) seen from `camera` (a dict, see make_camera).  rgba [k, 4]
+        overrides the model's geom_rgba per geom.  See Renderer."""
+        return Renderer(self, width, height, camera, geoms, rgba)
+
     @property
     def launch_count(self):
         return int(self._L.ur3e_batch_launch_count(self.ptr))
@@ -314,3 +320,103 @@ def _outs(batch, own, what, table):
 
 def _ptr(t):
     return C.c_void_p(t.data_ptr()) if t is not None else None
+
+
+def make_camera(model, camera):
+    """ur3e_camera from a dict, in one of two forms, both with fovy (vertical, degrees; 45), znear (0.01) and zfar (50.0) in metres:
+
+        {"pos": (3,), "xyaxes": (6,)} with optionally "body": name or id (the body frame) or "site": name or id -- MJCF <camera
+            pos xyaxes> in that anchor's frame (the world's without one): x right, y up, the view along -z;
+        {"lookat": (3,), "distance": d, "azimuth": az, "elevation": el} (degrees) -- gymnasium's default_camera_config keys, a world
+            camera in MuJoCo's free-camera parametrisation: forward f = (cos el cos az, cos el sin az, sin el), position
+            lookat - d f, up (-sin el cos az, -sin el sin az, cos el), right f x up.
+    """
+    cam = dict(camera)
+    c = _lib.Camera()
+    c.fovy = float(cam.pop("fovy", 45.0)); c.znear = float(cam.pop("znear", 0.01)); c.zfar = float(cam.pop("zfar", 50.0))
+    c.objtype, c.objid = -1, 0
+    if "lookat" in cam:
+        lookat = np.asarray(cam.pop("lookat"), dtype=np.float64)
+        dist = float(cam.pop("distance")); az = np.radians(float(cam.pop("azimuth"))); el = np.radians(float(cam.pop("elevation")))
+        f = np.array([np.cos(el) * np.cos(az), np.cos(el) * np.sin(az), np.sin(el)])
+        up = np.array([-np.sin(el) * np.cos(az), -np.sin(el) * np.sin(az), np.cos(el)])
+        pos, xyaxes = lookat - dist * f, np.concatenate([np.cross(f, up), up])
+    else:
+        pos = np.asarray(cam.pop("pos"), dtype=np.float64); xyaxes = np.asarray(cam.pop("xyaxes"), dtype=np.float64)
+        for kind, t in (("body", _lib.OBJ_XBODY), ("site", _lib.OBJ_SITE)):
+            if kind in cam:
+                obj = cam.pop(kind)
+                i = model.name2id(_lib.OBJ_BODY if kind == "body" else t, obj) if isinstance(obj, str) else int(obj)
+                if i < 0:
+                    raise KeyError("%s %r is not in the model" % (kind, obj))
+                c.objtype, c.objid = t, i
+    if cam:
+        raise ValueError("unknown camera keys %s" % sorted(cam))
+    if pos.shape != (3,) or xyaxes.shape != (6,):
+        raise ValueError("camera pos needs 3 numbers and xyaxes 6")
+    for i in range(3):
+        c.pos[i] = pos[i]
+    for i in range(6):
+        c.xyaxes[i] = xyaxes[i]
+    return c
+
+
+def default_geoms(model):
+    """Ids of the geoms a renderer draws by default: every geom whose geom_rgba alpha is > 0."""
+    return [int(i) for i in np.nonzero(np.asarray(model.array("geom_rgba")).reshape(-1, 4)[:, 3] > 0)[0]]
+
+
+class Renderer:
+    """Offscreen RGB, depth and geom-segmentation images of selected environments (ur3e_batch_render).
+
+    Calling it launches two kernels on the current torch stream and returns (rgb [m, H, W, 3] uint8, depth [m, H, W] in the batch's
+    dtype, seg [m, H, W] int32), None for an output not asked for; each output argument is False, True (a tensor owned by the
+    renderer, overwritten by its next call) or a caller tensor of that shape to write into.  env_ids is an int32 CUDA tensor [m]
+    (None = every environment); an id outside [0, n) renders as background.  Row 0 is the top of the image.
+
+    depth is the z-depth in metres along the camera's view axis (gymnasium's linearised depth_array, not the ray length); a miss or
+    a hit beyond zfar reports zfar and hits nearer than znear are ignored.  seg is the hit geom's id in the model, -1 for background.
+    Geoms are opaque boxes and planes (a plane is seen only from its front side) under a headlight, rgb * (0.3 + 0.7 max(0, -n.d)),
+    on black; no shadows, textures or anti-aliasing.
+
+    The images are of the stored state: what MuJoCo's d.geom_xpos / d.geom_xmat hold after reset or set_state + mj_forward.  After a
+    step MuJoCo's arrays still hold the last substep's pre-integration kinematics (SURVEY F9); the images are one substep newer than
+    those, the state query() sees.  A batch's renderers share one pose scratch: calls on different streams must be ordered.
+    """
+
+    def __init__(self, batch, width, height, camera, geoms=None, rgba=None):
+        self.batch, self.width, self.height = batch, int(width), int(height)
+        ids = default_geoms(batch.model) if geoms is None else []
+        for g in (geoms if geoms is not None else []):
+            i = batch.model.name2id(_lib.OBJ_GEOM, g) if isinstance(g, str) else int(g)
+            if i < 0:
+                raise KeyError("geom %r is not in the model" % (g,))
+            ids.append(i)
+        self.geoms, self.k = ids, len(ids)
+        self.camera = make_camera(batch.model, camera)
+        col = None
+        if rgba is not None:
+            col = np.ascontiguousarray(rgba, dtype=np.float32)
+            if col.shape != (self.k, 4):
+                raise ValueError("rgba must be [k, 4] = [%d, 4], got %s" % (self.k, col.shape))
+        g = (C.c_int32 * max(self.k, 1))(*ids)
+        rid = batch._L.ur3e_batch_render_create(batch.ptr, C.byref(self.camera), g, self.k,
+                                                col.ctypes.data_as(C.POINTER(C.c_float)) if col is not None else None, self.width, self.height)
+        if rid < 0:
+            raise ValueError("ur3e_batch_render_create: " + _lib.last_error())
+        self.id = rid
+        self._own = {}
+
+    def __call__(self, env_ids=None, rgb=True, depth=False, seg=False):
+        b = self.batch
+        if env_ids is None:
+            m, ep = b.n, None
+        else:
+            m = int(env_ids.numel())
+            ep = b._chk(env_ids, (m,), torch.int32)
+        H, W = self.height, self.width
+        for name in [k for k, t in self._own.items() if t.shape[0] != m]:
+            del self._own[name]   # owned outputs follow the latest call's m
+        outs = _outs(b, self._own, "Renderer", dict(rgb=(rgb, (m, H, W, 3), torch.uint8), depth=(depth, (m, H, W), None), seg=(seg, (m, H, W), torch.int32)))
+        _lib.check(b._L.ur3e_batch_render(b.ptr, self.id, ep, m, *map(_ptr, outs.values()), b._stream()), "ur3e_batch_render")
+        return tuple(outs.values())

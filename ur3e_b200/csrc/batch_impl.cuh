@@ -13,6 +13,7 @@
 #include "env.cuh"
 #include "query.cuh"
 #include "query_fwd.cuh"
+#include "render.cuh"
 
 #ifndef UR3E_BLOCKS_PER_SM
 #define UR3E_BLOCKS_PER_SM 2
@@ -299,6 +300,77 @@ __global__ void __launch_bounds__(warps_per_block<Real, D>() * 32, 1) query_fwd_
   forward_query_env(m, s, a.opt, a.ctrl ? a.ctrl + e * m.nu : nullptr, o);
 }
 
+template <typename Real, typename D>
+struct RPArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;
+  const QueryEntry<Real>* q; int k;   // k geoms, then the camera
+  long long n, count;                 // batch size, selected environments
+  const int* env_ids;                 // [count] or null (environment i)
+  Real* pose;                         // [count, k + 1, 12]
+};
+
+// Render pose pass (render.cuh render_pose_env): one warp per selected environment on the kinematics queries' arena; reads qpos of
+// the record, writes the world poses of the renderer's geoms and camera.  An environment id outside [0, n) gets no pose (the pixel
+// pass draws background for it).
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) render_pose_kernel(const RPArgs<Real, D> a) {
+  using DK = QueryDims<D>;
+  constexpr int WPB = warps_per_block<Real, DK>();
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long i = (long long)blockIdx.x * WPB + warp;
+  if (i >= a.count) return;
+  const long long e = a.env_ids ? (long long)a.env_ids[i] : i;
+  if (e < 0 || e >= a.n) return;
+  Arena<Real, DK>& s = *reinterpret_cast<Arena<Real, DK>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, DK>());
+  const DevModel<Real>& m = *a.m;
+  const EnvState<Real, D>& rec = a.st[e];
+  WARP_FOR(j, m.nq) s.st.qpos[j] = rec.qpos[j];
+  WARP_SYNC();
+  render_pose_env(m, s, a.q, a.k, a.pose + i * 12 * (a.k + 1));
+}
+
+template <typename Real>
+struct RArgs {
+  const RenderGeom<Real>* geoms; int k;
+  RenderCam<Real> cam;
+  const Real* pose;                   // [m, k + 1, 12] from render_pose_kernel
+  const int* env_ids; long long n;
+  unsigned char* rgb; Real* depth; int* seg;   // [m, H, W, 3], [m, H, W], [m, H, W]; any may be null
+};
+
+constexpr int RENDER_THREADS = 256, RENDER_TILE = 1024;   // pixels per block: the staged scene is shared by RENDER_TILE rays
+// Render pixel pass (render.cuh render_pixel): block (i, tile) stages environment i's camera and geoms in shared memory, then each
+// thread casts the rays of its pixels; outputs are written along image rows.
+template <typename Real>
+__global__ void __launch_bounds__(RENDER_THREADS) render_kernel(const RArgs<Real> a) {
+  extern __shared__ int4 smem_raw[];
+  const int k = a.k;
+  Real* sp = reinterpret_cast<Real*>(smem_raw);
+  RenderGeom<Real>* sg = reinterpret_cast<RenderGeom<Real>*>(sp + 12 * (k + 1));
+  const long long i = blockIdx.x;
+  const long long e = a.env_ids ? (long long)a.env_ids[i] : i;
+  const bool valid = e >= 0 && e < a.n;   // uniform over the block
+  if (valid) {
+    const Real* src = a.pose + i * 12 * (k + 1);
+    for (int t = threadIdx.x; t < 12 * (k + 1); t += blockDim.x) sp[t] = src[t];
+    for (int t = threadIdx.x; t < k; t += blockDim.x) sg[t] = a.geoms[t];
+  }
+  __syncthreads();
+  const int W = a.cam.width, npx = W * a.cam.height;
+  const int p0 = blockIdx.y * RENDER_TILE, p1 = p0 + RENDER_TILE < npx ? p0 + RENDER_TILE : npx;
+  for (int p = p0 + threadIdx.x; p < p1; p += blockDim.x) {
+    RenderPixel<Real> r;
+    if (valid) r = render_pixel(a.cam, sp, sg, k, p % W, p / W);
+    else { r.depth = a.cam.zfar; r.seg = -1; r.rgb[0] = r.rgb[1] = r.rgb[2] = 0; }
+    const long long o = i * npx + p;
+    if (a.rgb) { a.rgb[3 * o] = r.rgb[0]; a.rgb[3 * o + 1] = r.rgb[1]; a.rgb[3 * o + 2] = r.rgb[2]; }
+    if (a.depth) a.depth[o] = r.depth;
+    if (a.seg) a.seg[o] = r.seg;
+  }
+}
+
 // D: generic size class of the model family; DL: lite twin (small caps, exact-fit) or D; DM: grasp-tier twin (caps between DL's and D's,
 // exact-fit) or D.  Tiers hand environments up through device-side lists: DL -> DM -> D.
 template <typename Real, typename D, typename DL = D, typename DM = D>
@@ -336,14 +408,18 @@ struct Batch : BatchBase {
     for (auto& t : timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
     for (auto e : ev_pool) cudaEventDestroy(e);
     for (auto& q : queries) cudaFree(q.table);
+    for (auto& r : renders) { cudaFree(r.table); cudaFree(r.geoms); }
+    cudaFree(d_pose);
     if (own_stream) cudaStreamDestroy(own_stream);
     if (own_stream2) cudaStreamDestroy(own_stream2);
   }
   static constexpr int WPB = warps_per_block<Real, D>();
   // env_kernel and the queries: one warp per environment of the batch, one arena of class DA per warp
-  template <typename DA, typename A> int launch_warps(void (*kernel)(A), const A& a, cudaStream_t s) {
+  // (count: how many environments the kernel runs, the batch's n when 0)
+  template <typename DA, typename A> int launch_warps(void (*kernel)(A), const A& a, cudaStream_t s, long long count = 0) {
     constexpr int W = warps_per_block<Real, DA>();
-    kernel<<<(unsigned)((n + W - 1) / W), W * 32, arena_stride<Real, DA>() * W, s>>>(a);
+    const long long c = count > 0 ? count : n;
+    kernel<<<(unsigned)((c + W - 1) / W), W * 32, arena_stride<Real, DA>() * W, s>>>(a);
     ++launches;
     CUDA_OK(cudaGetLastError());
     return 0;
@@ -432,7 +508,9 @@ struct Batch : BatchBase {
     { using DK = QueryDims<D>;
       const int qsmem = (int)(arena_stride<Real, DK>() * warps_per_block<Real, DK>());
       CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
-      CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
+      CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
+      CUDA_OK(cudaFuncSetAttribute(render_pose_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
+    static_assert(sizeof(Real) * 12 * (RENDER_MAX_GEOMS + 1) + sizeof(RenderGeom<Real>) * RENDER_MAX_GEOMS <= 48 * 1024, "render_kernel's staged scene fits the default shared-memory limit");
     cudaDeviceProp prop; CUDA_OK(cudaGetDeviceProperties(&prop, dev)); sm_count = prop.multiProcessorCount;
     if constexpr (HAS_LITE) {
       constexpr int WL = warps_per_block<Real, DL>();
@@ -652,6 +730,45 @@ struct Batch : BatchBase {
                       FwdOut<Real>{(Real*)out->qacc, (Real*)out->qfrc_constraint, out->info, out->contact_geom, (Real*)out->contact_dist,
                                    (Real*)out->contact_pos, (Real*)out->contact_frame, (Real*)out->contact_force, out->flags, (Real*)out->sensordata}};
     return launch_warps<D>(query_fwd_kernel<Real, D>, a, s);
+  }
+  // ---- offscreen rendering (render.cuh); renderers and the pose scratch live until the batch is destroyed
+  struct Render { QueryEntry<Real>* table; RenderGeom<Real>* geoms; int k; RenderCam<Real> cam; };
+  std::vector<Render> renders;
+  Real* d_pose = nullptr; long long pose_cap = 0;   // [m, k + 1, 12] of the latest call, grown to the largest seen
+  static size_t render_smem(int k) { return sizeof(Real) * 12 * (k + 1) + sizeof(RenderGeom<Real>) * k; }
+  int render_create(const ur3e_camera* cam, const int32_t* geom_ids, int k, const float* rgba, int width, int height) override {
+    CUDA_OK(cudaSetDevice(device));
+    std::vector<QueryEntry<Real>> tab; std::vector<RenderGeom<Real>> geoms; RenderCam<Real> rc{};
+    const std::string err = compile_render<Real>(hm, cam, geom_ids, k, rgba, width, height, tab, geoms, rc);
+    if (!err.empty()) return set_err("render_create: " + err);
+    Render r{nullptr, nullptr, k, rc};
+    CUDA_OK(cudaMalloc(&r.table, sizeof(QueryEntry<Real>) * (k + 1)));
+    if (cudaMalloc(&r.geoms, sizeof(RenderGeom<Real>) * k) != cudaSuccess) { cudaFree(r.table); return set_err("render_create: out of device memory", -2); }
+    renders.push_back(r);
+    CUDA_OK(cudaMemcpy(r.table, tab.data(), sizeof(QueryEntry<Real>) * (k + 1), cudaMemcpyHostToDevice));
+    CUDA_OK(cudaMemcpy(r.geoms, geoms.data(), sizeof(RenderGeom<Real>) * k, cudaMemcpyHostToDevice));
+    return (int)renders.size() - 1;
+  }
+  int render(int id, const int32_t* env_ids, long long m, uint8_t* rgb, void* depth, int32_t* seg, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const std::string err = render_check(id, (int)renders.size(), rgb || depth || seg, m, n, env_ids != nullptr);
+    if (!err.empty()) return set_err("render: " + err);
+    const Render& r = renders[id];
+    const long long need = m * 12 * (r.k + 1);
+    if (need > pose_cap) {
+      // cudaFree waits for the device, so a call still reading the old scratch finishes first
+      CUDA_OK(cudaFree(d_pose)); d_pose = nullptr; pose_cap = 0;
+      CUDA_OK(cudaMalloc(&d_pose, sizeof(Real) * need)); pose_cap = need;
+    }
+    // read-only, like query(): last_stream stays that of the latest state-changing call
+    RPArgs<Real, D> pa{d_model, d_state, r.table, r.k, n, m, env_ids, d_pose};
+    if (int rc = launch_warps<QueryDims<D>>(render_pose_kernel<Real, D>, pa, s, m)) return rc;
+    RArgs<Real> ra{r.geoms, r.k, r.cam, d_pose, env_ids, n, rgb, (Real*)depth, seg};
+    const unsigned tiles = (unsigned)((r.cam.width * r.cam.height + RENDER_TILE - 1) / RENDER_TILE);
+    render_kernel<Real><<<dim3((unsigned)m, tiles), RENDER_THREADS, render_smem(r.k), s>>>(ra);
+    ++launches;
+    CUDA_OK(cudaGetLastError());
+    return 0;
   }
   int set_sensor_buffer(void* buf) override { sens_dev = buf; return 0; }
   int get_state(void* qpos, void* qvel, void* ws, cudaStream_t s) override {

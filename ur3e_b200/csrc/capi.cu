@@ -119,5 +119,12 @@ int ur3e_batch_max_contacts(const ur3e_batch* b) { GUARD(b); return b->impl->max
 int ur3e_batch_forward(ur3e_batch* b, const void* ctrl, const ur3e_forward_out* out, void* stream) {
   GUARD(b); return b->impl->forward(ctrl, out, (cudaStream_t)stream);
 }
+int ur3e_batch_render_create(ur3e_batch* b, const ur3e_camera* cam, const int32_t* geom_ids, int32_t k, const float* rgba, int32_t width, int32_t height) {
+  GUARD(b);
+  try { return b->impl->render_create(cam, geom_ids, k, rgba, width, height); } catch (const std::exception& e) { return set_err(e.what()); }
+}
+int ur3e_batch_render(ur3e_batch* b, int render_id, const int32_t* env_ids_dev, int64_t m, uint8_t* rgb_dev, void* depth_dev, int32_t* seg_dev, void* stream) {
+  GUARD(b); return b->impl->render(render_id, env_ids_dev, m, rgb_dev, depth_dev, seg_dev, (cudaStream_t)stream);
+}
 
 }  // extern "C"

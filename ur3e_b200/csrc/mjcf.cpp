@@ -98,7 +98,7 @@ struct Builder {
   V jpos, jaxis, jrange, jarm, jdamp, jfl, jstiff, jspringref, jref, jmargin, jsolref, jsolimp;
   // geom
   std::vector<std::string> gname; std::vector<int> gtype, gbody, gcontype, gconaff, gcondim, gprio;
-  V gpos, gquat, gsize, gfriction, gsolref, gsolimp, gsolmix, gmargin, ggap;
+  V gpos, gquat, gsize, gfriction, gsolref, gsolimp, gsolmix, gmargin, ggap, grgba;
   // site
   std::vector<std::string> sname; std::vector<int> sbody; V spos, squat, ssize;
 
@@ -156,6 +156,7 @@ struct Builder {
         push(gfriction, floats(a, "friction", 3, {1, 0.005, 0.0001}));
         push(gsolref, floats(a, "solref", 2, kSolref)); push(gsolimp, floats(a, "solimp", 5, kSolimp));
         gsolmix.push_back(num(a, "solmix", 1)); gmargin.push_back(num(a, "margin", 0)); ggap.push_back(num(a, "gap", 0));
+        push(grgba, floats(a, "rgba", 4, {0.5, 0.5, 0.5, 1}));   // MuJoCo's default; offscreen rendering only
         if (gt == GEOM_BOX) {
           double vol = 8 * sz[0] * sz[1] * sz[2];
           double mass = has(a, "mass") ? num(a, "mass", 0) : num(a, "density", 1000) * vol;
@@ -429,6 +430,7 @@ HostModel load_mjcf(const std::string& path) {
   set_array(m, "geom_conaffinity", B.gconaff, {ng}); set_array(m, "geom_condim", B.gcondim, {ng}); set_array(m, "geom_priority", B.gprio, {ng});
   set_array(m, "geom_friction", B.gfriction, {ng, 3}); set_array(m, "geom_solref", B.gsolref, {ng, 2}); set_array(m, "geom_solimp", B.gsolimp, {ng, 5});
   set_array(m, "geom_solmix", B.gsolmix, {ng}); set_array(m, "geom_margin", B.gmargin, {ng}); set_array(m, "geom_gap", B.ggap, {ng});
+  set_array(m, "geom_rgba", B.grgba, {ng, 4});
   set_array(m, "site_bodyid", B.sbody, {ns}); set_array(m, "site_pos", B.spos, {ns, 3}); set_array(m, "site_quat", B.squat, {ns, 4}); set_array(m, "site_size", B.ssize, {ns, 3});
 
   // tendons (fixed)

@@ -16,6 +16,18 @@ namespace ur3e {
 // query runs kinematics only, so it fits more environments per SM than the step)
 template <typename D> using QueryDims = Dims<D::NB, D::NV, D::NQ, D::NU, D::NG, D::NPAIR, 0, 0, D::SPLIT>;
 
+// World frame of a compiled entry after kinematics(): position xpos[a] + R_a lpos, and element (r, c) of R_a lmat
+template <typename Real, typename D>
+UR3E_HD void entry_point(const Arena<Real, D>& s, const QueryEntry<Real>& o, Real* p) {
+  Real v[3]; mat_vec3(v, s.fr.k.xmat[o.body], o.lpos);
+  for (int c = 0; c < 3; ++c) p[c] = s.xpos[o.body][c] + v[c];
+}
+template <typename Real, typename D>
+UR3E_HD Real entry_rot(const Arena<Real, D>& s, const QueryEntry<Real>& o, int r, int c) {
+  const Real* Ra = s.fr.k.xmat[o.body] + 3 * r; const Real* L = o.lmat + c;
+  return Ra[0] * L[0] + Ra[1] * L[3] + Ra[2] * L[6];
+}
+
 // pos [k][3], mat [k][9] (row-major), vel [k][6] = [rot(3), lin(3)] of this environment; any may be null.  local != 0: velocities
 // in the object's frame (mj_objectVelocity's flg_local).
 template <typename Real, typename D>
@@ -33,10 +45,7 @@ UR3E_HD void query_env(const DevModel<Real>& m, Arena<Real, D>& s, const QueryEn
   }
   const auto& xmat = s.fr.k.xmat;
   // world position of object j: xpos[a] + R_a lpos
-  auto point = [&](const QueryEntry<Real>& o, Real* p) {
-    Real v[3]; mat_vec3(v, xmat[o.body], o.lpos);
-    for (int c = 0; c < 3; ++c) p[c] = s.xpos[o.body][c] + v[c];
-  };
+  auto point = [&](const QueryEntry<Real>& o, Real* p) { entry_point(s, o, p); };
   if (pos) {
     WARP_FOR(i, 3 * k) {
       const int j = i / 3, r = i - 3 * j;

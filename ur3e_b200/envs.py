@@ -20,6 +20,11 @@ import torch
 
 from . import _lib, presets
 from .batch import SimBatch
+
+# UR3eEnv's camera when no default_camera_config is given: a constant world camera that frames the arm (base at the origin, ~0.5 m
+# reach) and the mug's reset region (x 0.3 .. 0.45, y 0.13 .. 0.38 on the table), looking along +y and 45 degrees down.  It is not
+# derived from MuJoCo's model statistics (stat.center / stat.extent), so it does not match MuJoCo's default free camera.
+DEFAULT_CAMERA_CONFIG = {"lookat": (0.25, 0.2, 0.15), "distance": 1.4, "azimuth": 90.0, "elevation": -45.0, "fovy": 45.0}
 from .model import Model, asset
 
 ENV_IDS = tuple(presets.ENV_SPECS.keys())
@@ -69,14 +74,20 @@ _SB3VecEnvBase = _optional_base("stable_baselines3.common.vec_env", "VecEnv")
 class UR3eVecEnv(_VectorEnvBase):
     """N environments of one of the reference's four ids on one GPU (torch API; a gymnasium.vector.VectorEnv when gymnasium imports)."""
 
-    metadata = {"render_modes": [], "autoreset_mode": "same_step"}
+    metadata = {"render_modes": ["rgb_array", "depth_array"], "autoreset_mode": "same_step"}
 
-    def __init__(self, env_id="gymnasium_env/ur3e-v2", num_envs=1, device=0, dtype=torch.float32, auto_reset=True, env_id_base=0, render_mode=None, **config_overrides):
+    def __init__(self, env_id="gymnasium_env/ur3e-v2", num_envs=1, device=0, dtype=torch.float32, auto_reset=True, env_id_base=0, render_mode=None,
+                 width=480, height=480, default_camera_config=None, camera_id=None, camera_name=None, **config_overrides):
         if env_id not in presets.ENV_SPECS:
             raise ValueError("unknown env id %r (known: %s)" % (env_id, ", ".join(ENV_IDS)))
+        if camera_id is not None or camera_name is not None:
+            raise ValueError("camera_id / camera_name: the model's <camera> elements are not loaded; use default_camera_config")
         xml, kw, _, _ = presets.ENV_SPECS[env_id]
         self.env_id, self.num_envs = env_id, int(num_envs)
-        self.render_mode = render_mode      # accepted for call compatibility (train_rl.py:41); nothing is rendered
+        self.render_mode = render_mode      # "rgb_array" / "depth_array" render (render()); None and "human" (train_rl.py:41) render nothing
+        self.width, self.height = int(width), int(height)
+        self.default_camera_config = dict(DEFAULT_CAMERA_CONFIG if default_camera_config is None else default_camera_config)
+        self._renderer = None
         self.model = Model(asset(xml))
         self.cfg = presets.make_config(self.model, kw, auto_reset=int(bool(auto_reset)), env_id_base=env_id_base, **config_overrides)
         self.batch = SimBatch(self.model, self.cfg, self.num_envs, device, dtype)
@@ -107,6 +118,19 @@ class UR3eVecEnv(_VectorEnvBase):
         obs, rew, term, trunc = self.batch.step(actions)
         return obs, rew, term.bool(), trunc.bool(), {"final_obs": self.batch.final_obs}
 
+    def render(self, env_ids=None):
+        """Images of the stored state (see ur3e_b200.batch.Renderer) on the device: render_mode "rgb_array" gives uint8 [m, H, W, 3],
+        "depth_array" the z-depth [m, H, W] in metres; env_ids (int32 CUDA tensor [m]) selects environments, None = all.  The
+        camera is default_camera_config (UR3eVecEnv.DEFAULT_CAMERA_CONFIG when none was given).  Any other render_mode returns None.
+        The returned tensor is owned by the env and overwritten by the next call."""
+        if self.render_mode not in ("rgb_array", "depth_array"):
+            return None
+        if self._renderer is None:
+            self._renderer = self.batch.renderer(self.width, self.height, self.default_camera_config)
+        rgb = self.render_mode == "rgb_array"
+        out = self._renderer(env_ids, rgb=rgb, depth=not rgb)
+        return out[0] if rgb else out[1]
+
     def set_state(self, qpos, qvel):
         """MujocoEnv.set_state for every env (qpos [N,nq], qvel [N,nv])."""
         self.batch.set_state(qpos, qvel)
@@ -129,8 +153,10 @@ class UR3eEnv(_EnvBase):
 
     metadata = {"render_modes": ["human", "rgb_array", "depth_array"]}
 
-    def __init__(self, env_id="gymnasium_env/ur3e-v2", render_mode=None, device=0, dtype=torch.float64, **config_overrides):
-        self.venv = UR3eVecEnv(env_id, 1, device, dtype, auto_reset=False, render_mode=render_mode, **config_overrides)
+    def __init__(self, env_id="gymnasium_env/ur3e-v2", render_mode=None, device=0, dtype=torch.float64, width=480, height=480, default_camera_config=None,
+                 camera_id=None, camera_name=None, **config_overrides):
+        self.venv = UR3eVecEnv(env_id, 1, device, dtype, auto_reset=False, render_mode=render_mode, width=width, height=height,
+                               default_camera_config=default_camera_config, camera_id=camera_id, camera_name=camera_name, **config_overrides)
         self.observation_space, self.action_space = self.venv.single_observation_space, self.venv.single_action_space
         self.render_mode = render_mode
         self.metadata = dict(self.metadata, render_fps=self.venv.metadata["render_fps"])
@@ -148,7 +174,14 @@ class UR3eEnv(_EnvBase):
         return obs[0].double().cpu().numpy(), float(rew[0].item()), bool(term[0].item()), bool(trunc[0].item()), {}
 
     def render(self):
-        return None
+        """gymnasium MujocoEnv.render: render_mode "rgb_array" gives a (height, width, 3) uint8 numpy image, "depth_array" a
+        (height, width) float64 z-depth in metres, of the stored state (ur3e_b200.batch.Renderer); None and "human" (no viewer)
+        give None.  width / height (480) and default_camera_config are constructor arguments as in MujocoEnv; without a
+        default_camera_config the camera is the constant DEFAULT_CAMERA_CONFIG, not MuJoCo's model-statistics free camera."""
+        img = self.venv.render()
+        if img is None:
+            return None
+        return img[0].cpu().numpy() if self.render_mode == "rgb_array" else img[0].double().cpu().numpy()
 
     def close(self):
         self.venv.close()
@@ -229,7 +262,12 @@ class SB3VecEnv(_SB3VecEnvBase):
         return [False for _ in self._indices(indices)]
 
     def get_images(self):
-        return [None] * self.num_envs
+        """One (H, W, 3) uint8 numpy image per environment when the wrapped env's render_mode is "rgb_array" (SB3's
+        VecEnv.render("rgb_array") and VecVideoRecorder ask for every environment's image: all N are rendered and copied to the
+        host), else [None] * n."""
+        if self.render_mode != "rgb_array":
+            return [None] * self.num_envs
+        return list(self.venv.render().cpu().numpy())
 
     def close(self):
         self.venv.close()
