@@ -539,9 +539,13 @@ UR3E_HD int clip_poly(const Real* px, const Real* py, int n, Real* ox, Real* oy,
   return k;
 }
 
-// box-box manifold; same rules as the oracle's box_box (oracle/ur3e_oracle.c), normal from box 1 to box 2
+// box-box manifold; same rules as the oracle's box_box (oracle/ur3e_oracle.c), normal from box 1 to box 2.
+// `out` is the slot's staging row (STAGE_W values, shared memory).  On entry it holds the two world frames (R1 = out[0, 9),
+// R2 = out[9, 18)), so that no argument is passed by address from the caller's stack; the frames are dead once the
+// clipping starts, and the row then holds one of the two clip polygons until the contact points overwrite it.
 template <typename Real>
-UR3E_PHASE int box_box(const Real* p1, const Real* R1, const Real* s1, const Real* p2, const Real* R2, const Real* s2, Real margin, Real* out) {
+UR3E_PHASE int box_box(const Real* p1, const Real* s1, const Real* p2, const Real* s2, Real margin, Real* out) {
+  const Real* const R1 = out; const Real* const R2 = out + 9;
   Real d[3] = {p2[0] - p1[0], p2[1] - p1[1], p2[2] - p1[2]}, A1[3][3], A2[3][3];
   for (int i = 0; i < 3; ++i) for (int k = 0; k < 3; ++k) { A1[i][k] = R1[3 * k + i]; A2[i][k] = R2[3 * k + i]; }
   Real AC[3][3];
@@ -605,7 +609,8 @@ UR3E_PHASE int box_box(const Real* p1, const Real* R1, const Real* s1, const Rea
     px[c] = dot3(r, RAu); py[c] = dot3(r, RAv);
   }
   int n = 4;
-  Real qx[16], qy[16];
+  static_assert(STAGE_W >= 2 * 16, "the second clip polygon lives in the staging row");
+  Real* const qx = out; Real* const qy = out + 16;   // the frames are dead from here on (IAa / RAu / ... hold what is still needed)
   n = clip_poly(px, py, n, qx, qy, Real(1), Real(0), rs[ru]); n = clip_poly(qx, qy, n, px, py, Real(-1), Real(0), rs[ru]);
   n = clip_poly(px, py, n, qx, qy, Real(0), Real(1), rs[rv]); n = clip_poly(qx, qy, n, px, py, Real(0), Real(-1), rs[rv]);
   if (n == 0) return 0;
@@ -664,12 +669,17 @@ UR3E_HD void collision(const DevModel<Real>& m, Arena<Real, D>& s) {
       const int p = s.act_pair[a], g1 = m.pair_g1[p], g2 = m.pair_g2[p];
       const Real margin = m.pair_margin[p];
       Real R1[9], R2[9];
-      const Real x1[3] = {s.cu.gpos[g1][0], s.cu.gpos[g1][1], s.cu.gpos[g1][2]}, x2[3] = {s.cu.gpos[g2][0], s.cu.gpos[g2][1], s.cu.gpos[g2][2]};
       mat_mul3(R1, s.fr.k.xmat[m.geom_body[g1]], m.geom_mat[g1]); mat_mul3(R2, s.fr.k.xmat[m.geom_body[g2]], m.geom_mat[g2]);
       Real* st = s.u.stage[a];
       int n;
-      if (m.geom_kind[g1] == GK_PLANE) n = plane_box(x1, R1, x2, R2, m.geom_size[g2], margin, st);
-      else n = box_box(x1, R1, m.geom_size[g1], x2, R2, m.geom_size[g2], margin, st);
+      if (m.geom_kind[g1] == GK_PLANE) {
+        const Real x1[3] = {s.cu.gpos[g1][0], s.cu.gpos[g1][1], s.cu.gpos[g1][2]}, x2[3] = {s.cu.gpos[g2][0], s.cu.gpos[g2][1], s.cu.gpos[g2][2]};
+        n = plane_box(x1, R1, x2, R2, m.geom_size[g2], margin, st);
+      } else {
+        // the out-of-line box_box takes everything through the arena: arrays passed by address would live on the stack
+        for (int k = 0; k < 9; ++k) { st[k] = R1[k]; st[9 + k] = R2[k]; }
+        n = box_box(s.cu.gpos[g1], m.geom_size[g1], s.cu.gpos[g2], m.geom_size[g2], margin, st);
+      }
       int keep = 0;   // MuJoCo keeps a contact only when dist < margin
       for (int c = 0; c < n; ++c) if (st[3 + 4 * c + 3] < margin) { if (keep != c) for (int k = 0; k < 4; ++k) st[3 + 4 * keep + k] = st[3 + 4 * c + k]; ++keep; }
       s.stage_n[a] = (uint8_t)keep;
