@@ -201,6 +201,40 @@ typedef struct ur3e_camera {
 } ur3e_camera;
 int ur3e_batch_render_create(ur3e_batch* b, const ur3e_camera* cam, const int32_t* geom_ids, int32_t k, const float* rgba, int32_t width, int32_t height);
 int ur3e_batch_render(ur3e_batch* b, int render_id, const int32_t* env_ids_dev, int64_t m, uint8_t* rgb_dev, void* depth_dev, int32_t* seg_dev, void* stream);
+/* Rollouts (mujoco.rollout): m independent copies of environments of the batch, each stepped T env-steps with the given actions,
+ * with every step's outputs; the batch itself is left untouched.  For lookahead: sampling-based MPC (predictive sampling, MPPI,
+ * CEM), lookahead rewards, "what if" evaluation.
+ * Source, exactly one of:
+ *   src_env_ids_dev int32 [m]: rollout j starts from a copy of environment src[j]'s whole record (state, solver warm start, the
+ *     controller's stale-kinematics cache, episode step counter t and tier word), so that its steps are bit-identical to what
+ *     ur3e_batch_step would do to environment src[j] with the same actions, up to its first done.  Ids may repeat and m may exceed
+ *     n (K branches per environment).  An id outside [0, n) starts from a bad (NaN) state, which the step's own guard
+ *     (mj_checkPos/Vel) resets to qpos0 at the first substep; info[j, 0] >= 1 reports it.
+ *   qpos0_dev [m, nq], qvel0_dev [m, nv] and optionally qacc_warmstart0_dev [m, nv] (NULL = zero): rollout j starts as
+ *     ur3e_batch_set_state leaves a fresh record (forward pass, fresh cache, t = 0, tier 0).
+ * Dynamics: T env-steps of the batch's own environment (controller, frame_skip, observation, reward, termination, truncation); a
+ * UR3E_CTRL_RAW batch with frame_skip 1 gives mujoco.rollout's semantics.  There is no auto-reset: after a done the rollout keeps
+ * stepping and the flags are whatever the environment computes (v2 keeps reporting truncated once t >= max_steps); callers mask the
+ * steps after the first done.
+ * actions_dev [T, m, act_dim] (batch dtype).  Outputs, time-major (step t's outputs are the contiguous [m, ...] slice t; transpose
+ * the first two axes for mujoco.rollout's [nroll, nstep, ...]), device pointers, any may be NULL, not all:
+ *   qpos [T, m, nq], qvel [T, m, nv]: the state after each env-step; obs [T, m, obs_dim], reward [T, m], terminated / truncated
+ *   uint8 [T, m]: what ur3e_batch_step returns; sensordata [T, m, UR3E_NSENSOR]: the step's logging record (ur3e_batch_set_sensor_buffer)
+ *   from each env-step's last mj_step; info int32 [m, 2]: env-steps with a bad-state reset (mj_checkPos/Vel/Acc), env-steps with an
+ *   overflow of the contact / row caps.
+ * Rejected: m < 1 or m > 2^31 - 1, T < 1, actions NULL, both sources or neither, qpos0 without qvel0 or the reverse, a warm start
+ * without qpos0, out NULL, every output NULL.
+ * Asynchronous on `stream`: T tiered steps (the kernels of ur3e_batch_step) on a scratch copy.  The batch's records, statistics,
+ * attached sensor buffer and ur3e_batch_tier_info's counts are not modified (only the launch count grows); like the queries, the call
+ * does not become the stream ur3e_batch_step_host orders itself after.  A batch's rollouts share one workspace (grown to the largest
+ * m seen): calls on different streams must be ordered by the caller. */
+typedef struct ur3e_rollout_out {
+  void* qpos; void* qvel; void* obs; void* reward;
+  uint8_t* terminated; uint8_t* truncated;
+  void* sensordata; int32_t* info;
+} ur3e_rollout_out;
+int ur3e_batch_rollout(ur3e_batch* b, const int32_t* src_env_ids_dev, const void* qpos0_dev, const void* qvel0_dev, const void* qacc_warmstart0_dev,
+                       int64_t m, int32_t T, const void* actions_dev, const ur3e_rollout_out* out, void* stream);
 
 #ifdef __cplusplus
 }

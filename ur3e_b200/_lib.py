@@ -39,6 +39,14 @@ class ForwardOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in FORWARD_OUTPUTS]
 
 
+# ur3e_rollout_out: the eight device pointers of ur3e_batch_rollout, in this order (ROLLOUT_OUTPUTS)
+ROLLOUT_OUTPUTS = ("qpos", "qvel", "obs", "reward", "terminated", "truncated", "sensordata", "info")
+
+
+class RolloutOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ROLLOUT_OUTPUTS]
+
+
 class Camera(C.Structure):
     """ur3e_camera: anchor (objtype -1 = world, OBJ_XBODY or OBJ_SITE; objid), pos / xyaxes in the anchor frame, fovy (degrees), znear, zfar."""
     _fields_ = [("objtype", C.c_int32), ("objid", C.c_int32), ("pos", C.c_double * 3), ("xyaxes", C.c_double * 6), ("fovy", C.c_double),
@@ -50,7 +58,7 @@ EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_mod
            "ur3e_batch_step", "ur3e_batch_step_host", "ur3e_batch_get_state", "ur3e_batch_set_state", "ur3e_batch_stats", "ur3e_batch_set_sensor_buffer",
            "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
            "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward",
-           "ur3e_batch_render_create", "ur3e_batch_render"]
+           "ur3e_batch_render_create", "ur3e_batch_render", "ur3e_batch_rollout"]
 
 _lib = None
 
@@ -96,6 +104,7 @@ def load():
     L.ur3e_batch_forward.argtypes = [vp, vp, C.POINTER(ForwardOut), vp]
     L.ur3e_batch_render_create.argtypes = [vp, C.POINTER(Camera), C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_float), C.c_int32, C.c_int32]
     L.ur3e_batch_render.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp]
+    L.ur3e_batch_rollout.argtypes = [vp, vp, vp, vp, vp, i64, C.c_int32, vp, C.POINTER(RolloutOut), vp]
     _lib = L
     return L
 

@@ -34,6 +34,7 @@ def env_config(**kw):
 
 
 ForwardResult = namedtuple("ForwardResult", _lib.FORWARD_OUTPUTS)
+RolloutResult = namedtuple("RolloutResult", _lib.ROLLOUT_OUTPUTS)
 
 
 class SimBatch:
@@ -194,6 +195,61 @@ class SimBatch:
         plane geoms; None = every geom whose geom_rgba alpha is > 0) seen from `camera` (a dict, see make_camera).  rgba [k, 4]
         overrides the model's geom_rgba per geom.  See Renderer."""
         return Renderer(self, width, height, camera, geoms, rgba)
+
+    def rollout(self, actions, env_ids=None, state=None, qpos=False, qvel=False, obs=True, reward=True, terminated=True, truncated=True,
+                sensordata=False, info=False):
+        """mujoco.rollout for this batch (ur3e_batch_rollout): m copies of environments stepped T env-steps with `actions`, leaving
+        the batch untouched.  Returns a RolloutResult named tuple with None for every output not asked for; outputs follow
+        forward()'s convention (False, True = a tensor owned by the batch, reallocated when (T, m) changes, or a caller tensor).
+
+            actions [T, m, act_dim]            contiguous, the batch's dtype; step t's actions are actions[t]
+            env_ids int32 [m] (CUDA)           rollout j starts from a copy of environment env_ids[j]'s whole record, so it is
+                                               bit-identical to stepping that environment with the same actions up to its first
+                                               done; ids may repeat and m may exceed n.  An id outside [0, n) starts from a bad
+                                               state that the step resets to qpos0 (info[j, 0] >= 1)
+            state (qpos [m, nq], qvel [m, nv][, qacc_warmstart [m, nv]])   or rollouts start as set_state leaves a fresh record
+            neither                            every environment branched once (m = n)
+
+            qpos [T, m, nq], qvel [T, m, nv]   the state after each env-step
+            obs [T, m, obs_dim], reward [T, m], terminated, truncated uint8 [T, m]   what step returns
+            sensordata [T, m, 46]              the step's sensor record (enable_sensors) from each env-step's last mj_step
+            info int32 [m, 2]                  env-steps with a bad-state reset, env-steps with a contact / row overflow
+
+        There is no auto-reset: after a done the rollout keeps stepping and the flags are what the environment computes; mask the
+        steps after the first done.  Time-major: .transpose(0, 1) gives mujoco.rollout's [nroll, nstep, ...].  The call runs the
+        step kernels T times on the current torch stream; the batch's records, statistics and sensor buffer are not modified.  A
+        batch's rollouts share one workspace: calls on different streams must be ordered.
+        """
+        if env_ids is not None and state is not None:
+            raise ValueError("rollout: give env_ids or state, not both")
+        if actions.dim() != 3:
+            raise ValueError("rollout: actions must be [T, m, act_dim], got shape %s" % (tuple(actions.shape),))
+        T = int(actions.shape[0])
+        ids = qp = qv = ws = None
+        if state is not None:
+            if len(state) not in (2, 3):
+                raise ValueError("rollout: state is (qpos, qvel) or (qpos, qvel, qacc_warmstart)")
+            m = int(state[0].shape[0])
+            qp = self._chk(state[0], (m, self.model.nq)); qv = self._chk(state[1], (m, self.model.nv))
+            ws = self._chk(state[2], (m, self.model.nv)) if len(state) == 3 and state[2] is not None else None
+        else:
+            if env_ids is None:
+                if getattr(self, "_all_ids", None) is None:
+                    self._all_ids = torch.arange(self.n, dtype=torch.int32, device=self.device)
+                env_ids = self._all_ids
+            m = int(env_ids.numel())
+            ids = self._chk(env_ids, (m,), torch.int32)
+        a = self._chk(actions, (T, m, self.act_dim))
+        if getattr(self, "_rollout_tm", None) != (T, m):
+            self._rollout_own, self._rollout_tm = {}, (T, m)   # owned outputs follow the latest call's (T, m)
+        u8, i32 = torch.uint8, torch.int32
+        table = dict(qpos=(qpos, (T, m, self.model.nq), None), qvel=(qvel, (T, m, self.model.nv), None), obs=(obs, (T, m, self.obs_dim), None),
+                     reward=(reward, (T, m), None), terminated=(terminated, (T, m), u8), truncated=(truncated, (T, m), u8),
+                     sensordata=(sensordata, (T, m, _lib.NSENSOR), None), info=(info, (m, 2), i32))
+        outs = RolloutResult(**_outs(self, self._rollout_own, "rollout", table))
+        st = _lib.RolloutOut(*[o.data_ptr() if o is not None else None for o in outs])
+        _lib.check(self._L.ur3e_batch_rollout(self.ptr, ids, qp, qv, ws, m, T, a, C.byref(st), self._stream()), "ur3e_batch_rollout")
+        return outs
 
     @property
     def launch_count(self):

@@ -41,6 +41,9 @@ struct BatchBase {
   // offscreen rendering (render.cuh): the batch owns its renderers and their pose scratch; render_create returns the renderer's id
   virtual int render_create(const ur3e_camera* cam, const int32_t* geom_ids, int k, const float* rgba, int width, int height) = 0;
   virtual int render(int id, const int32_t* env_ids, long long m, uint8_t* rgb, void* depth, int32_t* seg, cudaStream_t s) = 0;
+  // T tiered steps of m scratch copies of records (src ids) or of fresh records (qpos0 / qvel0 / ws0); the batch is not modified
+  virtual int rollout(const int32_t* src, const void* qpos0, const void* qvel0, const void* ws0, long long m, int T, const void* act,
+                      const ur3e_rollout_out* out, cudaStream_t s) = 0;
   int64_t launches = 0;
   virtual void tier_steps(int64_t* lite, int64_t* full) const { *lite = 0; *full = 0; }
   virtual int64_t last_overflow() const { return 0; }

@@ -4,6 +4,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <limits>
 #include <type_traits>
 #include <vector>
 
@@ -14,6 +15,7 @@
 #include "query.cuh"
 #include "query_fwd.cuh"
 #include "render.cuh"
+#include "rollout.h"
 
 #ifndef UR3E_BLOCKS_PER_SM
 #define UR3E_BLOCKS_PER_SM 2
@@ -200,6 +202,46 @@ __global__ void stats_kernel(EnvState<Real, D>* st, long long n, double* out, in
   }
 }
 
+// Rollout sources: one warp per rollout j copies record ids[j] of the batch with 128-bit accesses, as step_kernel loads it, and zeroes
+// the copy's stat[] counters (rollout_info_kernel reads them; the step never reads them, so no trajectory changes).  An id outside
+// [0, n) gets a bad state instead: NaN qpos / qvel / warm start / cache, zero elsewhere, which the step's mj_checkPos/Vel guard resets
+// to qpos0 at the first substep and counts in stat[ST_UNSTABLE].
+template <typename Real, typename D>
+__global__ void rollout_gather_kernel(const EnvState<Real, D>* src, long long n, const int* ids, EnvState<Real, D>* dst, long long m) {
+  const long long j = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int lane = threadIdx.x & 31;
+  if (j >= m) return;
+  constexpr int NW = sizeof(EnvState<Real, D>) / 16;
+  const long long e = ids[j];
+  int4* d = reinterpret_cast<int4*>(dst + j);
+  const bool valid = e >= 0 && e < n;
+  if (valid) {
+    const int4* g = reinterpret_cast<const int4*>(src + e);
+    for (int i = lane; i < NW; i += 32) d[i] = g[i];
+  } else {
+    for (int i = lane; i < NW; i += 32) d[i] = make_int4(0, 0, 0, 0);
+  }
+  __syncwarp();
+  EnvState<Real, D>& r = dst[j];
+  if (valid) {
+    if (lane < NSTAT) r.stat[lane].i = 0;
+  } else {
+    const Real nan = std::numeric_limits<Real>::quiet_NaN();
+    for (int i = lane; i < D::NQ; i += 32) r.qpos[i] = nan;
+    for (int i = lane; i < D::NV; i += 32) { r.qvel[i] = nan; r.qacc_ws[i] = nan; }
+    for (int i = lane; i < CACHE_SIZE; i += 32) r.cache[i] = nan;
+  }
+}
+
+// Rollout info: env-steps with a bad-state reset and env-steps with an overflow, counted by the step in the scratch records since the gather.
+template <typename Real, typename D>
+__global__ void rollout_info_kernel(const EnvState<Real, D>* st, long long m, int32_t* info) {
+  const long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (j >= m) return;
+  info[2 * j] = st[j].stat[ST_UNSTABLE].i;
+  info[2 * j + 1] = st[j].stat[ST_OVERFLOW].i;
+}
+
 template <typename Real, typename D>
 struct QArgs {
   const DevModel<Real>* m;
@@ -379,7 +421,9 @@ struct Batch : BatchBase {
   static constexpr bool HAS_MID = !std::is_same<D, DM>::value;
   static_assert(sizeof(EnvState<Real, D>) == sizeof(EnvState<Real, DM>), "all size classes of a model must share the record layout");
   int *d_ovf_list2 = nullptr, *d_ovf_list3 = nullptr;
-  cudaStream_t aux_stream[4] = {nullptr, nullptr, nullptr, nullptr}; cudaEvent_t fork_ev[4] = {nullptr, nullptr, nullptr, nullptr}, join_ev[4] = {nullptr, nullptr, nullptr, nullptr};
+  // overflow-counter slots, each with its own side stream and events: one per range of step_host (slot 0 is also step's), then the rollouts'
+  static constexpr int HOST_CHUNKS = 4, ROLLOUT_SLOT = HOST_CHUNKS, NSLOT = HOST_CHUNKS + 1;
+  cudaStream_t aux_stream[NSLOT] = {}; cudaEvent_t fork_ev[NSLOT] = {}, join_ev[NSLOT] = {};
   static_assert(sizeof(EnvState<Real, D>) == sizeof(EnvState<Real, DL>), "lite and full size classes must share the record layout");
   int *d_ovf_count = nullptr, *d_ovf_list = nullptr, *h_ovf = nullptr; cudaEvent_t ovf_ev = nullptr, order_ev = nullptr; bool ovf_pending = false; int h_ovf_seen = 0;
   cudaStream_t last_stream = nullptr;   // stream of the latest asynchronous call on this handle (step_host orders itself after it)
@@ -403,13 +447,13 @@ struct Batch : BatchBase {
   ~Batch() override {
     cudaSetDevice(device);
     cudaFree(d_ovf_count); cudaFree(d_ovf_list); cudaFree(d_ovf_list2); cudaFree(d_ovf_list3);
-    for (int k = 0; k < 4; ++k) { if (aux_stream[k]) cudaStreamDestroy(aux_stream[k]); if (fork_ev[k]) cudaEventDestroy(fork_ev[k]); if (join_ev[k]) cudaEventDestroy(join_ev[k]); } if (h_ovf) cudaFreeHost(h_ovf); if (ovf_ev) cudaEventDestroy(ovf_ev); if (order_ev) cudaEventDestroy(order_ev);
+    for (int k = 0; k < NSLOT; ++k) { if (aux_stream[k]) cudaStreamDestroy(aux_stream[k]); if (fork_ev[k]) cudaEventDestroy(fork_ev[k]); if (join_ev[k]) cudaEventDestroy(join_ev[k]); } if (h_ovf) cudaFreeHost(h_ovf); if (ovf_ev) cudaEventDestroy(ovf_ev); if (order_ev) cudaEventDestroy(order_ev);
     cudaFree(d_model); cudaFree(d_consts); cudaFree(d_state); cudaFree(d_act); cudaFree(d_obs); cudaFree(d_rew); cudaFree(d_term); cudaFree(d_trunc);
     for (auto& t : timed) { cudaEventDestroy(t.a); cudaEventDestroy(t.b); }
     for (auto e : ev_pool) cudaEventDestroy(e);
     for (auto& q : queries) cudaFree(q.table);
     for (auto& r : renders) { cudaFree(r.table); cudaFree(r.geoms); }
-    cudaFree(d_pose);
+    cudaFree(d_pose); cudaFree(d_roll);
     if (own_stream) cudaStreamDestroy(own_stream);
     if (own_stream2) cudaStreamDestroy(own_stream2);
   }
@@ -516,7 +560,7 @@ struct Batch : BatchBase {
       constexpr int WL = warps_per_block<Real, DL>();
       CUDA_OK(cudaFuncSetAttribute(step_kernel<Real, DL>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(arena_stride<Real, DL>() * WL)));
       CUDA_OK(cudaFuncSetAttribute(step_kernel<Real, DL, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(arena_stride<Real, DL>() * WL)));
-      CUDA_OK(cudaMalloc(&d_ovf_count, sizeof(int) * 4 * HOST_CHUNKS)); CUDA_OK(cudaMalloc(&d_ovf_list, sizeof(int) * n_envs));
+      CUDA_OK(cudaMalloc(&d_ovf_count, sizeof(int) * 4 * NSLOT)); CUDA_OK(cudaMalloc(&d_ovf_list, sizeof(int) * n_envs));
       CUDA_OK(cudaMallocHost(&h_ovf, sizeof(int))); *h_ovf = 0;
       CUDA_OK(cudaEventCreateWithFlags(&ovf_ev, cudaEventDisableTiming));
       cudaFuncAttributes fl; CUDA_OK(cudaFuncGetAttributes(&fl, step_kernel<Real, DL>));
@@ -571,16 +615,28 @@ struct Batch : BatchBase {
     CUDA_OK(cudaSetDevice(device));
     if (!act || !obs || !rew || !term || !trunc) return set_err("step: null buffer");
     last_stream = s;
-    return step_range(act, obs, rew, term, trunc, fobs, s, 0, n, 0);
+    return step_range(live_range(0, n, 0), act, obs, rew, term, trunc, fobs, s);
   }
-  // Steps the environments [lo, lo + cnt) (buffers are the whole batch's; `slot` selects the overflow counter, so that
-  // ranges stepped concurrently on different streams do not share one).
-  int step_range(const void* act, void* obs, void* rew, uint8_t* term, uint8_t* trunc, void* fobs, cudaStream_t s, long long lo, long long cnt, int slot) {
+  // What one tiered step runs on: `cnt` records at `st`; the overflow counters, side stream and events of `slot` (so that targets
+  // stepped concurrently on different streams share none) and its tier lists ([cnt] each); the sensor output (null = none); the
+  // global id of the first record (auto-reset noise).  `live`: the batch's own records, auto-reset as configured and counted in
+  // tier_info; otherwise a rollout's scratch records, never auto-reset.
+  struct StepTarget { EnvState<Real, D>* st; long long cnt; int slot; int *list1, *list2, *list3; Real* sens; unsigned long long env_base; bool live; };
+  // the batch's environments [lo, lo + cnt)
+  StepTarget live_range(long long lo, long long cnt, int slot) const {
+    auto at = [lo](int* l) { return l ? l + lo : nullptr; };
+    return {d_state + lo, cnt, slot, at(d_ovf_list), at(d_ovf_list2), at(d_ovf_list3), sens_dev ? (Real*)sens_dev + lo * NSENSOR : nullptr,
+            base.env_base + (unsigned long long)lo, true};
+  }
+  // One step of target g; the buffers are g's own ([g.cnt, ...]).
+  int step_range(const StepTarget& g, const void* act, void* obs, void* rew, uint8_t* term, uint8_t* trunc, void* fobs, cudaStream_t s) {
     KArgs<Real> a = base; a.op = OP_STEP; a.seed = seed;
-    a.n = cnt; a.st = d_state + lo; a.env_base = base.env_base + (unsigned long long)lo;
-    a.act = (const Real*)act + lo * act_dim; a.obs = (Real*)obs + lo * obs_dim; a.rew = (Real*)rew + lo; a.term = term + lo; a.trunc = trunc + lo;
-    a.final_obs = fobs ? (Real*)fobs + lo * obs_dim : nullptr;
-    a.sens = sens_dev ? (Real*)sens_dev + lo * NSENSOR : nullptr;
+    if (!g.live) a.c.auto_reset = 0;
+    const long long cnt = g.cnt; const int slot = g.slot;
+    a.n = cnt; a.st = g.st; a.env_base = g.env_base;
+    a.act = (const Real*)act; a.obs = (Real*)obs; a.rew = (Real*)rew; a.term = term; a.trunc = trunc;
+    a.final_obs = (Real*)fobs;
+    a.sens = g.sens;
     constexpr int WF = warps_per_block<Real, D>();
     const unsigned full_blocks = (unsigned)((cnt + WF - 1) / WF);
     if constexpr (!HAS_LITE) return launch_step<D>(a, s, full_blocks);
@@ -596,7 +652,7 @@ struct Batch : BatchBase {
       if (single_tier) {   // testing aid: the full size class alone, every environment
         a.lite_maxcon = 0;
         if (int rc = launch_step<D>(a, s, full_blocks)) return rc;
-        ++full_steps;
+        if (g.live) ++full_steps;
         return 0;
       }
       constexpr int WL = warps_per_block<Real, DL>();
@@ -605,7 +661,7 @@ struct Batch : BatchBase {
       if constexpr (!CAN_OVERFLOW) {
         KArgs<Real> l = a; l.lite_maxcon = 0; l.ovf_stat = nullptr;
         if (int rc = launch_step<DL>(l, s, lite_blocks)) return rc;
-        ++lite_steps;
+        if (g.live) ++lite_steps;
         return 0;
       }
       int* const counter2 = counter + 2;   // list 2: straight to the generic class (from the lite tier's routing)
@@ -613,7 +669,7 @@ struct Batch : BatchBase {
       CUDA_OK(cudaMemsetAsync(counter, 0, 4 * sizeof(int), s));
       const unsigned tail_blocks = (unsigned)(UR3E_BLOCKS_PER_SM * sm_count);
       KArgs<Real> l = a;
-      l.ovf_count = counter; l.ovf_list = d_ovf_list + lo; l.cap_con = lite_cap_con; l.cap_efc = lite_cap_efc; l.lite_maxcon = 0; l.ovf_stat = nullptr;
+      l.ovf_count = counter; l.ovf_list = g.list1; l.cap_con = lite_cap_con; l.cap_efc = lite_cap_efc; l.lite_maxcon = 0; l.ovf_stat = nullptr;
       if constexpr (HAS_MID) {
         // Three tiers: lite -> grasp tier (list 1) -> generic class (lists 2 and 3).  The generic class's kernel takes the latency of one
         // environment step however short its list is, so the environments known to need it (list 2, routed by the lite tier from their
@@ -625,22 +681,23 @@ struct Batch : BatchBase {
           CUDA_OK(cudaStreamCreateWithFlags(&aux_stream[slot], cudaStreamNonBlocking));
           CUDA_OK(cudaEventCreateWithFlags(&fork_ev[slot], cudaEventDisableTiming)); CUDA_OK(cudaEventCreateWithFlags(&join_ev[slot], cudaEventDisableTiming));
         }
-        l.ovf2_count = counter2; l.ovf2_list = d_ovf_list2 + lo;
+        l.ovf2_count = counter2; l.ovf2_list = g.list2;
         if (int rc = launch_step<DL>(l, s, lite_blocks)) return rc;
         a.mid_maxcon = DM::MAXCON; a.mid_maxefc = DM::MAXEFC;
         CUDA_OK(cudaEventRecord(fork_ev[slot], s)); CUDA_OK(cudaStreamWaitEvent(aux_stream[slot], fork_ev[slot], 0));
-        KArgs<Real> f2 = a; f2.list_count = counter2; f2.list = d_ovf_list2 + lo;
+        KArgs<Real> f2 = a; f2.list_count = counter2; f2.list = g.list2;
         if (int rc = launch_step<D>(f2, aux_stream[slot], tail_blocks < full_blocks ? tail_blocks : full_blocks, 2)) return rc;
         KArgs<Real> mk = a;
-        mk.list_count = counter; mk.list = d_ovf_list + lo; mk.ovf_count = counter3; mk.ovf_list = d_ovf_list3 + lo;
+        mk.list_count = counter; mk.list = g.list1; mk.ovf_count = counter3; mk.ovf_list = g.list3;
         if (int rc = launch_step<DM>(mk, s, tail_blocks < mid_blocks ? tail_blocks : mid_blocks)) return rc;
         CUDA_OK(cudaEventRecord(join_ev[slot], aux_stream[slot])); CUDA_OK(cudaStreamWaitEvent(s, join_ev[slot], 0));
-        a.list_count = counter3; a.list = d_ovf_list3 + lo;
+        a.list_count = counter3; a.list = g.list3;
       } else {
         if (int rc = launch_step<DL>(l, s, lite_blocks)) return rc;
-        a.list_count = counter; a.list = d_ovf_list + lo;
+        a.list_count = counter; a.list = g.list1;
       }
       if (int rc = launch_step<D>(a, s, tail_blocks < full_blocks ? tail_blocks : full_blocks)) return rc;
+      if (!g.live) return 0;
       ++lite_steps;
       if (!ovf_pending && slot == 0) {   // information only (ur3e_batch_tier_info): size of the full tier's list, read back without synchronising
         CUDA_OK(cudaMemcpyAsync(h_ovf, counter, sizeof(int), cudaMemcpyDeviceToHost, s));
@@ -659,7 +716,6 @@ struct Batch : BatchBase {
   // Host-buffer entry point.  The batch is cut into HOST_CHUNKS ranges that alternate between two streams, so that the
   // action upload and the result download of one range overlap the stepping of the next (pinned host buffers assumed;
   // pageable ones still work, the copies then serialise).
-  static constexpr int HOST_CHUNKS = 4;
   int step_host(const void* act, void* obs, void* rew, uint8_t* term, uint8_t* trunc) override {
     CUDA_OK(cudaSetDevice(device));
     if (int rc = ensure_staging()) return rc;
@@ -677,7 +733,7 @@ struct Batch : BatchBase {
       if (cnt <= 0) break;
       cudaStream_t s = (c & 1) ? own_stream2 : own_stream;
       CUDA_OK(cudaMemcpyAsync(d_act + lo * act_dim, (const Real*)act + lo * act_dim, sizeof(Real) * cnt * act_dim, cudaMemcpyHostToDevice, s));
-      if (int rc = step_range(d_act, d_obs, d_rew, d_term, d_trunc, nullptr, s, lo, cnt, c)) return rc;
+      if (int rc = step_range(live_range(lo, cnt, c), d_act + lo * act_dim, d_obs + lo * obs_dim, d_rew + lo, d_term + lo, d_trunc + lo, nullptr, s)) return rc;
       CUDA_OK(cudaMemcpyAsync((Real*)obs + lo * obs_dim, d_obs + lo * obs_dim, sizeof(Real) * cnt * obs_dim, cudaMemcpyDeviceToHost, s));
       CUDA_OK(cudaMemcpyAsync((Real*)rew + lo, d_rew + lo, sizeof(Real) * cnt, cudaMemcpyDeviceToHost, s));
       CUDA_OK(cudaMemcpyAsync(term + lo, d_term + lo, cnt, cudaMemcpyDeviceToHost, s));
@@ -768,6 +824,62 @@ struct Batch : BatchBase {
     render_kernel<Real><<<dim3((unsigned)m, tiles), RENDER_THREADS, render_smem(r.k), s>>>(ra);
     ++launches;
     CUDA_OK(cudaGetLastError());
+    return 0;
+  }
+  // ---- rollouts: T tiered steps (step_range) of a scratch batch of m records on the counter slot ROLLOUT_SLOT.  The workspace is
+  // grown to the largest m seen: records [m], the three tier lists [m], and obs [m, obs_dim], reward [m], terminated [m] and
+  // truncated [m] for the outputs the caller did not ask for (the step kernels always write them).
+  unsigned char* d_roll = nullptr; long long roll_cap = 0;
+  static size_t align256(size_t b) { return (b + 255) / 256 * 256; }
+  int rollout(const int32_t* src, const void* qpos0, const void* qvel0, const void* ws0, long long m, int T, const void* act,
+              const ur3e_rollout_out* out, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const bool any = out && (out->qpos || out->qvel || out->obs || out->reward || out->terminated || out->truncated || out->sensordata || out->info);
+    const std::string err = rollout_check(m, T, act != nullptr, src != nullptr, qpos0 != nullptr, qvel0 != nullptr, ws0 != nullptr, out != nullptr, any);
+    if (!err.empty()) return set_err("rollout: " + err);
+    const size_t b_st = align256(sizeof(EnvState<Real, D>) * m), b_list = align256(sizeof(int) * m), b_obs = align256(sizeof(Real) * m * obs_dim),
+                 b_rew = align256(sizeof(Real) * m);
+    if (m > roll_cap) {
+      // cudaFree waits for the device, so a call still using the old workspace finishes first
+      CUDA_OK(cudaFree(d_roll)); d_roll = nullptr; roll_cap = 0;
+      CUDA_OK(cudaMalloc(&d_roll, b_st + 3 * b_list + b_obs + b_rew + 2 * align256(m))); roll_cap = m;
+    }
+    EnvState<Real, D>* const st = reinterpret_cast<EnvState<Real, D>*>(d_roll);
+    unsigned char* p = d_roll + b_st;
+    int* const lists = reinterpret_cast<int*>(p); p += 3 * b_list;
+    Real* const s_obs = reinterpret_cast<Real*>(p); p += b_obs;
+    Real* const s_rew = reinterpret_cast<Real*>(p); p += b_rew;
+    uint8_t* const s_term = p; uint8_t* const s_trunc = p + align256(m);
+    // read-only for the batch, like query(): last_stream stays that of the latest state-changing call
+    if (src) {
+      rollout_gather_kernel<Real, D><<<(unsigned)((m * 32 + 255) / 256), 256, 0, s>>>(d_state, n, src, st, m);
+      ++launches;
+      CUDA_OK(cudaGetLastError());
+    } else {
+      CUDA_OK(cudaMemsetAsync(st, 0, sizeof(EnvState<Real, D>) * m, s));
+      KArgs<Real> a = base; a.op = OP_SET_STATE; a.st = st; a.n = m;
+      a.qpos_in = (const Real*)qpos0; a.qvel_in = (const Real*)qvel0; a.ws_in = (const Real*)ws0;
+      if (int rc = launch_warps<D>(env_kernel<Real, D>, a, s, m)) return rc;
+    }
+    StepTarget g{st, m, ROLLOUT_SLOT, lists, lists + b_list / sizeof(int), lists + 2 * (b_list / sizeof(int)), nullptr, 0, false};
+    const int nq = hm.nq, nv = hm.nv;
+    for (int t = 0; t < T; ++t) {
+      const long long o = (long long)t * m;
+      g.sens = out->sensordata ? (Real*)out->sensordata + o * NSENSOR : nullptr;
+      if (int rc = step_range(g, (const Real*)act + o * act_dim, out->obs ? (Real*)out->obs + o * obs_dim : s_obs, out->reward ? (Real*)out->reward + o : s_rew,
+                              out->terminated ? out->terminated + o : s_term, out->truncated ? out->truncated + o : s_trunc, nullptr, s)) return rc;
+      if (out->qpos || out->qvel) {
+        state_io_kernel<Real, D><<<(unsigned)((m * 64 + 255) / 256), 256, 0, s>>>(st, m, nq, nv, out->qpos ? (Real*)out->qpos + o * nq : nullptr,
+                                                                                 out->qvel ? (Real*)out->qvel + o * nv : nullptr, nullptr);
+        ++launches;
+        CUDA_OK(cudaGetLastError());
+      }
+    }
+    if (out->info) {
+      rollout_info_kernel<Real, D><<<(unsigned)((m + 255) / 256), 256, 0, s>>>(st, m, out->info);
+      ++launches;
+      CUDA_OK(cudaGetLastError());
+    }
     return 0;
   }
   int set_sensor_buffer(void* buf) override { sens_dev = buf; return 0; }

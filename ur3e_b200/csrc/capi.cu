@@ -126,5 +126,9 @@ int ur3e_batch_render_create(ur3e_batch* b, const ur3e_camera* cam, const int32_
 int ur3e_batch_render(ur3e_batch* b, int render_id, const int32_t* env_ids_dev, int64_t m, uint8_t* rgb_dev, void* depth_dev, int32_t* seg_dev, void* stream) {
   GUARD(b); return b->impl->render(render_id, env_ids_dev, m, rgb_dev, depth_dev, seg_dev, (cudaStream_t)stream);
 }
+int ur3e_batch_rollout(ur3e_batch* b, const int32_t* src_env_ids_dev, const void* qpos0_dev, const void* qvel0_dev, const void* qacc_warmstart0_dev,
+                       int64_t m, int32_t T, const void* actions_dev, const ur3e_rollout_out* out, void* stream) {
+  GUARD(b); return b->impl->rollout(src_env_ids_dev, qpos0_dev, qvel0_dev, qacc_warmstart0_dev, m, T, actions_dev, out, (cudaStream_t)stream);
+}
 
 }  // extern "C"
