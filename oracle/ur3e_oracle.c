@@ -427,13 +427,16 @@ static int clip_poly(double* px, double* py, int n, double a, double b, double c
   return k;
 }
 
+#define EDGE_END_SLACK 1e-5   /* csrc/engine.cuh EDGE_END_SLACK */
 static int box_box(const double* p1, const double* R1, const double* s1, const double* p2, const double* R2, const double* s2,
                    double margin, double* dist, double* pos, double* normal) {
   /* This repo's box-box manifold (stands in for mjc_BoxBox, whose exact point selection is not
    * reproducible from memory, SURVEY hard-part 4): 15-axis SAT -> face case: incident face clipped
    * against the reference face's side planes, points kept where depth > -margin, contact at
    * mid-penetration; edge case: closest points of the two edges.  Normal points from box1 to box2.
-   * Kernel (csrc/collide.cuh) implements the same rules. */
+   * The edge case stands only when the closest points lie within both edges (up to EDGE_END_SLACK): outside them the edge-edge
+   * axis was degenerate (nearly parallel edges, or an axis within rounding of a face normal) and the face case decides.
+   * Kernel (csrc/engine.cuh box_box) implements the same rules. */
   double d[3], A1[3][3], A2[3][3];
   for (int k = 0; k < 3; k++) d[k] = p2[k] - p1[k];
   for (int i = 0; i < 3; i++) for (int k = 0; k < 3; k++) { A1[i][k] = R1[3 * k + i]; A2[i][k] = R2[3 * k + i]; } /* axis i = column i */
@@ -476,13 +479,16 @@ static int box_box(const double* p1, const double* R1, const double* s1, const d
     double w[3]; for (int k = 0; k < 3; k++) w[k] = c1[k] - c2[k];
     double b = dot3(u, v), dd = dot3(u, w), e = dot3(v, w), den = 1 - b * b;
     double sa = (b * e - dd) / den, sb = (e - b * dd) / den;
-    if (sa > s1[ei]) sa = s1[ei]; if (sa < -s1[ei]) sa = -s1[ei];
-    if (sb > s2[ej]) sb = s2[ej]; if (sb < -s2[ej]) sb = -s2[ej];
-    double q1[3], q2[3];
-    for (int k = 0; k < 3; k++) { q1[k] = c1[k] + sa * u[k]; q2[k] = c2[k] + sb * v[k]; }
-    dist[0] = ebest;
-    for (int k = 0; k < 3; k++) { pos[k] = 0.5 * (q1[k] + q2[k]); normal[k] = en[k]; }
-    return 1;
+    /* a real edge-edge contact meets within both edges; otherwise the axis was degenerate and the face case decides */
+    if (fabs(sa) <= s1[ei] * (1 + EDGE_END_SLACK) && fabs(sb) <= s2[ej] * (1 + EDGE_END_SLACK)) {
+      if (sa > s1[ei]) sa = s1[ei]; if (sa < -s1[ei]) sa = -s1[ei];
+      if (sb > s2[ej]) sb = s2[ej]; if (sb < -s2[ej]) sb = -s2[ej];
+      double q1[3], q2[3];
+      for (int k = 0; k < 3; k++) { q1[k] = c1[k] + sa * u[k]; q2[k] = c2[k] + sb * v[k]; }
+      dist[0] = ebest;
+      for (int k = 0; k < 3; k++) { pos[k] = 0.5 * (q1[k] + q2[k]); normal[k] = en[k]; }
+      return 1;
+    }
   }
   /* face case */
   int ref_is_1 = code < 3; int ra = ref_is_1 ? code : code - 3;

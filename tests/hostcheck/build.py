@@ -33,6 +33,8 @@ def lib():
         _L.hc_forward.argtypes = [C.c_char_p, dp, dp, dp, dp, C.POINTER(dp), C.POINTER(ip)]
         _L.hc_max_contacts.argtypes = [C.c_char_p]
         _L.hc_forward_check.argtypes = [C.c_int] * 4
+        _L.hc_box_box.argtypes = [C.c_int, dp, dp, dp, dp, dp, dp, C.c_double, dp]
+        _L.hc_plane_box.argtypes = [C.c_int, dp, dp, dp, dp, dp, C.c_double, dp]
     return _L
 
 
@@ -96,6 +98,33 @@ def query_jac(xml, qpos, qvel, objtype=(), objid=(), jacp=True, jacr=True, M=Tru
     if rc != 0:
         raise ValueError("hc_query_jac rejected the call (%d)" % rc)
     return tuple(outs)
+
+
+STAGE_W = 3 + 4 * 8   # engine.cuh: normal, then STAGE_PTS x (pos, dist)
+
+
+def _stage(n, row):
+    """(n, normal [3], pos [n, 3], dist [n]) of a staging row.  Past the n points the row holds box_box's frames and clip
+    polygon, which collision() never reads."""
+    pts = row[3:3 + 4 * n].reshape(n, 4)
+    return n, row[:3].copy(), pts[:, :3].copy(), pts[:, 3].copy()
+
+
+def box_box(p1, R1, s1, p2, R2, s2, margin=0.0, use_float=False):
+    """The kernel's box_box<float / double> on boxes (centre, world frame [3, 3], half-sizes): (n, normal from box 1 to box 2,
+    pos [n, 3], dist [n]).  The normal is meaningless when n = 0."""
+    a = [np.ascontiguousarray(x, dtype=np.float64).reshape(-1) for x in (p1, R1, s1, p2, R2, s2)]
+    row = np.zeros(STAGE_W)
+    n = lib().hc_box_box(int(bool(use_float)), *[_p(x) for x in a], C.c_double(margin), _p(row))
+    return _stage(n, row)
+
+
+def plane_box(ppos, pmat, bpos, bmat, size, margin=0.0, use_float=False):
+    """The kernel's plane_box<float / double>: (n, plane normal, pos [n, 3], dist [n]), at most 4 corners in corner order."""
+    a = [np.ascontiguousarray(x, dtype=np.float64).reshape(-1) for x in (ppos, pmat, bpos, bmat, size)]
+    row = np.zeros(STAGE_W)
+    n = lib().hc_plane_box(int(bool(use_float)), *[_p(x) for x in a], C.c_double(margin), _p(row))
+    return _stage(n, row)
 
 
 def forward_check(out, con, any_, ncmax):

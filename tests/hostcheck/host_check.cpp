@@ -3,6 +3,7 @@
 // package, never loaded by ur3e_b200: the product has no CPU path.
 #include <cstdio>
 #include <cstring>
+#include <limits>
 #include <map>
 #include <memory>
 #include <string>
@@ -28,7 +29,7 @@ static int with_dims(const char* name, const char* xml, F&& f) {
   try {
     const HostModel& h = get_model(xml);
     if (h.nv <= DimsRaw::NV && h.npair == 0) return f(h, DimsRaw{});
-    if (h.nv <= DimsGrip::NV) return f(h, DimsGrip{});
+    if (h.nv <= DimsGrip::NV && h.nq <= DimsGrip::NQ) return f(h, DimsGrip{});
     return f(h, DimsMain{});
   } catch (const std::exception& e) { std::fprintf(stderr, "%s: %s\n", name, e.what()); return -2; }
 }
@@ -178,3 +179,35 @@ extern "C" int hc_max_contacts(const char* xml) {
 
 // forward_query_check itself: 0 when the combination is accepted, -1 when rejected
 extern "C" int hc_forward_check(int out, int con, int any, int ncmax) { return forward_query_check(out != 0, con != 0, any != 0, ncmax).empty() ? 0 : -1; }
+
+// The narrow phase's own functions in Real, called as collision() calls them: out is one STAGE_W staging row, filled with NaN first
+// so that a value the function does not write shows, and returned whole (normal in [0, 3), then (pos 3, dist 1) per point).
+template <typename Real>
+static int box_box_row(const double* p1, const double* R1, const double* s1, const double* p2, const double* R2, const double* s2, double margin, double* out) {
+  Real a1[3], a2[3], z1[3], z2[3], st[STAGE_W];
+  for (int k = 0; k < 3; ++k) { a1[k] = (Real)p1[k]; a2[k] = (Real)p2[k]; z1[k] = (Real)s1[k]; z2[k] = (Real)s2[k]; }
+  for (int k = 0; k < STAGE_W; ++k) st[k] = std::numeric_limits<Real>::quiet_NaN();
+  for (int k = 0; k < 9; ++k) { st[k] = (Real)R1[k]; st[9 + k] = (Real)R2[k]; }   // the frames go in through the row
+  const int n = box_box<Real>(a1, z1, a2, z2, (Real)margin, st);
+  for (int k = 0; k < STAGE_W; ++k) out[k] = st[k];
+  return n;
+}
+template <typename Real>
+static int plane_box_row(const double* ppos, const double* pmat, const double* bpos, const double* bmat, const double* size, double margin, double* out) {
+  Real pp[3], pm[9], bp[3], bm[9], sz[3], st[STAGE_W];
+  for (int k = 0; k < 3; ++k) { pp[k] = (Real)ppos[k]; bp[k] = (Real)bpos[k]; sz[k] = (Real)size[k]; }
+  for (int k = 0; k < 9; ++k) { pm[k] = (Real)pmat[k]; bm[k] = (Real)bmat[k]; }
+  for (int k = 0; k < STAGE_W; ++k) st[k] = std::numeric_limits<Real>::quiet_NaN();
+  const int n = plane_box<Real>(pp, pm, bp, bm, sz, (Real)margin, st);
+  for (int k = 0; k < STAGE_W; ++k) out[k] = st[k];
+  return n;
+}
+// box_box / plane_box in float (use_float) or double: the number of points; frames row-major [9], out [STAGE_W]
+extern "C" int hc_box_box(int use_float, const double* p1, const double* R1, const double* s1, const double* p2, const double* R2, const double* s2, double margin,
+                          double* out) {
+  return use_float ? box_box_row<float>(p1, R1, s1, p2, R2, s2, margin, out) : box_box_row<double>(p1, R1, s1, p2, R2, s2, margin, out);
+}
+extern "C" int hc_plane_box(int use_float, const double* ppos, const double* pmat, const double* bpos, const double* bmat, const double* size, double margin,
+                            double* out) {
+  return use_float ? plane_box_row<float>(ppos, pmat, bpos, bmat, size, margin, out) : plane_box_row<double>(ppos, pmat, bpos, bmat, size, margin, out);
+}

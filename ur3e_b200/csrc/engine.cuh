@@ -39,6 +39,9 @@ using DimsMainMid = Dims<19, 20, 21, 7, 14, 48, 16, 68, 14, true>;   // the gras
 
 constexpr int STAGE_PTS = 8;  // contact points a pair can emit
 constexpr int STAGE_W = 3 + 4 * STAGE_PTS;
+// box_box keeps an edge-edge contact only when the closest points of the two edges lie within both, up to this fraction of each
+// edge's half-length (rounding); the oracle's box_box uses the same value
+constexpr double EDGE_END_SLACK = 1e-5;
 
 // row kinds; the rows of a launch are ordered [connect equalities | contacts] (dense: these have a stored Jacobian row)
 // then [joint equalities | friction loss | joint limits] (sparse: one or two +-1 / polynomial entries, never stored)
@@ -543,6 +546,14 @@ UR3E_HD int clip_poly(const Real* px, const Real* py, int n, Real* ox, Real* oy,
 // `out` is the slot's staging row (STAGE_W values, shared memory).  On entry it holds the two world frames (R1 = out[0, 9),
 // R2 = out[9, 18)), so that no argument is passed by address from the caller's stack; the frames are dead once the
 // clipping starts, and the row then holds one of the two clip polygons until the contact points overwrite it.
+// 15-axis SAT: face axes (box 2's only when deeper by 1e-6 x box 1's size), then edge-edge axes, which win only when better than
+// the best face axis by 1e-3 |best| + 1e-9 and give one point, the closest points of the two supporting edges.  Those lie within
+// both edges for a real edge-edge contact.  When they do not (beyond EDGE_END_SLACK), the axis was degenerate -- two nearly parallel
+// edges, whose closest points are ill-conditioned, or an axis within rounding of a face normal, whose supporting edges were picked
+// from signs of ~0 -- and the face case below gives the manifold.  Without that check nearly parallel stacked faces at um
+// penetration got one contact up to 2 cm off both boxes (tests/test_narrow_phase_cpu.py pins the manifold against the exact
+// penetration of the boxes' Minkowski difference).  A slightly tilted face-on-face touch whose edge-edge axis wins keeps its one
+// on-surface edge point.
 template <typename Real>
 UR3E_PHASE int box_box(const Real* p1, const Real* s1, const Real* p2, const Real* s2, Real margin, Real* out) {
   const Real* const R1 = out; const Real* const R2 = out + 9;
@@ -583,10 +594,13 @@ UR3E_PHASE int box_box(const Real* p1, const Real* s1, const Real* p2, const Rea
     Real w[3] = {c1[0] - c2[0], c1[1] - c2[1], c1[2] - c2[2]};
     Real b = dot3(u, v), dd = dot3(u, w), e = dot3(v, w), den = 1 - b * b;
     Real sa = (b * e - dd) / den, sb = (e - b * dd) / den;
-    sa = rmin(rmax(sa, -s1[ei]), s1[ei]); sb = rmin(rmax(sb, -s2[ej]), s2[ej]);
-    for (int k = 0; k < 3; ++k) { out[3 + k] = Real(0.5) * (c1[k] + sa * u[k] + c2[k] + sb * v[k]); out[k] = en[k]; }
-    out[6] = ebest;
-    return 1;
+    // a real edge-edge contact meets within both edges; outside them the axis was degenerate (see above) and the face case decides
+    if (Num<Real>::abs(sa) <= s1[ei] * Real(1 + EDGE_END_SLACK) && Num<Real>::abs(sb) <= s2[ej] * Real(1 + EDGE_END_SLACK)) {
+      sa = rmin(rmax(sa, -s1[ei]), s1[ei]); sb = rmin(rmax(sb, -s2[ej]), s2[ej]);
+      for (int k = 0; k < 3; ++k) { out[3 + k] = Real(0.5) * (c1[k] + sa * u[k] + c2[k] + sb * v[k]); out[k] = en[k]; }
+      out[6] = ebest;
+      return 1;
+    }
   }
   bool ref1 = code < 3; int ra = ref1 ? code : code - 3;
   const Real *rp = ref1 ? p1 : p2, *ip = ref1 ? p2 : p1, *rs = ref1 ? s1 : s2, *is = ref1 ? s2 : s1;
