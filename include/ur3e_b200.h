@@ -173,6 +173,37 @@ typedef struct ur3e_forward_out {
 } ur3e_forward_out;
 int ur3e_batch_max_contacts(const ur3e_batch* b);
 int ur3e_batch_forward(ur3e_batch* b, const void* ctrl_dev, const ur3e_forward_out* out, void* stream);
+/* Inverse dynamics (mj_inverse): the generalised force that produces a given acceleration at a given state, and the constraint and
+ * contact forces the soft-constraint model implies at that acceleration.  For feedforward torques of planned motions, inverse-dynamics
+ * labels along recorded trajectories and the residual of the forward solver (MuJoCo's mjENBL_FWDINV).
+ * State, exactly one source:
+ *   qpos_dev and qvel_dev both NULL: the STORED state of the batch's n environments (m must equal n).  As for ur3e_batch_forward,
+ *     after a step this is one substep newer than MuJoCo's stale arrays (SURVEY F9).
+ *   qpos_dev [m, nq], qvel_dev [m, nv] (batch dtype): m >= 1 given states, independent of n (a [T, m'] trajectory of
+ *     ur3e_batch_rollout flattens into one call).  No record is read or written.
+ * qacc_dev [m, nv] (batch dtype).  With discrete = 0 it is the continuous acceleration a (MuJoCo's default).  With discrete != 0
+ * (mjENBL_INVDISCRETE, mj_discreteAcc) it is the acceleration the Euler step applied, (qvel_next - qvel) / timestep of one mj_step,
+ * and a = M^-1 (M + timestep diag(dof_damping)) qacc, the exact inverse of the step's implicit damping; a model without damping has
+ * a = qacc.  With frame_skip > 1 one env-step is frame_skip mj_steps: the discrete convention applies per mj_step (substep), not per
+ * env-step.
+ * Computed, at (qpos, qvel) and a, with no solver iterations and no warm start (ctrl plays no part):
+ *   jar = J a - aref;  efc_force = the constraint law at jar (elliptic cones, friction loss, limits: mj_invConstraint);
+ *   qfrc_constraint = J^T efc_force;
+ *   qfrc_inverse = M a + qfrc_bias - qfrc_passive - qfrc_constraint,  qfrc_passive = -dof_damping qvel - stiffness (q - springref).
+ * qfrc_inverse excludes actuation: at a = forward's qacc it equals qfrc_actuator up to the forward solver's residual.  Sensors are not
+ * evaluated.
+ * Device outputs, any may be NULL, not all; float ones in the batch's dtype; C = ur3e_batch_max_contacts(b):
+ *   qfrc_inverse, qfrc_constraint [m, nv]
+ *   info [m, 3] int32: ncon, nefc, overflow bits (1 contacts, 2 constraint rows; the bits the step sets)
+ *   contact_geom [m, C, 2] int32 and contact_force [m, C, 6]: ur3e_batch_forward's conventions (geom -1 and zeros past ncon;
+ *        mj_contactForce [fn, ft1, ft2, 0, 0, 0] in the contact frame at the given acceleration, 0 for a contact without rows)
+ * Rejected: qpos_dev without qvel_dev or the reverse, m < 1 or m > 2^31 - 1, m != n for the stored state, qacc_dev NULL, out NULL,
+ * every output NULL, a contact output when C = 0.  Asynchronous on `stream`, one kernel launch; no record is modified. */
+typedef struct ur3e_inverse_out {
+  void* qfrc_inverse; void* qfrc_constraint; int32_t* info; int32_t* contact_geom; void* contact_force;
+} ur3e_inverse_out;
+int ur3e_batch_inverse(ur3e_batch* b, const void* qpos_dev, const void* qvel_dev, int64_t m, const void* qacc_dev, int32_t discrete,
+                       const ur3e_inverse_out* out, void* stream);
 /* Offscreen rendering: rgb_array / depth_array images (gymnasium MujocoEnv.render, ur3e_env2.py:25-28) and geom segmentation for
  * selected environments, from a camera anchored to the world or to one object of the loaded model.
  * ur3e_batch_render_create compiles a renderer and returns its id (>= 0); the batch owns it until ur3e_batch_destroy.

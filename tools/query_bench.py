@@ -1,4 +1,4 @@
-"""Query timing (ur3e_batch_query, ur3e_batch_query_jac, ur3e_batch_forward) on the float32 main.xml batch, beside one env-step for scale.
+"""Query timing (ur3e_batch_query, ur3e_batch_query_jac, ur3e_batch_forward, ur3e_batch_inverse) on the float32 main.xml batch, beside one env-step for scale.
 
     python tools/query_bench.py [--envs 65536] [--settle 1500] [--launches 500] [--out FILE]
 
@@ -12,8 +12,12 @@ state.  Then, with CUDA events around `--launches` back-to-back launches after a
   fwd_a  contacts only: info, contact_geom and flags   (the contacts-only pass: kinematics and collision; what get_ncon and the
          collision predicates of ur3e_b200/utils.py run)
   fwd_b  everything, with ctrl: qacc, qfrc_constraint, info, the five contact outputs, flags and sensordata   (the full mj_forward)
+  inv_a  qfrc_inverse at the stored state, qacc from a previous fwd_b   (SimBatch.inverse: mj_inverse, no solver iterations)
+  inv_b  given states: a 16 x 4 096 rollout trajectory flattened to 65 536 states, discrete convention, qfrc_inverse + contact_force
+         (inverse-dynamics labels along rollouts)
 and one env-step over `--launches / 10` steps.  The byte floor counts what a call must move: the record fields it reads (qpos and
-qvel for kin and jac; the whole 544-byte record for fwd, which the kernel loads whole, and ctrl for fwd_b) and the outputs written.
+qvel for kin, jac and inv_a; the whole 544-byte record for fwd, which the kernel loads whole, and ctrl for fwd_b; the given qpos and
+qvel for inv_b; qacc for inv) and the outputs written.
 The L2 is not flushed between launches: kin_a's working set (qpos + qvel of the records, 18 MB of outputs) stays in the 126 MB L2;
 kin_b's 363 MB of outputs, jac_a's 142 MB and jac_b's 110 MB per call at 65 536 environments do not.  Prints one JSON line with the
 GPU's name, power limit and SM clock.
@@ -107,11 +111,28 @@ def main():
                                                          contact_pos=True, contact_frame=True, contact_force=True, flags=True, sensordata=True), args.launches),
                   "bytes_floor": n * (rec + 4 * nu + 4 * (2 * nv + 4 + C * (2 + 1 + 3 + 9 + 6) + 1 + lib.NSENSOR))},
     }
+    # inverse dynamics: qacc of a previous forward (inv_a); a 16-step rollout of 4 096 branched environments, flattened (inv_b)
+    fq = b.forward(ctrl=u, qacc=True).qacc.clone()
+    res["inv_a"] = {"outputs": "qfrc_inverse, stored state", "us_per_call": timed(lambda: b.inverse(fq), args.launches),
+                    "bytes_floor": n * (state_bytes + 4 * nv + 4 * nv)}
+    T, mr = 16, n // 16
+    ra = torch.stack([acts[k % 16][:mr] for k in range(T)]).contiguous()
+    ids = torch.arange(mr, dtype=torch.int32, device=dev)
+    r = b.rollout(ra, env_ids=ids, qpos=True, qvel=True, obs=False, reward=False, terminated=False, truncated=False)
+    q0, v0, _ = b.get_state()
+    tq = torch.cat([q0[:mr][None], r.qpos[:-1]]).reshape(-1, nq).contiguous()
+    tv = torch.cat([v0[:mr][None], r.qvel[:-1]]).reshape(-1, nv).contiguous()
+    ta = (torch.cat([v0[:mr][None], r.qvel]).diff(dim=0) / model.timestep).reshape(-1, nv).contiguous()
+    res["inv_b"] = {"outputs": "qfrc_inverse+contact_force, given states (16 x %d trajectory), discrete" % mr,
+                    "us_per_call": timed(lambda: b.inverse(ta, state=(tq, tv), discrete=True, qfrc_inverse=True, contact_force=True), args.launches),
+                    "bytes_floor": T * mr * (4 * (nq + nv) + 4 * nv + 4 * (nv + 6 * C))}
+    ib = b.inverse(ta, state=(tq, tv), discrete=True, qfrc_inverse=False, info=True).info
+    res["inv_b"]["mean_ncon"] = ib[:, 0].double().mean().item(); res["inv_b"]["mean_nefc"] = ib[:, 1].double().mean().item()
     res["mean_ncon"] = b.forward(qacc=False, info=True).info[:, 0].double().mean().item()
     res["mean_nefc"] = b.forward(qacc=True, info=True).info[:, 1].double().mean().item()
     it = iter(range(10 ** 9))
     res["env_step_us"] = timed(lambda: b.step(acts[next(it) % 16]), max(args.launches // 10, 10))
-    for q in ("kin_a", "kin_b", "jac_a", "jac_b", "fwd_a", "fwd_b"):
+    for q in ("kin_a", "kin_b", "jac_a", "jac_b", "fwd_a", "fwd_b", "inv_a", "inv_b"):
         r = res[q]
         r["GB_per_s"] = r["bytes_floor"] / (r["us_per_call"] * 1e-6) / 1e9
         r["fraction_of_env_step"] = r["us_per_call"] / res["env_step_us"]

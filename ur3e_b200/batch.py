@@ -35,6 +35,7 @@ def env_config(**kw):
 
 ForwardResult = namedtuple("ForwardResult", _lib.FORWARD_OUTPUTS)
 RolloutResult = namedtuple("RolloutResult", _lib.ROLLOUT_OUTPUTS)
+InverseResult = namedtuple("InverseResult", _lib.INVERSE_OUTPUTS)
 
 
 class SimBatch:
@@ -188,6 +189,62 @@ class SimBatch:
             u = self._chk(ctrl, (n, nu))
         st = _lib.ForwardOut(*[o.data_ptr() if o is not None else None for o in outs])
         _lib.check(self._L.ur3e_batch_forward(self.ptr, u, C.byref(st), self._stream()), "ur3e_batch_forward")
+        return outs
+
+    def inverse(self, qacc, state=None, discrete=False, qfrc_inverse=True, qfrc_constraint=False, info=False, contact_geom=False,
+                contact_force=False):
+        """mj_inverse of m states (ur3e_batch_inverse): the generalised force that produces the acceleration `qacc` [m, nv], and the
+        constraint and contact forces the soft-constraint model implies at it.  One launch on the current torch stream, returning an
+        InverseResult named tuple with None for every output not asked for; outputs follow forward()'s convention (False, True = a
+        tensor owned by the batch, reallocated when m changes, or a caller tensor).  C = max_contacts.
+
+            state None                         the stored state of every environment (m = n)
+            state (qpos [m, nq], qvel [m, nv]) m >= 1 given states, any m; no record is read or written
+
+            qfrc_inverse [m, nv]               M a + qfrc_bias - qfrc_passive - qfrc_constraint (actuation excluded)
+            qfrc_constraint [m, nv]            J^T efc_force, efc_force the constraint law at jar = J a - aref
+            info [m, 3] int32                  ncon, nefc, overflow bits (1 contacts, 2 constraint rows)
+            contact_geom [m, C, 2] int32       as forward()'s, -1 past ncon
+            contact_force [m, C, 6]            mj_contactForce at the given acceleration: [fn, ft1, ft2, 0, 0, 0] in the contact frame
+
+        discrete=False: qacc is the continuous acceleration a (MuJoCo's default).  discrete=True (mjENBL_INVDISCRETE): qacc is the
+        acceleration one Euler mj_step applied, (qvel_next - qvel) / timestep, and a = M^-1 (M + timestep diag(damping)) qacc undoes
+        the step's implicit damping (a model without damping gets a = qacc).  With frame_skip > 1 an env-step is frame_skip mj_steps
+        and the discrete convention holds per mj_step, not per env-step.  ctrl plays no part; no solver runs and sensors are not
+        evaluated.
+
+        Inverse dynamics of a trajectory: from a rollout of a CTRL_RAW, frame_skip 1 batch with qpos=True, qvel=True (states [T, m', ...]
+        after each step), state t's acceleration is (qvel[t + 1] - qvel[t]) / timestep, so
+            q, v = r.qpos[:-1].reshape(-1, nq), r.qvel[:-1].reshape(-1, nv)
+            a = ((r.qvel[1:] - r.qvel[:-1]) / timestep).reshape(-1, nv)
+            tau = b.inverse(a, state=(q, v), discrete=True).qfrc_inverse    # qfrc_actuator of actions[1:], up to the solver's residual
+        forward(ctrl).qacc fed back with discrete=False returns qfrc_actuator(ctrl) up to the forward solver's residual.
+
+        The stored state is what forward() and query() see: after a step MuJoCo's arrays are one substep older (SURVEY F9).
+        """
+        nv = self.model.nv
+        qp = qv = None
+        if state is not None:
+            if len(state) != 2:
+                raise ValueError("inverse: state is (qpos, qvel)")
+            m = int(state[0].shape[0]) if state[0].dim() >= 1 else 0
+            qp = self._chk(state[0], (m, self.model.nq)); qv = self._chk(state[1], (m, nv))
+        else:
+            m = self.n
+        a = self._chk(qacc, (m, nv))
+        Cn = self.max_contacts
+        if Cn == 0:
+            asked = [k for k, v in (("contact_geom", contact_geom), ("contact_force", contact_force)) if v is not False and v is not None]
+            if asked:
+                raise ValueError("%s: the model has no contact pairs (max_contacts = 0)" % ", ".join(asked))
+        if getattr(self, "_inverse_m", None) != m:
+            self._inverse_own, self._inverse_m = {}, m   # owned outputs follow the latest call's m
+        i32 = torch.int32
+        table = dict(qfrc_inverse=(qfrc_inverse, (m, nv), None), qfrc_constraint=(qfrc_constraint, (m, nv), None), info=(info, (m, 3), i32),
+                     contact_geom=(contact_geom, (m, Cn, 2), i32), contact_force=(contact_force, (m, Cn, 6), None))
+        outs = InverseResult(**_outs(self, self._inverse_own, "inverse", table))
+        st = _lib.InverseOut(*[o.data_ptr() if o is not None else None for o in outs])
+        _lib.check(self._L.ur3e_batch_inverse(self.ptr, qp, qv, m, a, int(bool(discrete)), C.byref(st), self._stream()), "ur3e_batch_inverse")
         return outs
 
     def renderer(self, width, height, camera, geoms=None, rgba=None):

@@ -38,6 +38,8 @@ struct BatchBase {
   // one mj_forward per environment at the stored state: contacts, contact forces, qacc, sensordata (query_fwd.cuh forward_query_env)
   virtual int max_contacts() const = 0;
   virtual int forward(const void* ctrl, const ur3e_forward_out* out, cudaStream_t s) = 0;
+  // mj_inverse of m states: the stored state (qpos / qvel null, m = n) or given ones (query_inv.cuh inverse_query_env)
+  virtual int inverse(const void* qpos, const void* qvel, long long m, const void* qacc, int discrete, const ur3e_inverse_out* out, cudaStream_t s) = 0;
   // offscreen rendering (render.cuh): the batch owns its renderers and their pose scratch; render_create returns the renderer's id
   virtual int render_create(const ur3e_camera* cam, const int32_t* geom_ids, int k, const float* rgba, int width, int height) = 0;
   virtual int render(int id, const int32_t* env_ids, long long m, uint8_t* rgb, void* depth, int32_t* seg, cudaStream_t s) = 0;

@@ -14,6 +14,7 @@
 #include "env.cuh"
 #include "query.cuh"
 #include "query_fwd.cuh"
+#include "query_inv.cuh"
 #include "render.cuh"
 #include "rollout.h"
 
@@ -343,6 +344,50 @@ __global__ void __launch_bounds__(warps_per_block<Real, D>() * 32, 1) query_fwd_
 }
 
 template <typename Real, typename D>
+struct QIArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;            // the stored state, read when qpos / qvel are null
+  const Real* qpos; const Real* qvel;     // [count, nq], [count, nv] given states, or null
+  long long count;
+  const Real* qacc;                       // [count, nv]
+  int discrete;
+  InvOut<Real> o;                         // outputs: state i's start at i times each output's per-state size
+};
+
+// Inverse-dynamics queries (query_inv.cuh inverse_query_env): one warp per state on the generic size class's own arena, so the
+// contact and row caps are those of the forward query; reads qpos and qvel of the record or of the given arrays, never writes a record.
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, D>() * 32, 1) query_inv_kernel(const QIArgs<Real, D> a) {
+  constexpr int WPB = warps_per_block<Real, D>();
+  constexpr long long C = D::HAS_CONTACT ? D::MAXCON : 0;
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long i = (long long)blockIdx.x * WPB + warp;
+  if (i >= a.count) return;
+  Arena<Real, D>& s = *reinterpret_cast<Arena<Real, D>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, D>());
+  const DevModel<Real>& m = *a.m;
+  const long long nq = m.nq, nv = m.nv;
+  const Real* qp = a.qpos ? a.qpos + i * nq : a.st[i].qpos;
+  const Real* qv = a.qvel ? a.qvel + i * nv : a.st[i].qvel;
+  WARP_FOR(j, m.nq) s.st.qpos[j] = qp[j];
+  WARP_FOR(j, m.nv) s.st.qvel[j] = qv[j];
+#ifdef UR3E_CANARY
+  canary_set(s);
+#endif
+  InvOut<Real> o;
+  o.qfrc_inverse = a.o.qfrc_inverse ? a.o.qfrc_inverse + i * nv : nullptr;
+  o.qfrc_constraint = a.o.qfrc_constraint ? a.o.qfrc_constraint + i * nv : nullptr;
+  o.info = a.o.info ? a.o.info + i * 3 : nullptr;
+  o.contact_geom = a.o.contact_geom ? a.o.contact_geom + i * C * 2 : nullptr;
+  o.contact_force = a.o.contact_force ? a.o.contact_force + i * C * 6 : nullptr;
+  inverse_query_env(m, s, a.discrete != 0, a.qacc + i * nv, o);
+#ifdef UR3E_CANARY
+  WARP_SYNC();
+  { const int bad = canary_bad(s); if (bad) { IF_LANE0 printf("ur3e_b200: arena guard word clobbered (mask 0x%x, inverse state %lld)\n", bad, i); } }
+#endif
+}
+
+template <typename Real, typename D>
 struct RPArgs {
   const DevModel<Real>* m;
   const EnvState<Real, D>* st;
@@ -549,6 +594,7 @@ struct Batch : BatchBase {
     CUDA_OK(cudaFuncSetAttribute(step_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_OK(cudaFuncSetAttribute(step_kernel<Real, D, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     CUDA_OK(cudaFuncSetAttribute(query_fwd_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    CUDA_OK(cudaFuncSetAttribute(query_inv_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     { using DK = QueryDims<D>;
       const int qsmem = (int)(arena_stride<Real, DK>() * warps_per_block<Real, DK>());
       CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
@@ -786,6 +832,17 @@ struct Batch : BatchBase {
                       FwdOut<Real>{(Real*)out->qacc, (Real*)out->qfrc_constraint, out->info, out->contact_geom, (Real*)out->contact_dist,
                                    (Real*)out->contact_pos, (Real*)out->contact_frame, (Real*)out->contact_force, out->flags, (Real*)out->sensordata}};
     return launch_warps<D>(query_fwd_kernel<Real, D>, a, s);
+  }
+  int inverse(const void* qpos, const void* qvel, long long m, const void* qacc, int discrete, const ur3e_inverse_out* out, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const bool con = out && (out->contact_geom || out->contact_force);
+    const bool any = out && (con || out->qfrc_inverse || out->qfrc_constraint || out->info);
+    const std::string err = inverse_query_check(qpos != nullptr, qvel != nullptr, m, n, qacc != nullptr, out != nullptr, con, any, NCMAX);
+    if (!err.empty()) return set_err("inverse: " + err);
+    // read-only, like query(): last_stream stays that of the latest state-changing call
+    QIArgs<Real, D> a{d_model, d_state, (const Real*)qpos, (const Real*)qvel, m, (const Real*)qacc, discrete != 0,
+                      InvOut<Real>{(Real*)out->qfrc_inverse, (Real*)out->qfrc_constraint, out->info, out->contact_geom, (Real*)out->contact_force}};
+    return launch_warps<D>(query_inv_kernel<Real, D>, a, s, m);
   }
   // ---- offscreen rendering (render.cuh); renderers and the pose scratch live until the batch is destroyed
   struct Render { QueryEntry<Real>* table; RenderGeom<Real>* geoms; int k; RenderCam<Real> cam; };

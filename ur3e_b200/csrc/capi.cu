@@ -119,6 +119,10 @@ int ur3e_batch_max_contacts(const ur3e_batch* b) { GUARD(b); return b->impl->max
 int ur3e_batch_forward(ur3e_batch* b, const void* ctrl, const ur3e_forward_out* out, void* stream) {
   GUARD(b); return b->impl->forward(ctrl, out, (cudaStream_t)stream);
 }
+int ur3e_batch_inverse(ur3e_batch* b, const void* qpos, const void* qvel, int64_t m, const void* qacc, int32_t discrete, const ur3e_inverse_out* out,
+                       void* stream) {
+  GUARD(b); return b->impl->inverse(qpos, qvel, m, qacc, discrete, out, (cudaStream_t)stream);
+}
 int ur3e_batch_render_create(ur3e_batch* b, const ur3e_camera* cam, const int32_t* geom_ids, int32_t k, const float* rgba, int32_t width, int32_t height) {
   GUARD(b);
   try { return b->impl->render_create(cam, geom_ids, k, rgba, width, height); } catch (const std::exception& e) { return set_err(e.what()); }

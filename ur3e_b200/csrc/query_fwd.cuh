@@ -37,6 +37,34 @@ inline std::string forward_query_check(bool out, bool con, bool any, int ncmax) 
   return "";
 }
 
+// The contact list (d.contact[k].geom1 / geom2, dist, pos, frame) of the `ncon` contacts collision() found, padded to C = D::MAXCON
+// entries with geom -1 and zeros; any output may be null.  Call it right after collision(), while every contact frame is intact (the
+// solver keeps its cone Hessians in the tangents' storage).  Shared by the forward and the inverse query.
+template <typename Real, typename D>
+UR3E_HD void contact_list_out(const DevModel<Real>& m, const Arena<Real, D>& s, int ncon, int32_t* geom, Real* dist, Real* pos, Real* frame) {
+  constexpr int C = D::MAXCON;
+  if (geom) {
+    WARP_FOR(i, 2 * C) {
+      const int c = i >> 1;
+      geom[i] = c < ncon ? ((i & 1) ? m.pair_src_g2[s.con_pair[c]] : m.pair_src_g1[s.con_pair[c]]) : -1;
+    }
+  }
+  if (dist) { WARP_FOR(c, C) dist[c] = c < ncon ? s.con_dist[c] : Real(0); }
+  if (pos) { WARP_FOR(i, 3 * C) { const int c = i / 3; pos[i] = c < ncon ? s.con_pos[c][i - 3 * c] : Real(0); } }
+  if (frame) { WARP_FOR(i, 9 * C) { const int c = i / 9; frame[i] = c < ncon ? s.cu.frame[c][i - 9 * c] : Real(0); } }
+}
+
+// mj_contactForce of every contact from the rows' efc_force, [C][6]: [fn, ft1, ft2, 0, 0, 0] in the contact frame.  s.ncon is the
+// count make_constraint() left, the contacts it found rows for (con_row[c] is the normal row, the two tangent rows follow); a contact
+// past it, cut on a row overflow, and the padding report zero.
+template <typename Real, typename D>
+UR3E_HD void contact_force_out(const Arena<Real, D>& s, Real* out) {
+  WARP_FOR(i, 6 * D::MAXCON) {
+    const int c = i / 6, k = i - 6 * c;
+    out[i] = (c < s.ncon && k < 3) ? s.efc_force[s.con_row[c] + k] : Real(0);
+  }
+}
+
 // The full pass runs when an output needs dynamics (qacc, qfrc_constraint, contact_force, sensordata); otherwise the
 // contacts-only pass runs (contact geometry, info, flags): kinematics and collision alone, since collision reads nothing else.
 template <typename Real>
@@ -63,17 +91,7 @@ UR3E_HD void forward_query_env(const DevModel<Real>& m, Arena<Real, D>& s, const
   if (full) dynamics(m, s);
   collision(m, s);
   const int ncon = s.ncon;
-  if constexpr (C > 0) {
-    if (o.contact_geom) {
-      WARP_FOR(i, 2 * C) {
-        const int c = i >> 1;
-        o.contact_geom[i] = c < ncon ? ((i & 1) ? m.pair_src_g2[s.con_pair[c]] : m.pair_src_g1[s.con_pair[c]]) : -1;
-      }
-    }
-    if (o.contact_dist) { WARP_FOR(c, C) o.contact_dist[c] = c < ncon ? s.con_dist[c] : Real(0); }
-    if (o.contact_pos) { WARP_FOR(i, 3 * C) { const int c = i / 3; o.contact_pos[i] = c < ncon ? s.con_pos[c][i - 3 * c] : Real(0); } }
-    if (o.contact_frame) { WARP_FOR(i, 9 * C) { const int c = i / 9; o.contact_frame[i] = c < ncon ? s.cu.frame[c][i - 9 * c] : Real(0); } }
-  }
+  if constexpr (C > 0) contact_list_out(m, s, ncon, o.contact_geom, o.contact_dist, o.contact_pos, o.contact_frame);
   if (o.flags) {
     const int f = contact_bits(m, s);
     IF_LANE0 o.flags[0] = f;
@@ -84,13 +102,7 @@ UR3E_HD void forward_query_env(const DevModel<Real>& m, Arena<Real, D>& s, const
     solve(m, s, opt);
   }
   if constexpr (C > 0) {
-    if (o.contact_force) {
-      // s.ncon <= ncon: the contacts make_constraint() found rows for; con_row[c] is the normal row, the two tangent rows follow
-      WARP_FOR(i, 6 * C) {
-        const int c = i / 6, k = i - 6 * c;
-        o.contact_force[i] = (c < s.ncon && k < 3) ? s.efc_force[s.con_row[c] + k] : Real(0);
-      }
-    }
+    if (o.contact_force) contact_force_out(s, o.contact_force);
   }
   if (o.qacc) { WARP_FOR(d, nv_<D>(m)) o.qacc[d] = s.qacc[d]; }
   if (o.qfrc_constraint) { WARP_FOR(d, nv_<D>(m)) o.qfrc_constraint[d] = s.qfrc_constraint[d]; }
