@@ -266,6 +266,51 @@ typedef struct ur3e_rollout_out {
 } ur3e_rollout_out;
 int ur3e_batch_rollout(ur3e_batch* b, const int32_t* src_env_ids_dev, const void* qpos0_dev, const void* qvel0_dev, const void* qacc_warmstart0_dev,
                        int64_t m, int32_t T, const void* actions_dev, const ur3e_rollout_out* out, void* stream);
+/* Inverse kinematics (dm_control.utils.inverse_kinematics.qpos_from_site_pose, batched): the joint positions that put one object at a
+ * target position and / or orientation.  For reset and goal distributions at sampled tool poses, task-space waypoints converted into
+ * joint waypoints for UR3E_CTRL_PD_JOINT, and reachability checks.
+ * ur3e_batch_ik_create compiles a problem family and returns its id (>= 0); the batch owns it until ur3e_batch_destroy:
+ *   objtype / objid: one object of the kinds ur3e_batch_query_create accepts (UR3E_OBJ_SITE, UR3E_OBJ_XBODY, UR3E_OBJ_BODY,
+ *     UR3E_OBJ_GEOM); its world point p(q) and frame R(q) are what a kinematics query returns for it.
+ *   joint_ids [nj], 1 <= nj <= nv: distinct hinge or slide joints of the loaded model, the only qpos entries the solve changes.
+ * ur3e_batch_ik solves m problems, one warp each.  Start configuration q (all nq entries), exactly one source:
+ *   env_ids_dev int32 [m]: the stored qpos of those environments (ids may repeat; an id outside [0, n) gives NaN qpos and err_norm
+ *     and status 3);  qpos0_dev [m, nq] (batch dtype): given configurations;  neither: every environment's stored qpos (m = n).
+ * Targets (batch dtype, at least one): target_pos_dev [m, 3] world position p*; target_quat_dev [m, 4] world orientation q*
+ * (w, x, y, z; normalised first, a zero quaternion is the identity).  For step = 0 .. max_steps - 1:
+ *   kinematics at q;  e_pos = p* - p,  e_rot = the rotation vector of R(q*) R(q)^T (world frame);
+ *   err_norm = |e_pos| + rot_weight |e_rot| (dm_control's sum of norms);  err_norm < tol: converged (status 0);
+ *   J = the r x nj block of [jacp; jacr] at the object's point for the joints' dofs, r = 3 or 6 (rows for the targets given);
+ *   lambda = regularization_strength if err_norm > regularization_threshold, else 0;  dq = (J^T J + lambda I)^-1 J^T e, solved as
+ *     J^T (J J^T + lambda I)^-1 e when r <= nj (the smaller SPD system, at most 6 x 6); with lambda = 0 a pivot below 1e-13
+ *     (float64) / 1e-5 (float32) of the system's largest diagonal entry contributes zero, so dq is the minimum-norm least-squares
+ *     step except at exact singularities;
+ *   err_norm / |dq| > progress_thresh: insufficient progress (status 2), dq not applied;
+ *   dq scaled down to max_update_norm; added to the joints' qpos; every limited joint clamped to its jnt_range.
+ * max_steps updates applied without convergence: status 1.
+ * Differences from dm_control: the limit clamp (runs whose iterates stay inside the limits are dm_control's); err_norm and steps
+ * describe the returned qpos (its error, updates applied; converged means it is within tol); any kinematics-query object, not
+ * only sites; with lambda = 0 the minimum-norm step (dm_control's lstsq(J^T J, J^T e, rcond=-1) keeps rounding-noise directions
+ * of J^T J when r < nj).  Only the selected joints' qpos entries change (all others are copied bit for bit); equality constraints
+ * (the 2F85's four-bar) and contacts are not considered.
+ * opt: NULL = the defaults, dm_control's: tol 1e-14 (float64) / 1e-5 (float32), rot_weight 1, regularization_threshold 0.1,
+ * regularization_strength 3e-2, max_update_norm 2, progress_thresh 20, max_steps 100.  The float32 tol sits above the float32 noise
+ * floor of err_norm (DESIGN §3).
+ * Outputs (device, any may be NULL, not all): qpos [m, nq] (batch dtype), err_norm [m] (batch dtype), info int32 [m, 2] = steps,
+ * status.
+ * Rejected: an unknown id, m < 1 or m > 2^31 - 1, both env_ids_dev and qpos0_dev, m != n when neither is given, no target, out NULL,
+ * every output NULL, tol / rot_weight / regularization_threshold / regularization_strength < 0 or NaN, max_update_norm or progress_thresh
+ * not > 0, max_steps outside [1, 10000].
+ * Asynchronous on `stream`, one kernel launch; no record is read beyond qpos and none is written (like the queries, the call does not
+ * become the stream ur3e_batch_step_host orders itself after). */
+typedef struct ur3e_ik_options {
+  double tol, rot_weight, regularization_threshold, regularization_strength, max_update_norm, progress_thresh;
+  int32_t max_steps, reserved_;
+} ur3e_ik_options;
+typedef struct ur3e_ik_out { void* qpos; void* err_norm; int32_t* info; } ur3e_ik_out;
+int ur3e_batch_ik_create(ur3e_batch* b, int32_t objtype, int32_t objid, const int32_t* joint_ids, int32_t nj);
+int ur3e_batch_ik(ur3e_batch* b, int ik_id, const int32_t* env_ids_dev, const void* qpos0_dev, int64_t m, const void* target_pos_dev,
+                  const void* target_quat_dev, const ur3e_ik_options* opt, const ur3e_ik_out* out, void* stream);
 
 #ifdef __cplusplus
 }

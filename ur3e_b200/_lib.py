@@ -55,6 +55,20 @@ class RolloutOut(C.Structure):
     _fields_ = [(n, C.c_void_p) for n in ROLLOUT_OUTPUTS]
 
 
+class IKOptions(C.Structure):
+    """ur3e_ik_options"""
+    _fields_ = [(n, C.c_double) for n in ("tol", "rot_weight", "regularization_threshold", "regularization_strength", "max_update_norm",
+                                          "progress_thresh")] + [("max_steps", C.c_int32), ("reserved_", C.c_int32)]
+
+
+# ur3e_ik_out: the three device pointers of ur3e_batch_ik, in this order (IK_OUTPUTS)
+IK_OUTPUTS = ("qpos", "err_norm", "info")
+
+
+class IKOut(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in IK_OUTPUTS]
+
+
 class Camera(C.Structure):
     """ur3e_camera: anchor (objtype -1 = world, OBJ_XBODY or OBJ_SITE; objid), pos / xyaxes in the anchor frame, fovy (degrees), znear, zfar."""
     _fields_ = [("objtype", C.c_int32), ("objid", C.c_int32), ("pos", C.c_double * 3), ("xyaxes", C.c_double * 6), ("fovy", C.c_double),
@@ -66,7 +80,8 @@ EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_mod
            "ur3e_batch_step", "ur3e_batch_step_host", "ur3e_batch_get_state", "ur3e_batch_set_state", "ur3e_batch_stats", "ur3e_batch_set_sensor_buffer",
            "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
            "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward",
-           "ur3e_batch_render_create", "ur3e_batch_render", "ur3e_batch_rollout", "ur3e_batch_inverse"]
+           "ur3e_batch_render_create", "ur3e_batch_render", "ur3e_batch_rollout", "ur3e_batch_inverse",
+           "ur3e_batch_ik_create", "ur3e_batch_ik"]
 
 _lib = None
 
@@ -114,6 +129,8 @@ def load():
     L.ur3e_batch_render_create.argtypes = [vp, C.POINTER(Camera), C.POINTER(C.c_int32), C.c_int32, C.POINTER(C.c_float), C.c_int32, C.c_int32]
     L.ur3e_batch_render.argtypes = [vp, C.c_int, vp, i64, vp, vp, vp, vp]
     L.ur3e_batch_rollout.argtypes = [vp, vp, vp, vp, vp, i64, C.c_int32, vp, C.POINTER(RolloutOut), vp]
+    L.ur3e_batch_ik_create.argtypes = [vp, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32]
+    L.ur3e_batch_ik.argtypes = [vp, C.c_int, vp, vp, i64, vp, vp, C.POINTER(IKOptions), C.POINTER(IKOut), vp]
     _lib = L
     return L
 

@@ -36,6 +36,7 @@ def env_config(**kw):
 ForwardResult = namedtuple("ForwardResult", _lib.FORWARD_OUTPUTS)
 RolloutResult = namedtuple("RolloutResult", _lib.ROLLOUT_OUTPUTS)
 InverseResult = namedtuple("InverseResult", _lib.INVERSE_OUTPUTS)
+IKResult = namedtuple("IKResult", _lib.IK_OUTPUTS)
 
 
 class SimBatch:
@@ -247,6 +248,12 @@ class SimBatch:
         _lib.check(self._L.ur3e_batch_inverse(self.ptr, qp, qv, m, a, int(bool(discrete)), C.byref(st), self._stream()), "ur3e_batch_inverse")
         return outs
 
+    def ik(self, obj, joints=None):
+        """An inverse-kinematics solver of this batch (ur3e_batch_ik_create) for one object, (kind, name_or_id) with Query's kinds, moving
+        `joints` (names or ids of hinge joints; None = the joints driven by joint-transmission actuators, the six arm joints of the
+        reference models).  See IK."""
+        return IK(self, obj, joints)
+
     def renderer(self, width, height, camera, geoms=None, rgba=None):
         """An offscreen renderer of this batch (ur3e_batch_render_create): width x height images of `geoms` (names or ids of box /
         plane geoms; None = every geom whose geom_rgba alpha is > 0) seen from `camera` (a dict, see make_camera).  rgba [k, 4]
@@ -409,6 +416,92 @@ class Query:
                                                               M=(M, (n, nv, nv), None), qfrc_bias=(qfrc_bias, (n, nv), None)))
         _lib.check(self.batch._L.ur3e_batch_query_jac(self.batch.ptr, self.id, *map(_ptr, outs.values()), self.batch._stream()), "ur3e_batch_query_jac")
         return tuple(outs.values())
+
+
+class IK:
+    """Joint positions that put one object at target poses (ur3e_batch_ik): dm_control's qpos_from_site_pose, one problem per warp.
+
+    Calling it launches one kernel on the current torch stream and returns IKResult(qpos [m, nq], err_norm [m], info int32 [m, 2] =
+    steps, status), None for an output not asked for.  Each output argument (qpos_out for qpos) is False, True (a tensor owned by the
+    solver, reallocated when m changes) or a caller tensor.  Start configurations, at most one source:
+
+        env_ids int32 [m] (CUDA)           the stored qpos of those environments (repeats allowed; an id outside [0, n) gives NaN
+                                           qpos and err_norm and status 3)
+        qpos [m, nq]                       given configurations
+        neither                            every environment's stored qpos (m = n)
+
+    Targets, at least one: target_pos [m, 3] (world position of the object's point) and / or target_quat [m, 4] (world orientation of
+    its frame, w x y z; normalised, a zero quaternion is the identity).  Per problem, for step = 0 .. max_steps - 1: err_norm =
+    |p* - p| + rot_weight |rotvec(R* R^T)|; converged (status 0) when err_norm < tol; else the damped least-squares step
+    dq = (J^T J + lambda I)^-1 J^T e with lambda = regularization_strength while err_norm > regularization_threshold (else 0, the
+    minimum-norm step); status 2 when err_norm / |dq| > progress_thresh (dq not applied); dq scaled to at most max_update_norm,
+    added to the joints' qpos, limited joints clamped to their range.  Status 1: max_steps updates without convergence.
+
+    tol None is dm_control's 1e-14 in float64 and 1e-5 in float32 (above float32's noise floor of err_norm, DESIGN §3); the other
+    defaults are dm_control's.  Differences from dm_control: the clamp to joint limits; err_norm and steps describe the returned qpos;
+    any object kind; the minimum-norm step at lambda = 0.  Only the selected joints' entries of qpos change (the rest are copied bit
+    for bit); equality constraints (the 2F85's four-bar) and contacts are ignored.  The batch's records are not modified: write a
+    solution with set_state.
+    """
+
+    def __init__(self, batch, obj, joints=None):
+        self.batch = batch
+        kind, o = obj
+        if kind not in Query.KINDS:
+            raise ValueError("object kind %r is not one of %s" % (kind, sorted(Query.KINDS)))
+        if isinstance(o, str):
+            i = batch.model.name2id(_lib.OBJ_BODY if kind == "xbody" else Query.KINDS[kind], o)
+            if i < 0:
+                raise KeyError("%s %r is not in the model" % (kind, o))
+            o = i
+        if joints is None:
+            trn = np.asarray(batch.model.array("actuator_trntype")).reshape(-1)
+            tid = np.asarray(batch.model.array("actuator_trnid")).reshape(len(trn), -1)[:, 0]
+            joints = [int(j) for t, j in zip(trn, tid) if t == 0]   # mjTRN_JOINT
+        ids = []
+        for j in joints:
+            i = batch.model.name2id(_lib.OBJ_JOINT, j) if isinstance(j, str) else int(j)
+            if i < 0:
+                raise KeyError("joint %r is not in the model" % (j,))
+            ids.append(i)
+        self.joints, self.nj = ids, len(ids)
+        arr = (C.c_int32 * max(self.nj, 1))(*ids)
+        iid = batch._L.ur3e_batch_ik_create(batch.ptr, Query.KINDS[kind], int(o), arr, self.nj)
+        if iid < 0:
+            raise ValueError("ur3e_batch_ik_create: " + _lib.last_error())
+        self.id = iid
+        self._own, self._m = {}, None
+
+    def __call__(self, target_pos=None, target_quat=None, env_ids=None, qpos=None, *, qpos_out=True, err_norm=True, info=True, tol=None,
+                 rot_weight=1.0, regularization_threshold=0.1, regularization_strength=3e-2, max_update_norm=2.0, progress_thresh=20.0,
+                 max_steps=100):
+        b = self.batch
+        if env_ids is not None and qpos is not None:
+            raise ValueError("ik: give env_ids or qpos, not both")
+        if target_pos is None and target_quat is None:
+            raise ValueError("ik: needs target_pos and / or target_quat")
+        ids = qp = None
+        if qpos is not None:
+            m = int(qpos.shape[0]) if qpos.dim() >= 1 else 0
+            qp = b._chk(qpos, (m, b.model.nq))
+        elif env_ids is not None:
+            m = int(env_ids.numel())
+            ids = b._chk(env_ids, (m,), torch.int32)
+        else:
+            m = b.n
+        tp = b._chk(target_pos, (m, 3)) if target_pos is not None else None
+        tq = b._chk(target_quat, (m, 4)) if target_quat is not None else None
+        if self._m != m:
+            self._own, self._m = {}, m   # owned outputs follow the latest call's m
+        outs = IKResult(**_outs(b, self._own, "IK", dict(qpos=(qpos_out, (m, b.model.nq), None), err_norm=(err_norm, (m,), None),
+                                                         info=(info, (m, 2), torch.int32))))
+        if tol is None:
+            tol = 1e-14 if b.dtype == torch.float64 else 1e-5
+        opt = _lib.IKOptions(float(tol), float(rot_weight), float(regularization_threshold), float(regularization_strength), float(max_update_norm),
+                             float(progress_thresh), int(max_steps), 0)
+        st = _lib.IKOut(*[o.data_ptr() if o is not None else None for o in outs])
+        _lib.check(b._L.ur3e_batch_ik(b.ptr, self.id, ids, qp, m, tp, tq, C.byref(opt), C.byref(st), b._stream()), "ur3e_batch_ik")
+        return outs
 
 
 def _outs(batch, own, what, table):

@@ -43,6 +43,10 @@ struct BatchBase {
   // offscreen rendering (render.cuh): the batch owns its renderers and their pose scratch; render_create returns the renderer's id
   virtual int render_create(const ur3e_camera* cam, const int32_t* geom_ids, int k, const float* rgba, int width, int height) = 0;
   virtual int render(int id, const int32_t* env_ids, long long m, uint8_t* rgb, void* depth, int32_t* seg, cudaStream_t s) = 0;
+  // inverse kinematics (ik.cuh): the batch owns the compiled problem families; ik_create returns the family's id
+  virtual int ik_create(int32_t objtype, int32_t objid, const int32_t* joint_ids, int nj) = 0;
+  virtual int ik(int id, const int32_t* env_ids, const void* qpos0, long long m, const void* target_pos, const void* target_quat,
+                 const ur3e_ik_options* opt, const ur3e_ik_out* out, cudaStream_t s) = 0;
   // T tiered steps of m scratch copies of records (src ids) or of fresh records (qpos0 / qvel0 / ws0); the batch is not modified
   virtual int rollout(const int32_t* src, const void* qpos0, const void* qvel0, const void* ws0, long long m, int T, const void* act,
                       const ur3e_rollout_out* out, cudaStream_t s) = 0;

@@ -12,6 +12,7 @@
 #include "compile_model.h"
 #include "merge_bodies.h"
 #include "env.cuh"
+#include "ik.cuh"
 #include "query.cuh"
 #include "query_fwd.cuh"
 #include "query_inv.cuh"
@@ -388,6 +389,54 @@ __global__ void __launch_bounds__(warps_per_block<Real, D>() * 32, 1) query_inv_
 }
 
 template <typename Real, typename D>
+struct IKArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;
+  const IkTable<Real>* tab;
+  long long n, count;                 // batch size, problems
+  const int* env_ids;                 // [count] or null
+  const Real* qpos0;                  // [count, nq] or null (neither: environment i)
+  const Real* target_pos; const Real* target_quat;   // [count, 3], [count, 4]; either may be null
+  IkOpts<Real> opt;
+  Real* qpos; Real* err_norm; int32_t* info;         // [count, nq], [count], [count, 2]; any may be null
+};
+
+// Inverse kinematics (ik.cuh ik_env): one warp per problem on the kinematics queries' arena; reads qpos of the record or of the
+// caller's array, never writes a record.  An environment id outside [0, n) gets NaN qpos and err_norm and status IK_BAD_ENV.
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) ik_kernel(const IKArgs<Real, D> a) {
+  using DK = QueryDims<D>;
+  constexpr int WPB = warps_per_block<Real, DK>();
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long i = (long long)blockIdx.x * WPB + warp;
+  if (i >= a.count) return;
+  const DevModel<Real>& m = *a.m;
+  const long long nq = m.nq;
+  Real* const qo = a.qpos ? a.qpos + i * nq : nullptr;
+  Real* const eo = a.err_norm ? a.err_norm + i : nullptr;
+  int32_t* const io = a.info ? a.info + 2 * i : nullptr;
+  const Real* src;
+  if (a.qpos0) src = a.qpos0 + i * nq;
+  else {
+    const long long e = a.env_ids ? (long long)a.env_ids[i] : i;
+    if (e < 0 || e >= a.n) {
+      const Real nan = std::numeric_limits<Real>::quiet_NaN();
+      if (qo) { WARP_FOR(j, m.nq) qo[j] = nan; }
+      IF_LANE0 { if (eo) *eo = nan; if (io) { io[0] = 0; io[1] = IK_BAD_ENV; } }
+      return;
+    }
+    src = a.st[e].qpos;
+  }
+  Arena<Real, DK>& s = *reinterpret_cast<Arena<Real, DK>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, DK>());
+  WARP_FOR(j, m.nq) s.st.qpos[j] = src[j];
+  WARP_SYNC();
+  const IkResult<Real> r = ik_env(m, s, *a.tab, a.target_pos ? a.target_pos + 3 * i : nullptr, a.target_quat ? a.target_quat + 4 * i : nullptr, a.opt);
+  if (qo) { WARP_FOR(j, m.nq) qo[j] = s.st.qpos[j]; }
+  IF_LANE0 { if (eo) *eo = r.err_norm; if (io) { io[0] = r.steps; io[1] = r.status; } }
+}
+
+template <typename Real, typename D>
 struct RPArgs {
   const DevModel<Real>* m;
   const EnvState<Real, D>* st;
@@ -498,6 +547,7 @@ struct Batch : BatchBase {
     for (auto e : ev_pool) cudaEventDestroy(e);
     for (auto& q : queries) cudaFree(q.table);
     for (auto& r : renders) { cudaFree(r.table); cudaFree(r.geoms); }
+    for (auto t : iks) cudaFree(t);
     cudaFree(d_pose); cudaFree(d_roll);
     if (own_stream) cudaStreamDestroy(own_stream);
     if (own_stream2) cudaStreamDestroy(own_stream2);
@@ -599,7 +649,8 @@ struct Batch : BatchBase {
       const int qsmem = (int)(arena_stride<Real, DK>() * warps_per_block<Real, DK>());
       CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
       CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
-      CUDA_OK(cudaFuncSetAttribute(render_pose_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
+      CUDA_OK(cudaFuncSetAttribute(render_pose_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
+      CUDA_OK(cudaFuncSetAttribute(ik_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
     static_assert(sizeof(Real) * 12 * (RENDER_MAX_GEOMS + 1) + sizeof(RenderGeom<Real>) * RENDER_MAX_GEOMS <= 48 * 1024, "render_kernel's staged scene fits the default shared-memory limit");
     cudaDeviceProp prop; CUDA_OK(cudaGetDeviceProperties(&prop, dev)); sm_count = prop.multiProcessorCount;
     if constexpr (HAS_LITE) {
@@ -882,6 +933,34 @@ struct Batch : BatchBase {
     ++launches;
     CUDA_OK(cudaGetLastError());
     return 0;
+  }
+  // ---- inverse kinematics (ik.cuh); the tables live until the batch is destroyed
+  std::vector<IkTable<Real>*> iks;
+  int ik_create(int32_t objtype, int32_t objid, const int32_t* joint_ids, int nj) override {
+    CUDA_OK(cudaSetDevice(device));
+    IkTable<Real> tab;
+    const std::string err = compile_ik<Real>(hm, objtype, objid, joint_ids, nj, tab);
+    if (!err.empty()) return set_err("ik_create: " + err);
+    IkTable<Real>* d = nullptr;
+    CUDA_OK(cudaMalloc(&d, sizeof tab));
+    iks.push_back(d);
+    CUDA_OK(cudaMemcpy(d, &tab, sizeof tab, cudaMemcpyHostToDevice));
+    return (int)iks.size() - 1;
+  }
+  int ik(int id, const int32_t* env_ids, const void* qpos0, long long m, const void* target_pos, const void* target_quat, const ur3e_ik_options* opt,
+         const ur3e_ik_out* out, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const bool any = out && (out->qpos || out->err_norm || out->info);
+    const std::string err = ik_check(id, (int)iks.size(), m, n, env_ids != nullptr, qpos0 != nullptr, target_pos != nullptr, target_quat != nullptr,
+                                     out != nullptr, any, opt);
+    if (!err.empty()) return set_err("ik: " + err);
+    const ur3e_ik_options o = opt ? *opt : ur3e_ik_options{ik_default_tol<Real>(), 1.0, 0.1, 3e-2, 2.0, 20.0, 100, 0};
+    const IkOpts<Real> ko{(Real)o.tol, (Real)o.rot_weight, (Real)o.regularization_threshold, (Real)o.regularization_strength, (Real)o.max_update_norm,
+                          (Real)o.progress_thresh, o.max_steps};
+    // read-only, like query(): last_stream stays that of the latest state-changing call
+    IKArgs<Real, D> a{d_model, d_state, iks[id], n, m, env_ids, (const Real*)qpos0, (const Real*)target_pos, (const Real*)target_quat, ko,
+                      (Real*)out->qpos, (Real*)out->err_norm, out->info};
+    return launch_warps<QueryDims<D>>(ik_kernel<Real, D>, a, s, m);
   }
   // ---- rollouts: T tiered steps (step_range) of a scratch batch of m records on the counter slot ROLLOUT_SLOT.  The workspace is
   // grown to the largest m seen: records [m], the three tier lists [m], and obs [m, obs_dim], reward [m], terminated [m] and

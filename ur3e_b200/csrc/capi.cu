@@ -134,5 +134,13 @@ int ur3e_batch_rollout(ur3e_batch* b, const int32_t* src_env_ids_dev, const void
                        int64_t m, int32_t T, const void* actions_dev, const ur3e_rollout_out* out, void* stream) {
   GUARD(b); return b->impl->rollout(src_env_ids_dev, qpos0_dev, qvel0_dev, qacc_warmstart0_dev, m, T, actions_dev, out, (cudaStream_t)stream);
 }
+int ur3e_batch_ik_create(ur3e_batch* b, int32_t objtype, int32_t objid, const int32_t* joint_ids, int32_t nj) {
+  GUARD(b);
+  try { return b->impl->ik_create(objtype, objid, joint_ids, nj); } catch (const std::exception& e) { return set_err(e.what()); }
+}
+int ur3e_batch_ik(ur3e_batch* b, int ik_id, const int32_t* env_ids_dev, const void* qpos0_dev, int64_t m, const void* target_pos_dev,
+                  const void* target_quat_dev, const ur3e_ik_options* opt, const ur3e_ik_out* out, void* stream) {
+  GUARD(b); return b->impl->ik(ik_id, env_ids_dev, qpos0_dev, m, target_pos_dev, target_quat_dev, opt, out, (cudaStream_t)stream);
+}
 
 }  // extern "C"
