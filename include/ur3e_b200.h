@@ -311,6 +311,29 @@ typedef struct ur3e_ik_out { void* qpos; void* err_norm; int32_t* info; } ur3e_i
 int ur3e_batch_ik_create(ur3e_batch* b, int32_t objtype, int32_t objid, const int32_t* joint_ids, int32_t nj);
 int ur3e_batch_ik(ur3e_batch* b, int ik_id, const int32_t* env_ids_dev, const void* qpos0_dev, int64_t m, const void* target_pos_dev,
                   const void* target_quat_dev, const ur3e_ik_options* opt, const ur3e_ik_out* out, void* stream);
+/* Geom distances (mj_geomDistance(m, d, geom1, geom2, distmax, fromto), batched over k pairs and m states): the signed distance and
+ * the closest points of box and plane geoms.  For clearance checks of IK solutions, reset samples or waypoints at given
+ * configurations, collision-avoidance costs along rollout trajectories, and graded (signed) versions of contact predicates.
+ * ur3e_batch_distance_create compiles a pair set and returns its id (>= 0); the batch owns it until ur3e_batch_destroy:
+ *   geom1 [k], geom2 [k], 1 <= k <= 256: box or plane geoms of the loaded model (contype / conaffinity and the candidate list play no
+ *     part); a geom paired with itself and a plane paired with a plane are rejected.
+ * ur3e_batch_distance evaluates the k pairs at m states, one warp each.  Configuration q (all nq entries), exactly one source:
+ *   env_ids_dev int32 [m]: the stored qpos of those environments (ids may repeat; an id outside [0, n) gives NaN dist and fromto);
+ *   qpos_dev [m, nq] (batch dtype): given configurations;  neither: every environment's stored qpos (m = n).
+ * Per pair, at the geoms' world poses of q:
+ *   box-box, disjoint (a SAT axis separates): dist = the exact Euclidean distance of the two solids, fromto its closest points;
+ *   box-box, overlapping: dist < 0 is the smallest dist of the collider's box-box contacts at margin 0 (for a pair of the step's
+ *     candidate list, the deepest contact the step and ur3e_batch_forward see), fromto = pos -/+ dist/2 normal;
+ *   plane-box: the plane is an infinite half-space (as in the step's collision); dist = the smallest signed height of the box's 8
+ *     vertices over it, fromto = that vertex projected onto the plane and the vertex.
+ *   fromto[0:3] lies on geom1 and fromto[3:6] on geom2 (swapping a pair swaps the halves).  When no pair of points is closer than
+ *   distmax (dist >= distmax), dist = distmax and fromto = 0.
+ * Outputs (device, batch dtype, either may be NULL, not both): dist [m, k], fromto [m, k, 6].
+ * Rejected: an unknown id, m < 1 or m > 2^31 - 1, both env_ids_dev and qpos_dev, m != n when neither is given, both outputs NULL,
+ * distmax NaN.  Asynchronous on `stream`, one kernel launch; no record is read beyond qpos and none is written. */
+int ur3e_batch_distance_create(ur3e_batch* b, const int32_t* geom1, const int32_t* geom2, int32_t k);
+int ur3e_batch_distance(ur3e_batch* b, int distance_id, const int32_t* env_ids_dev, const void* qpos_dev, int64_t m, double distmax, void* dist_dev,
+                        void* fromto_dev, void* stream);
 
 #ifdef __cplusplus
 }

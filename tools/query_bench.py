@@ -1,4 +1,4 @@
-"""Query timing (ur3e_batch_query, ur3e_batch_query_jac, ur3e_batch_forward, ur3e_batch_inverse) on the float32 main.xml batch, beside one env-step for scale.
+"""Query timing (ur3e_batch_query, ur3e_batch_query_jac, ur3e_batch_forward, ur3e_batch_inverse, ur3e_batch_distance) on the float32 main.xml batch, beside one env-step for scale.
 
     python tools/query_bench.py [--envs 65536] [--settle 1500] [--launches 500] [--out FILE]
 
@@ -15,9 +15,13 @@ state.  Then, with CUDA events around `--launches` back-to-back launches after a
   inv_a  qfrc_inverse at the stored state, qacc from a previous fwd_b   (SimBatch.inverse: mj_inverse, no solver iterations)
   inv_b  given states: a 16 x 4 096 rollout trajectory flattened to 65 536 states, discrete convention, qfrc_inverse + contact_force
          (inverse-dynamics labels along rollouts)
+  dist_a the candidate pairs (SimBatch.distance(None): main.xml's 60) at the stored state, dist only, distmax = inf
+         (the minimum clearance over everything the step can collide)
+  dist_b the self and table pairs (robot geoms against each other and against the table) on the same 16 x 4 096 trajectory, given
+         states, dist + fromto, distmax = inf   (a collision-avoidance cost along rollouts)
 and one env-step over `--launches / 10` steps.  The byte floor counts what a call must move: the record fields it reads (qpos and
 qvel for kin, jac and inv_a; the whole 544-byte record for fwd, which the kernel loads whole, and ctrl for fwd_b; the given qpos and
-qvel for inv_b; qacc for inv) and the outputs written.
+qvel for inv_b; qacc for inv; qpos for dist) and the outputs written.
 The L2 is not flushed between launches: kin_a's working set (qpos + qvel of the records, 18 MB of outputs) stays in the 126 MB L2;
 kin_b's 363 MB of outputs, jac_a's 142 MB and jac_b's 110 MB per call at 65 536 environments do not.  Prints one JSON line with the
 GPU's name, power limit and SM clock.
@@ -128,11 +132,21 @@ def main():
                     "bytes_floor": T * mr * (4 * (nq + nv) + 4 * nv + 4 * (nv + 6 * C))}
     ib = b.inverse(ta, state=(tq, tv), discrete=True, qfrc_inverse=False, info=True).info
     res["inv_b"]["mean_ncon"] = ib[:, 0].double().mean().item(); res["inv_b"]["mean_nefc"] = ib[:, 1].double().mean().item()
+    # geom distances: the candidate list at the stored state (dist_a); the self and table pairs along the trajectory (dist_b)
+    da = b.distance()
+    res["dist_a"] = {"pairs": da.k, "outputs": "dist, stored state", "us_per_call": timed(lambda: da(), args.launches),
+                     "bytes_floor": n * (4 * nq + 4 * da.k)}
+    name = lambda g: model.id2name(lib.OBJ_GEOM, g)
+    pairs = [(a, c) for a, c in zip(da.geom1, da.geom2) if name(c) != "fish" and (name(a) == "table" or name(a) not in ("floor", "table"))]
+    db = b.distance(pairs)
+    res["dist_b"] = {"pairs": db.k, "outputs": "dist+fromto, given states (16 x %d trajectory)" % mr,
+                     "us_per_call": timed(lambda: db(qpos=tq, fromto=True), args.launches), "bytes_floor": T * mr * (4 * nq + 4 * 7 * db.k)}
+    res["dist_a"]["min_dist_mean"] = da()[0].min(dim=1).values.double().mean().item()
     res["mean_ncon"] = b.forward(qacc=False, info=True).info[:, 0].double().mean().item()
     res["mean_nefc"] = b.forward(qacc=True, info=True).info[:, 1].double().mean().item()
     it = iter(range(10 ** 9))
     res["env_step_us"] = timed(lambda: b.step(acts[next(it) % 16]), max(args.launches // 10, 10))
-    for q in ("kin_a", "kin_b", "jac_a", "jac_b", "fwd_a", "fwd_b", "inv_a", "inv_b"):
+    for q in ("kin_a", "kin_b", "jac_a", "jac_b", "fwd_a", "fwd_b", "inv_a", "inv_b", "dist_a", "dist_b"):
         r = res[q]
         r["GB_per_s"] = r["bytes_floor"] / (r["us_per_call"] * 1e-6) / 1e9
         r["fraction_of_env_step"] = r["us_per_call"] / res["env_step_us"]

@@ -81,7 +81,7 @@ EXPORTS = ["ur3e_last_error", "ur3e_model_load", "ur3e_model_destroy", "ur3e_mod
            "ur3e_batch_launch_count", "ur3e_batch_kernel_info", "ur3e_batch_state_bytes", "ur3e_batch_tier_info", "ur3e_batch_kernel_timing", "ur3e_batch_kernel_times", "ur3e_batch_mid_tier_info",
            "ur3e_batch_query_create", "ur3e_batch_query", "ur3e_batch_query_jac", "ur3e_batch_max_contacts", "ur3e_batch_forward",
            "ur3e_batch_render_create", "ur3e_batch_render", "ur3e_batch_rollout", "ur3e_batch_inverse",
-           "ur3e_batch_ik_create", "ur3e_batch_ik"]
+           "ur3e_batch_ik_create", "ur3e_batch_ik", "ur3e_batch_distance_create", "ur3e_batch_distance"]
 
 _lib = None
 
@@ -131,6 +131,8 @@ def load():
     L.ur3e_batch_rollout.argtypes = [vp, vp, vp, vp, vp, i64, C.c_int32, vp, C.POINTER(RolloutOut), vp]
     L.ur3e_batch_ik_create.argtypes = [vp, C.c_int32, C.c_int32, C.POINTER(C.c_int32), C.c_int32]
     L.ur3e_batch_ik.argtypes = [vp, C.c_int, vp, vp, i64, vp, vp, C.POINTER(IKOptions), C.POINTER(IKOut), vp]
+    L.ur3e_batch_distance_create.argtypes = [vp, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.c_int32]
+    L.ur3e_batch_distance.argtypes = [vp, C.c_int, vp, vp, i64, C.c_double, vp, vp, vp]
     _lib = L
     return L
 

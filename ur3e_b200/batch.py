@@ -37,6 +37,7 @@ ForwardResult = namedtuple("ForwardResult", _lib.FORWARD_OUTPUTS)
 RolloutResult = namedtuple("RolloutResult", _lib.ROLLOUT_OUTPUTS)
 InverseResult = namedtuple("InverseResult", _lib.INVERSE_OUTPUTS)
 IKResult = namedtuple("IKResult", _lib.IK_OUTPUTS)
+DistanceResult = namedtuple("DistanceResult", ("dist", "fromto"))
 
 
 class SimBatch:
@@ -253,6 +254,11 @@ class SimBatch:
         `joints` (names or ids of hinge joints; None = the joints driven by joint-transmission actuators, the six arm joints of the
         reference models).  See IK."""
         return IK(self, obj, joints)
+
+    def distance(self, pairs=None):
+        """A geom-distance evaluator of this batch (ur3e_batch_distance_create) for a fixed list of pairs [(geom1, geom2), ...] of box or
+        plane geoms (names or ids); None = the model's contact candidate list (pair_geom1 / pair_geom2).  See Distance."""
+        return Distance(self, pairs)
 
     def renderer(self, width, height, camera, geoms=None, rgba=None):
         """An offscreen renderer of this batch (ur3e_batch_render_create): width x height images of `geoms` (names or ids of box /
@@ -501,6 +507,68 @@ class IK:
                              float(progress_thresh), int(max_steps), 0)
         st = _lib.IKOut(*[o.data_ptr() if o is not None else None for o in outs])
         _lib.check(b._L.ur3e_batch_ik(b.ptr, self.id, ids, qp, m, tp, tq, C.byref(opt), C.byref(st), b._stream()), "ur3e_batch_ik")
+        return outs
+
+
+class Distance:
+    """Signed distances and closest points of fixed geom pairs (ur3e_batch_distance): MuJoCo's mj_geomDistance, batched over the k
+    pairs and m states.  `geom1` / `geom2` are the resolved geom ids [k].
+
+    Calling it launches one kernel on the current torch stream and returns DistanceResult(dist [m, k], fromto [m, k, 6]), None for an
+    output not asked for; each output argument is False, True (a tensor owned by the evaluator, reallocated when m changes) or a
+    caller tensor, as in forward().  Configurations, at most one source:
+
+        env_ids int32 [m] (CUDA)           the stored qpos of those environments (repeats allowed; an id outside [0, n) gives NaN)
+        qpos [m, nq]                       given configurations, e.g. IK solutions or a flattened rollout trajectory
+        neither                            every environment's stored qpos (m = n)
+
+    Per pair: disjoint boxes give the exact distance of the two solids and its closest points; overlapping boxes give the collider's
+    deepest box-box contact (dist < 0, the contact forward() reports for a candidate pair), fromto = pos -/+ dist/2 normal; a plane is
+    an infinite half-space and a plane-box pair gives the lowest vertex's signed height, the vertex projected onto the plane and the
+    vertex.  fromto[..., 0:3] lies on geom1, fromto[..., 3:6] on geom2.  dist >= distmax gives dist = distmax and fromto = 0.  The
+    batch's records are not modified.
+    """
+
+    def __init__(self, batch, pairs=None):
+        self.batch = batch
+        if pairs is None:
+            g1 = np.asarray(batch.model.array("pair_geom1")).reshape(-1)
+            g2 = np.asarray(batch.model.array("pair_geom2")).reshape(-1)
+            pairs = list(zip(g1.tolist(), g2.tolist()))
+
+        def gid(g):
+            i = batch.model.name2id(_lib.OBJ_GEOM, g) if isinstance(g, str) else int(g)
+            if i < 0:
+                raise KeyError("geom %r is not in the model" % (g,))
+            return i
+        ids = [(gid(a), gid(b)) for a, b in pairs]
+        self.k = len(ids)
+        self.geom1 = [a for a, _ in ids]
+        self.geom2 = [b for _, b in ids]
+        k1 = max(self.k, 1)
+        did = batch._L.ur3e_batch_distance_create(batch.ptr, (C.c_int32 * k1)(*self.geom1), (C.c_int32 * k1)(*self.geom2), self.k)
+        if did < 0:
+            raise ValueError("ur3e_batch_distance_create: " + _lib.last_error())
+        self.id = did
+        self._own, self._m = {}, None
+
+    def __call__(self, env_ids=None, qpos=None, distmax=float("inf"), dist=True, fromto=False):
+        b = self.batch
+        if env_ids is not None and qpos is not None:
+            raise ValueError("distance: give env_ids or qpos, not both")
+        ids = qp = None
+        if qpos is not None:
+            m = int(qpos.shape[0]) if qpos.dim() >= 1 else 0
+            qp = b._chk(qpos, (m, b.model.nq))
+        elif env_ids is not None:
+            m = int(env_ids.numel())
+            ids = b._chk(env_ids, (m,), torch.int32)
+        else:
+            m = b.n
+        if self._m != m:
+            self._own, self._m = {}, m   # owned outputs follow the latest call's m
+        outs = DistanceResult(**_outs(b, self._own, "Distance", dict(dist=(dist, (m, self.k), None), fromto=(fromto, (m, self.k, 6), None))))
+        _lib.check(b._L.ur3e_batch_distance(b.ptr, self.id, ids, qp, m, float(distmax), *map(_ptr, outs), b._stream()), "ur3e_batch_distance")
         return outs
 
 

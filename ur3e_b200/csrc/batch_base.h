@@ -47,6 +47,9 @@ struct BatchBase {
   virtual int ik_create(int32_t objtype, int32_t objid, const int32_t* joint_ids, int nj) = 0;
   virtual int ik(int id, const int32_t* env_ids, const void* qpos0, long long m, const void* target_pos, const void* target_quat,
                  const ur3e_ik_options* opt, const ur3e_ik_out* out, cudaStream_t s) = 0;
+  // geom distances (distance.cuh): the batch owns the compiled pair sets; distance_create returns the set's id
+  virtual int distance_create(const int32_t* geom1, const int32_t* geom2, int k) = 0;
+  virtual int distance(int id, const int32_t* env_ids, const void* qpos, long long m, double distmax, void* dist, void* fromto, cudaStream_t s) = 0;
   // T tiered steps of m scratch copies of records (src ids) or of fresh records (qpos0 / qvel0 / ws0); the batch is not modified
   virtual int rollout(const int32_t* src, const void* qpos0, const void* qvel0, const void* ws0, long long m, int T, const void* act,
                       const ur3e_rollout_out* out, cudaStream_t s) = 0;

@@ -11,6 +11,7 @@
 #include "batch_base.h"
 #include "compile_model.h"
 #include "merge_bodies.h"
+#include "distance.cuh"
 #include "env.cuh"
 #include "ik.cuh"
 #include "query.cuh"
@@ -437,6 +438,58 @@ __global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) ik
 }
 
 template <typename Real, typename D>
+struct DistArgs {
+  const DevModel<Real>* m;
+  const EnvState<Real, D>* st;
+  const DistPair<Real>* tab; int k;
+  long long n, count;                 // batch size, states
+  const int* env_ids;                 // [count] or null
+  const Real* qpos;                   // [count, nq] or null (neither: environment i)
+  Real distmax;
+  Real* dist; Real* fromto;           // [count, k], [count, k, 6]; either may be null
+};
+
+// Geom distances (distance.cuh distance_env): one warp per state on the kinematics queries' arena, whose union u holds the overlapping
+// pairs' staging rows; reads qpos of the record or of the caller's array, never writes a record.  An environment id outside [0, n)
+// gets NaN dist and fromto.
+template <typename Real, typename D>
+__global__ void __launch_bounds__(warps_per_block<Real, QueryDims<D>>() * 32) distance_kernel(const DistArgs<Real, D> a) {
+  using DK = QueryDims<D>;
+  constexpr int WPB = warps_per_block<Real, DK>();
+  extern __shared__ int4 smem_raw[];
+  const int warp = threadIdx.x >> 5;
+  const long long i = (long long)blockIdx.x * WPB + warp;
+  if (i >= a.count) return;
+  const DevModel<Real>& m = *a.m;
+  const long long k = a.k;
+  Real* const dst = a.dist ? a.dist + i * k : nullptr;
+  Real* const ft = a.fromto ? a.fromto + i * k * 6 : nullptr;
+  const Real* src;
+  if (a.qpos) src = a.qpos + i * (long long)m.nq;
+  else {
+    const long long e = a.env_ids ? (long long)a.env_ids[i] : i;
+    if (e < 0 || e >= a.n) {
+      const Real nan = std::numeric_limits<Real>::quiet_NaN();
+      if (dst) { WARP_FOR(j, a.k) dst[j] = nan; }
+      if (ft) { WARP_FOR(j, 6 * a.k) ft[j] = nan; }
+      return;
+    }
+    src = a.st[e].qpos;
+  }
+  Arena<Real, DK>& s = *reinterpret_cast<Arena<Real, DK>*>(reinterpret_cast<unsigned char*>(smem_raw) + warp * arena_stride<Real, DK>());
+#ifdef UR3E_CANARY
+  canary_set(s);
+#endif
+  WARP_FOR(j, m.nq) s.st.qpos[j] = src[j];
+  WARP_SYNC();
+  distance_env(m, s, a.tab, a.k, a.distmax, dst, ft);
+#ifdef UR3E_CANARY
+  WARP_SYNC();
+  { const int bad = canary_bad(s); if (bad) { IF_LANE0 printf("ur3e_b200: arena guard word clobbered (mask 0x%x, distance state %lld)\n", bad, i); } }
+#endif
+}
+
+template <typename Real, typename D>
 struct RPArgs {
   const DevModel<Real>* m;
   const EnvState<Real, D>* st;
@@ -548,6 +601,7 @@ struct Batch : BatchBase {
     for (auto& q : queries) cudaFree(q.table);
     for (auto& r : renders) { cudaFree(r.table); cudaFree(r.geoms); }
     for (auto t : iks) cudaFree(t);
+    for (auto& d : dists) cudaFree(d.table);
     cudaFree(d_pose); cudaFree(d_roll);
     if (own_stream) cudaStreamDestroy(own_stream);
     if (own_stream2) cudaStreamDestroy(own_stream2);
@@ -650,7 +704,8 @@ struct Batch : BatchBase {
       CUDA_OK(cudaFuncSetAttribute(query_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
       CUDA_OK(cudaFuncSetAttribute(query_jac_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
       CUDA_OK(cudaFuncSetAttribute(render_pose_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
-      CUDA_OK(cudaFuncSetAttribute(ik_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
+      CUDA_OK(cudaFuncSetAttribute(ik_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem));
+      CUDA_OK(cudaFuncSetAttribute(distance_kernel<Real, D>, cudaFuncAttributeMaxDynamicSharedMemorySize, qsmem)); }
     static_assert(sizeof(Real) * 12 * (RENDER_MAX_GEOMS + 1) + sizeof(RenderGeom<Real>) * RENDER_MAX_GEOMS <= 48 * 1024, "render_kernel's staged scene fits the default shared-memory limit");
     cudaDeviceProp prop; CUDA_OK(cudaGetDeviceProperties(&prop, dev)); sm_count = prop.multiProcessorCount;
     if constexpr (HAS_LITE) {
@@ -961,6 +1016,28 @@ struct Batch : BatchBase {
     IKArgs<Real, D> a{d_model, d_state, iks[id], n, m, env_ids, (const Real*)qpos0, (const Real*)target_pos, (const Real*)target_quat, ko,
                       (Real*)out->qpos, (Real*)out->err_norm, out->info};
     return launch_warps<QueryDims<D>>(ik_kernel<Real, D>, a, s, m);
+  }
+  // ---- geom distances (distance.cuh); the pair tables live until the batch is destroyed
+  struct DistSet { DistPair<Real>* table; int k; };
+  std::vector<DistSet> dists;
+  int distance_create(const int32_t* geom1, const int32_t* geom2, int k) override {
+    CUDA_OK(cudaSetDevice(device));
+    std::vector<DistPair<Real>> tab;
+    const std::string err = compile_distance<Real>(hm, geom1, geom2, k, tab);
+    if (!err.empty()) return set_err("distance_create: " + err);
+    DistPair<Real>* d = nullptr;
+    CUDA_OK(cudaMalloc(&d, sizeof(DistPair<Real>) * k));
+    dists.push_back(DistSet{d, k});
+    CUDA_OK(cudaMemcpy(d, tab.data(), sizeof(DistPair<Real>) * k, cudaMemcpyHostToDevice));
+    return (int)dists.size() - 1;
+  }
+  int distance(int id, const int32_t* env_ids, const void* qpos, long long m, double distmax, void* dist, void* fromto, cudaStream_t s) override {
+    CUDA_OK(cudaSetDevice(device));
+    const std::string err = distance_check(id, (int)dists.size(), m, n, env_ids != nullptr, qpos != nullptr, dist || fromto, distmax);
+    if (!err.empty()) return set_err("distance: " + err);
+    // read-only, like query(): last_stream stays that of the latest state-changing call
+    DistArgs<Real, D> a{d_model, d_state, dists[id].table, dists[id].k, n, m, env_ids, (const Real*)qpos, (Real)distmax, (Real*)dist, (Real*)fromto};
+    return launch_warps<QueryDims<D>>(distance_kernel<Real, D>, a, s, m);
   }
   // ---- rollouts: T tiered steps (step_range) of a scratch batch of m records on the counter slot ROLLOUT_SLOT.  The workspace is
   // grown to the largest m seen: records [m], the three tier lists [m], and obs [m, obs_dim], reward [m], terminated [m] and

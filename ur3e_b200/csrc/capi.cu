@@ -142,5 +142,13 @@ int ur3e_batch_ik(ur3e_batch* b, int ik_id, const int32_t* env_ids_dev, const vo
                   const void* target_quat_dev, const ur3e_ik_options* opt, const ur3e_ik_out* out, void* stream) {
   GUARD(b); return b->impl->ik(ik_id, env_ids_dev, qpos0_dev, m, target_pos_dev, target_quat_dev, opt, out, (cudaStream_t)stream);
 }
+int ur3e_batch_distance_create(ur3e_batch* b, const int32_t* geom1, const int32_t* geom2, int32_t k) {
+  GUARD(b);
+  try { return b->impl->distance_create(geom1, geom2, k); } catch (const std::exception& e) { return set_err(e.what()); }
+}
+int ur3e_batch_distance(ur3e_batch* b, int distance_id, const int32_t* env_ids_dev, const void* qpos_dev, int64_t m, double distmax, void* dist_dev,
+                        void* fromto_dev, void* stream) {
+  GUARD(b); return b->impl->distance(distance_id, env_ids_dev, qpos_dev, m, distmax, dist_dev, fromto_dev, (cudaStream_t)stream);
+}
 
 }  // extern "C"
